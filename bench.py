@@ -16,6 +16,8 @@ With --gpus 8 the line also carries BASELINE config 5 (genome-wide 1 kb, 2 Mb ca
 cfg5_ms_per_step / cfg5_frac.  Other workloads: --workload cfg2 (chr1 @ 5 kb), cfg4 (chr1 @ 1 kb, two passes), cfg5.
 A "step" is one whole pass over the resident records; ms_per_step / value are one pass on its own.  two_passes_in_flight
 (one GPU by default, --overlap on elsewhere) is the throughput when independent passes alternate on two streams.
+--dump-outputs DIR writes what the last timed step computed (rank 0's rows) as float64 .npy files, so that two builds can be
+compared output for output: the inputs are generated from fixed seeds and are the same in every run with the same arguments.
 """
 import argparse
 import hashlib
@@ -36,6 +38,7 @@ DECAY = 1.08
 SEED = 20161108
 BYTES_PER_PAIR = 48          # 12 (K1 read) + 20 (K4 read+write) + 16 (K5 read+write), BASELINE.md section 2
 K4_BYTES_PER_PAIR = 20
+DUMP_ROWS = 1 << 20          # --dump-outputs: records of the seeded sample (at most 32 MiB: row, keep, p, q)
 
 HG19 = [249250621, 243199373, 198022430, 191154276, 180915260, 171115067, 159138663, 146364022, 141213431, 135534747,
         135006516, 133851895, 115169878, 107349540, 102531392, 90354753, 81195210, 78077248, 59128983, 63025520, 48129895,
@@ -402,6 +405,8 @@ def _measure(args, wl_name, world, rank, dev, full, out):
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
     ms_per_step = float(tms.item()) / args.steps
     out["clocks"] = sampler.stop() if sampler else None
+    if full and rank == 0 and args.dump_outputs:
+        _dump_outputs(args.dump_outputs, W, gp)
     out["ms_per_step"] = ms_per_step
     out["P_total"], out["P_local"] = W.P_total, W.P_local
     out["value"] = W.P_total / (ms_per_step * 1e-3)
@@ -629,6 +634,34 @@ def _score_state(gp):
     return _lib.ScoreState.from_buffer_copy(gp.score_state.cpu().numpy().tobytes())
 
 
+def _dump_outputs(path, W, gp):
+    """What a caller of GenomePass holds after the last timed step, as float64 .npy files under `path`: for a fixed, seeded
+    sample of this rank's records (row = the record's index in shard order) keep = (p <= 1) and the p and q of the kept
+    ones (a record that is not scored or is dropped holds NaN, fithic.py:431-434), the distance table and totals K1 left,
+    the fit's bins and spline, and the fit's scalars."""
+    import numpy as np
+    import torch
+    eng = W.eng
+    fit = eng.read_fit()
+    sizes = [sh.n for sh in gp.shards]
+    starts = np.cumsum([0] + sizes)
+    n = int(starts[-1])
+    rows = np.unique(np.random.default_rng(SEED).integers(0, n, DUMP_ROWS)) if n else np.zeros(0, dtype=np.int64)
+    shard = np.searchsorted(starts, rows, side="right") - 1
+    idx = torch.from_numpy(np.asarray(gp.offsets, dtype=np.int64)[shard] + rows - starts[shard]).to(eng.device)
+    p, q = gp.p[idx].cpu().numpy(), gp.q[idx].cpu().numpy()
+    keep = p <= 1
+    arrays = {
+        "row": rows, "keep": keep, "p": p[keep], "q": q[keep], "observed": eng.obs_sum, "totals": eng.totals,
+        "x": eng.x[:fit.n_out], "y": eng.y[:fit.n_out], "spline_y": eng.spline_y[:fit.L],
+        "fit": np.array([fit.S, fit.k0, fit.L, fit.n_out, fit.n_knots, fit.min_x, fit.max_x, fit.residual, fit.smoothing]),
+    }
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
+
+
 def run_ours(args, out_fd):
     import torch
     import torch.distributed as dist
@@ -733,7 +766,13 @@ def main():
                     help="the two-passes-in-flight throughput measurement: auto = on one GPU only")
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS),
                     help="cfg3 (default: the configuration the metric is quoted on), cfg2, cfg4 (two passes) or cfg5")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write keep / p / q (a seeded sample of rank 0's records) and the fit of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU pass (--impl ours)")
     out_fd = _claim_stdout()
     if args.impl == "reference":
         run_reference_arm(args, out_fd)

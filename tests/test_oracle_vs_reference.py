@@ -1,10 +1,12 @@
-"""Build-container only: the oracle against the reference executed live (skipped without /root/reference)."""
+"""The oracle against the original blueberry sources executed live.  They are not part of this repository: point
+BLUEBERRY_REFERENCE at a checkout to run these; without one they skip.  tests/test_oracle_golden.py checks the same
+functions against outputs of the original stored under tests/golden/."""
 import numpy as np
 import pytest
 
 from oracle import ref_loader
 
-pytestmark = pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference absent (GPU box)")
+pytestmark = pytest.mark.skipif(not ref_loader.reference_available(), reason="no checkout of the original blueberry sources (BLUEBERRY_REFERENCE)")
 
 
 def test_live_reference_small_pass():
