@@ -82,21 +82,13 @@ SIGNATURES = {
     "bbk_fit_from_bins": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "bbk_pvalues": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i64, _i64, _vp, _vp,
                                    ctypes.POINTER(BiasTable), _vp, _vp, _vp]),
-    "bbk_pvalues_bh": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i64, _i64, _vp, _vp,
-                                      ctypes.POINTER(BiasTable), _vp, _vp, _vp, _vp, _sz, _vp]),
     "bbk_bh_workspace_bytes": (_sz, [_i64]),
-    "bbk_bh_qvalues_prepared": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "bbk_bh_qvalues": (ctypes.c_int, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),
     "bbk_decimate_workspace_bytes": (_sz, [_i64]),
     "bbk_decimate": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "bbk_contact_band_ingest": (ctypes.c_int, [_vp, _vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
     "bbk_contact_band_normalize": (ctypes.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i32, _vp, _vp, _vp]),
-    "bbk_p_hist": (ctypes.c_int, [_vp, _i64, _vp, _vp]),
-    "bbk_bh_select": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "bbk_bh_select_prepared": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "bbk_bh_rank_gathered": (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "bbk_bh_scatter": (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp]),
-    "bbk_bh_fix_ones": (ctypes.c_int, [_vp, _i64, _f64, _vp, _vp]),
+    "bbk_bh_select": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "bbk_bh_fix_ones_dev": (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp]),
     "bbk_count_band": (ctypes.c_int, [_vp, _i64, _f64, _f64, _vp, _vp]),
     "bbk_stats_pack": (ctypes.c_int, [_vp, _vp, _i32, _i32, _vp]),

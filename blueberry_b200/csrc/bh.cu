@@ -41,7 +41,7 @@ struct BhState {                    // device-resident control block (first byte
     double total_max;               // running max over all candidates
     int need_ones_fix;              // q_ones != 1.0 -> rewrite the ones
     int skip[NPASS];
-    int use_list;                   // prepared mode: K4's small-p list holds every candidate (saturation below BBK_SMALL_P)
+    int use_list;                   // listed mode: K4's candidate list holds every candidate (saturation below BBK_SMALL_P)
 };
 
 struct BhLayout {
@@ -120,7 +120,7 @@ __global__ void __launch_bounds__(BH_THREADS) bh_hist_kernel(const double* p, lo
 }
 
 // one CTA of 1024 threads (4 buckets each): totals, N, and the saturation bucket
-__global__ void __launch_bounds__(1024) bh_threshold_kernel(BhState* st, const long long* phist, int prune, int prepared,
+__global__ void __launch_bounds__(1024) bh_threshold_kernel(BhState* st, const long long* phist, int prune, int listed,
                                                             const BbkScoreState* ss = nullptr) {
     __shared__ long long part[1024];
     __shared__ int first_bucket;
@@ -163,9 +163,9 @@ __global__ void __launch_bounds__(1024) bh_threshold_kernel(BhState* st, const l
         st->n_tests = n_tests;
         const unsigned long long tau = first_bucket < BBK_PHIST_BINS ? (((unsigned long long)first_bucket << 51) | 0x8000000000000000ull) : ~0ull;
         st->tau_key = tau;
-        // prepared mode: K4's bit per record (p < BBK_SMALL_P) stands in for the pass over p when it covers every candidate
+        // listed mode: K4's list of the rows with p < BBK_SMALL_P stands in for the pass over p when it covers every candidate
         // (a candidate list that overflowed is no list: the full pass over p takes over)
-        st->use_list = (prepared && tau <= bbk_key_of(BBK_SMALL_P) && !(ss && ss->cand_overflow)) ? 1 : 0;
+        st->use_list = (listed && tau <= bbk_key_of(BBK_SMALL_P) && !(ss && ss->cand_overflow)) ? 1 : 0;
     }
 }
 
@@ -228,58 +228,6 @@ __global__ void __launch_bounds__(BH_THREADS) bh_compact_kernel(const double* p,
                 pos += 1;
             }
         }
-    }
-}
-
-// prepared mode: the candidates are among the records K4 flagged (p < BBK_SMALL_P): m/8 bytes of flags plus one
-// sector per flagged record instead of the 16 B/pair pass.  One flag word per thread and grid step; every set bit is an
-// independent scattered read.  Candidates are staged in shared memory and appended with ONE global atomic per CTA
-// flush: a warp-aggregated atomic per round was 1e5 same-address atomics on cfg2 - 100 us on their own.
-constexpr int MF_CAP = 2048;
-__global__ void __launch_bounds__(BH_THREADS) bh_mask_filter_kernel(BhState* st, const unsigned* mask, const double* p, long long m,
-                                                                    unsigned long long* keys, unsigned* idx) {
-    __shared__ unsigned long long s_keys[MF_CAP];
-    __shared__ unsigned s_idx[MF_CAP];
-    __shared__ unsigned s_cnt;
-    __shared__ unsigned long long s_base;
-    if (!st->use_list) return;
-    if (threadIdx.x == 0) s_cnt = 0;
-    __syncthreads();
-    const unsigned long long tau = st->tau_key;
-    const long long n_words = ((m >> 2) + 31) / 32 * 4;      // 4 words per (started) block of 32 four-record groups
-    const long long stride = (long long)gridDim.x * blockDim.x;
-    const long long n_iter = (n_words + 1 + stride - 1) / stride;       // + 1: a pseudo word for the last m % 4 records
-    long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    for (long long it = 0; it <= n_iter; ++it, w += stride) {
-        if (it < n_iter) {
-            unsigned bits = 0;
-            long long rec0 = 0;
-            int step = 4;
-            if (w < n_words) { bits = mask[w]; rec0 = (w >> 2) * 128 + (w & 3); }
-            else if (w == n_words) { bits = (1u << (m & 3)) - 1; rec0 = (m >> 2) << 2; step = 1; }     // unflagged tail: look at all
-            while (bits) {
-                const int l = __ffs(bits) - 1;
-                bits &= bits - 1;
-                const long long rec = rec0 + (long long)step * l;
-                const double v = p[rec];
-                const unsigned long long k = bbk_key_of(v);
-                if (!isnan(v) && v != 1.0 && k < tau) {
-                    const unsigned pos = atomicAdd(&s_cnt, 1u);
-                    if (pos < MF_CAP) { s_keys[pos] = k; s_idx[pos] = (unsigned)rec; }
-                    else { const unsigned long long g = atomicAdd(&st->n_cand, 1ull); keys[g] = k; idx[g] = (unsigned)rec; }   // stage full
-                }
-            }
-        }
-        __syncthreads();
-        const unsigned staged = s_cnt < (unsigned)MF_CAP ? s_cnt : (unsigned)MF_CAP;
-        if (staged >= MF_CAP / 2 || (it == n_iter && staged > 0)) {      // CTA-uniform
-            if (threadIdx.x == 0) s_base = atomicAdd(&st->n_cand, (unsigned long long)staged);
-            __syncthreads();
-            for (unsigned i = threadIdx.x; i < staged; i += blockDim.x) { keys[s_base + i] = s_keys[i]; idx[s_base + i] = s_idx[i]; }
-            __syncthreads();
-            if (threadIdx.x == 0) s_cnt = 0;
-        }
-        __syncthreads();
     }
 }
 
@@ -553,7 +501,7 @@ constexpr size_t RK_DYN_SMEM = (size_t)RK_TILE * (sizeof(unsigned long long) + s
 
 struct RankParams {
     BhLayout L;
-    double* q;               // output (input order, or gathered order for bbk_bh_rank_gathered)
+    double* q;               // output (input order, or gathered order for bbk_bh_rank_gathered_padded)
     long long* rank;         // optional
     long long n_host;        // >= 0: number of (key, index) pairs, known to the host; < 0: BhState::n_cand
     int src;                 // buffer (0 / 1) the pairs start in; a sort-only launch leaves the result there
@@ -891,33 +839,11 @@ __global__ void export_state_kernel(const BhState* st, unsigned long long* out) 
     out[0] = st->n_cand; out[1] = st->tau_key; out[2] = (unsigned long long)st->n_tests; out[3] = st->n_ones;
 }
 
-__global__ void import_state_kernel(BhState* st, const unsigned long long* in, unsigned long long n_all) {
-    st->n_cand = n_all; st->tau_key = in[1]; st->n_tests = (long long)in[2]; st->n_ones = in[3];
-    st->n_nan = 0; st->n_valid = 0; st->q_ones = 1.0; st->total_max = 0.0; st->need_ones_fix = 0;
-    for (int p = 0; p < NPASS; ++p) st->skip[p] = 0;
-}
-
-__global__ void __launch_bounds__(BH_THREADS) load_keys_kernel(const unsigned long long* in, long long n, unsigned long long* keys, unsigned* idx) {
-    long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) { keys[i] = in[i]; idx[i] = (unsigned)i; }
-}
-
 __global__ void export_ones_kernel(const BhState* st, double* out) { out[0] = st->q_ones; out[1] = st->need_ones_fix ? 1.0 : 0.0; }
-
-__global__ void __launch_bounds__(BH_THREADS) scatter_q_kernel(const double* src, const unsigned* idx, long long n, double* dst) {
-    long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) dst[idx[i]] = src[i];
-}
 
 __global__ void __launch_bounds__(BH_THREADS) fix_ones_dev_kernel(const double* p, long long m, double* q, const double* q_ones) {
     if (q_ones[1] == 0.0) return;                           // q(p == 1) is 1.0: nothing to do
     const double qo = q_ones[0];
-    long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride)
-        if (p[i] == 1.0) q[i] = qo;
-}
-
-__global__ void __launch_bounds__(BH_THREADS) fix_ones_value_kernel(const double* p, long long m, double* q, double qo) {
     long long stride = (long long)gridDim.x * blockDim.x;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride)
         if (p[i] == 1.0) q[i] = qo;
@@ -984,52 +910,7 @@ extern "C" int bbk_bh_qvalues(const double* d_p, int64_t m, int64_t n_tests, int
     return BBK_OK;
 }
 
-// K4's flag bits (m/8 bytes) live in the sort's second index buffer (4 m bytes), which nothing uses before the first radix pass
-unsigned* bbk_bh_mask_buffer(void* workspace, long long m) {
-    BhLayout L;
-    bh_layout(workspace, m, sort_blocks(), &L);
-    return L.idx[1];
-}
-
-extern "C" int bbk_bh_qvalues_prepared(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist, double* d_q,
-                                       void* d_workspace, size_t workspace_bytes, void* stream) {
-    BBK_REQUIRE(m >= 0 && m < (1ll << 32), "bbk_bh_qvalues_prepared: m must be in [0, 2^32)");
-    if (m == 0) return BBK_OK;
-    BBK_REQUIRE(d_p && d_q && d_p_hist && d_workspace, "bbk_bh_qvalues_prepared: null pointer");
-    BBK_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "bbk_bh_qvalues_prepared: workspace must be 256-byte aligned");
-    const int G = sort_blocks();
-    BhLayout L;
-    size_t need = bh_layout(d_workspace, m, G, &L);
-    if (workspace_bytes < need) {
-        bbk_set_error("bbk_bh_qvalues_prepared: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
-        return BBK_E_WORKSPACE;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    const int sms = bbk_num_sms();
-    bh_init_kernel<<<(BBK_PHIST_BINS + 2 + 255) / 256, 256, 0, st>>>(L.st, L.phist, (const long long*)d_p_hist, n_tests);
-    BBK_CHECK_LAUNCH("bh_init_kernel");
-    bh_threshold_kernel<<<1, 1024, 0, st>>>(L.st, L.phist, 1, 1);
-    BBK_CHECK_LAUNCH("bh_threshold_kernel");
-    {
-        long long words = ((m >> 2) + 31) / 32 * 4 + 1, wantw = (words + BH_THREADS - 1) / BH_THREADS;
-        int gridw = (int)(wantw < (long long)sms * 8 ? wantw : (long long)sms * 8);
-        bh_mask_filter_kernel<<<gridw, BH_THREADS, 0, st>>>(L.st, L.idx[1], d_p, m, L.keys[0], L.idx[0]);
-        BBK_CHECK_LAUNCH("bh_mask_filter_kernel");
-    }
-    long long want = (m + BH_THREADS - 1) / BH_THREADS;
-    int grid = (int)(want < (long long)sms * 8 ? want : (long long)sms * 8);
-    // saturation above BBK_SMALL_P (many significant rows): the 16 B/pair pass after all; otherwise returns at once
-    bh_compact_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, m, d_q, L.st, L.keys[0], L.idx[0], 0, nullptr);
-    BBK_CHECK_LAUNCH("bh_compact_kernel");
-    int rc = launch_rank(L, d_q, nullptr, st);
-    if (rc != BBK_OK) return rc;
-    ones_fix_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, m, d_q, L.st);
-    BBK_CHECK_LAUNCH("ones_fix_kernel");
-    return BBK_OK;
-}
-
-
-// after bbk_pvalues_listed: q is pre-filled (1.0 / NaN) for every row and the rows with p < BBK_SMALL_P are listed in `cands`
+// after bbk_score_pairs / bbk_score_deferred: q is pre-filled (1.0 / NaN) for every row and the rows with p < BBK_SMALL_P are listed in `cands`
 extern "C" int bbk_bh_qvalues_listed(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist, double* d_q,
                                      const BbkCandidates* cands, const BbkScoreState* d_state, void* d_workspace,
                                      size_t workspace_bytes, void* stream) {
@@ -1068,46 +949,39 @@ extern "C" int bbk_bh_qvalues_listed(const double* d_p, int64_t m, int64_t n_tes
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Genome-wide q-values across ranks (SURVEY.md section 8e, collective 2), in three local steps around two
-// host-side collectives:
-//   all-reduce(p_hist)  ->  bbk_bh_select  ->  all-gather(candidate keys)  ->  bbk_bh_rank_gathered
-//   ->  bbk_bh_scatter (and bbk_bh_fix_ones in the rare case q(p == 1) < 1)
+// Genome-wide q-values across ranks (SURVEY.md section 8e, collective 2), in local steps around two host-side collectives:
+//   all-reduce(p_hist)  ->  bbk_bh_select[_listed]  ->  bbk_bh_pack_count  ->  all-gather(fixed-capacity key blocks)
+//   ->  bbk_bh_rank_gathered_padded  ->  bbk_bh_fix_ones_dev (the rare case q(p == 1) < 1)
 // ---------------------------------------------------------------------------------------------------
+// cands / d_score: the candidate list of bbk_score_pairs (listed mode), or NULL for a pass over p
 static int bh_select_impl(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
-                          uint64_t* d_keys, uint32_t* d_idx, uint64_t* d_state, void* d_workspace, size_t workspace_bytes,
-                          bool prepared, void* stream, const BbkCandidates* cands = nullptr, const BbkScoreState* d_score = nullptr,
-                          long long keys_cap = -1) {
+                          const BbkCandidates* cands, const BbkScoreState* d_score, uint64_t* d_keys, uint32_t* d_idx,
+                          int64_t keys_capacity, uint64_t* d_state, void* d_workspace, size_t workspace_bytes, void* stream) {
     BBK_REQUIRE(m >= 0 && m < (1ll << 32), "bbk_bh_select: m must be in [0, 2^32)");
+    BBK_REQUIRE(keys_capacity >= 0, "bbk_bh_select: negative key capacity");
     BBK_REQUIRE(d_p_hist_global && d_state && d_workspace, "bbk_bh_select: null pointer");
     BBK_REQUIRE(m == 0 || (d_p && d_q && d_keys && d_idx), "bbk_bh_select: null array");
     BBK_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "bbk_bh_select: workspace must be 256-byte aligned");
     const int G = sort_blocks();
     BhLayout L;
-    // prepared: the workspace is the one bbk_pvalues_bh left the flag bits in (laid out for m records)
-    size_t need = bh_layout(d_workspace, (prepared && !cands) ? m : 0, G, &L);
+    size_t need = bh_layout(d_workspace, 0, G, &L);
     if (workspace_bytes < need) { bbk_set_error("bbk_bh_select: workspace too small (%zu < %zu bytes)", workspace_bytes, need); return BBK_E_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
     const int sms = bbk_num_sms();
     bh_init_kernel<<<(BBK_PHIST_BINS + 2 + 255) / 256, 256, 0, st>>>(L.st, L.phist, (const long long*)d_p_hist_global, n_tests);
     BBK_CHECK_LAUNCH("bh_init_kernel");
-    bh_threshold_kernel<<<1, 1024, 0, st>>>(L.st, L.phist, 1, prepared ? 1 : 0, d_score);
+    bh_threshold_kernel<<<1, 1024, 0, st>>>(L.st, L.phist, 1, cands ? 1 : 0, d_score);
     BBK_CHECK_LAUNCH("bh_threshold_kernel");
     if (m > 0) {
-        if (cands) {
-            if (cands->capacity > 0) {
-                bh_cand_filter_kernel<<<sms * 2, BH_THREADS, 0, st>>>(L.st, d_score, (const unsigned long long*)cands->d_keys, cands->d_rows,
-                                                                      (unsigned long long*)d_keys, d_idx, keys_cap);
-                BBK_CHECK_LAUNCH("bh_cand_filter_kernel");
-            }
-        } else if (prepared) {
-            long long words = ((m >> 2) + 31) / 32 * 4 + 1, wantw = (words + BH_THREADS - 1) / BH_THREADS;
-            int gridw = (int)(wantw < (long long)sms * 8 ? wantw : (long long)sms * 8);
-            bh_mask_filter_kernel<<<gridw, BH_THREADS, 0, st>>>(L.st, L.idx[1], d_p, m, (unsigned long long*)d_keys, d_idx);
-            BBK_CHECK_LAUNCH("bh_mask_filter_kernel");
+        if (cands && cands->capacity > 0) {
+            bh_cand_filter_kernel<<<sms * 2, BH_THREADS, 0, st>>>(L.st, d_score, (const unsigned long long*)cands->d_keys, cands->d_rows,
+                                                                  (unsigned long long*)d_keys, d_idx, keys_capacity);
+            BBK_CHECK_LAUNCH("bh_cand_filter_kernel");
         }
         long long want = (m + BH_THREADS - 1) / BH_THREADS;
         int grid = (int)(want < (long long)sms * 8 ? want : (long long)sms * 8);
-        bh_compact_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, m, d_q, L.st, (unsigned long long*)d_keys, d_idx, 0, nullptr, keys_cap);
+        // listed mode with the saturation above BBK_SMALL_P, or an overflowed list: the 16 B/pair pass; otherwise returns at once
+        bh_compact_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, m, d_q, L.st, (unsigned long long*)d_keys, d_idx, 0, nullptr, keys_capacity);
         BBK_CHECK_LAUNCH("bh_compact_kernel");
     }
     export_state_kernel<<<1, 1, 0, st>>>(L.st, (unsigned long long*)d_state);
@@ -1116,51 +990,20 @@ static int bh_select_impl(const double* d_p, int64_t m, int64_t n_tests, const i
 }
 
 extern "C" int bbk_bh_select(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
-                             uint64_t* d_keys, uint32_t* d_idx, uint64_t* d_state, void* d_workspace, size_t workspace_bytes,
-                             void* stream) {
-    return bh_select_impl(d_p, m, n_tests, d_p_hist_global, d_q, d_keys, d_idx, d_state, d_workspace, workspace_bytes, false, stream);
+                             uint64_t* d_keys, uint32_t* d_idx, int64_t keys_capacity, uint64_t* d_state, void* d_workspace,
+                             size_t workspace_bytes, void* stream) {
+    return bh_select_impl(d_p, m, n_tests, d_p_hist_global, d_q, nullptr, nullptr, d_keys, d_idx, keys_capacity, d_state, d_workspace,
+                          workspace_bytes, stream);
 }
 
-extern "C" int bbk_bh_select_prepared(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
-                                      uint64_t* d_keys, uint32_t* d_idx, uint64_t* d_state, void* d_workspace,
-                                      size_t workspace_bytes, void* stream) {
-    return bh_select_impl(d_p, m, n_tests, d_p_hist_global, d_q, d_keys, d_idx, d_state, d_workspace, workspace_bytes, true, stream);
-}
-
-/* bbk_bh_select after bbk_pvalues_listed (q pre-filled, candidates listed) */
+/* bbk_bh_select after bbk_score_pairs / bbk_score_deferred (q pre-filled, candidates listed) */
 extern "C" int bbk_bh_select_listed(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
                                     const BbkCandidates* cands, const BbkScoreState* d_score, uint64_t* d_keys, uint32_t* d_idx,
                                     int64_t keys_capacity, uint64_t* d_state, void* d_workspace, size_t workspace_bytes, void* stream) {
-    BBK_REQUIRE(cands && d_score && keys_capacity >= 0, "bbk_bh_select_listed: null candidate list / score state");
+    BBK_REQUIRE(cands && d_score, "bbk_bh_select_listed: null candidate list / score state");
     BBK_REQUIRE(cands->capacity >= 0 && (cands->capacity == 0 || (cands->d_keys && cands->d_rows)), "bbk_bh_select_listed: incomplete candidate list");
-    return bh_select_impl(d_p, m, n_tests, d_p_hist_global, d_q, d_keys, d_idx, d_state, d_workspace, workspace_bytes, true, stream, cands, d_score,
-                          keys_capacity);
-}
-
-extern "C" int bbk_bh_rank_gathered(const uint64_t* d_keys_all, int64_t n_all, const uint64_t* d_state, double* d_q_all,
-                                    double* d_q_ones, void* d_workspace, size_t workspace_bytes, void* stream) {
-    BBK_REQUIRE(n_all >= 0 && n_all < (1ll << 32), "bbk_bh_rank_gathered: n_all must be in [0, 2^32)");
-    BBK_REQUIRE(d_state && d_q_ones && d_workspace, "bbk_bh_rank_gathered: null pointer");
-    BBK_REQUIRE(n_all == 0 || (d_keys_all && d_q_all), "bbk_bh_rank_gathered: null array");
-    BBK_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "bbk_bh_rank_gathered: workspace must be 256-byte aligned");
-    const int G = sort_blocks();
-    BhLayout L;
-    size_t need = bh_layout(d_workspace, n_all, G, &L);
-    if (workspace_bytes < need) { bbk_set_error("bbk_bh_rank_gathered: workspace too small (%zu < %zu bytes)", workspace_bytes, need); return BBK_E_WORKSPACE; }
-    cudaStream_t st = (cudaStream_t)stream;
-    import_state_kernel<<<1, 1, 0, st>>>(L.st, (const unsigned long long*)d_state, (unsigned long long)n_all);
-    BBK_CHECK_LAUNCH("import_state_kernel");
-    if (n_all > 0) {
-        long long want = (n_all + BH_THREADS - 1) / BH_THREADS;
-        int grid = (int)(want < (long long)bbk_num_sms() * 8 ? want : (long long)bbk_num_sms() * 8);
-        load_keys_kernel<<<grid, BH_THREADS, 0, st>>>((const unsigned long long*)d_keys_all, n_all, L.keys[0], L.idx[0]);
-        BBK_CHECK_LAUNCH("load_keys_kernel");
-    }
-    int rc = launch_rank(L, d_q_all, nullptr, st);
-    if (rc != BBK_OK) return rc;
-    export_ones_kernel<<<1, 1, 0, st>>>(L.st, d_q_ones);
-    BBK_CHECK_LAUNCH("export_ones_kernel");
-    return BBK_OK;
+    return bh_select_impl(d_p, m, n_tests, d_p_hist_global, d_q, cands, d_score, d_keys, d_idx, keys_capacity, d_state, d_workspace,
+                          workspace_bytes, stream);
 }
 
 // ---- the same with the gather left on the device: no candidate count ever travels to the host -------------------------
@@ -1262,40 +1105,6 @@ extern "C" int bbk_bh_rank_gathered_padded(const uint64_t* d_recv, int32_t world
         scatter_slice_kernel<<<grid, BH_THREADS, 0, st>>>(q_all, offsets, rank, d_idx_local, d_q_dst);
         BBK_CHECK_LAUNCH("scatter_slice_kernel");
     }
-    return BBK_OK;
-}
-
-extern "C" int bbk_bh_scatter(const double* d_q_src, const uint32_t* d_idx, int64_t n, double* d_q_dst, void* stream) {
-    BBK_REQUIRE(n >= 0, "bbk_bh_scatter: negative size");
-    if (n == 0) return BBK_OK;
-    BBK_REQUIRE(d_q_src && d_idx && d_q_dst, "bbk_bh_scatter: null pointer");
-    long long want = (n + BH_THREADS - 1) / BH_THREADS;
-    int grid = (int)(want < (long long)bbk_num_sms() * 8 ? want : (long long)bbk_num_sms() * 8);
-    scatter_q_kernel<<<grid, BH_THREADS, 0, (cudaStream_t)stream>>>(d_q_src, d_idx, n, d_q_dst);
-    BBK_CHECK_LAUNCH("scatter_q_kernel");
-    return BBK_OK;
-}
-
-extern "C" int bbk_bh_fix_ones(const double* d_p, int64_t m, double q_ones, double* d_q, void* stream) {
-    BBK_REQUIRE(m >= 0, "bbk_bh_fix_ones: negative size");
-    if (m == 0) return BBK_OK;
-    BBK_REQUIRE(d_p && d_q, "bbk_bh_fix_ones: null pointer");
-    long long want = (m + BH_THREADS - 1) / BH_THREADS;
-    int grid = (int)(want < (long long)bbk_num_sms() * 8 ? want : (long long)bbk_num_sms() * 8);
-    fix_ones_value_kernel<<<grid, BH_THREADS, 0, (cudaStream_t)stream>>>(d_p, m, d_q, q_ones);
-    BBK_CHECK_LAUNCH("fix_ones_value_kernel");
-    return BBK_OK;
-}
-
-// coarse p histogram alone (what K4 fills when asked): needed before the all-reduce when p did not come from K4
-extern "C" int bbk_p_hist(const double* d_p, int64_t m, int64_t* d_p_hist, void* stream) {
-    BBK_REQUIRE(m >= 0 && d_p_hist, "bbk_p_hist: bad arguments");
-    if (m == 0) return BBK_OK;
-    BBK_REQUIRE(d_p, "bbk_p_hist: null p");
-    long long want = (m + BH_THREADS - 1) / BH_THREADS;
-    int grid = (int)(want < (long long)bbk_num_sms() * 8 ? want : (long long)bbk_num_sms() * 8);
-    bh_hist_kernel<<<grid, BH_THREADS, 0, (cudaStream_t)stream>>>(d_p, m, (long long*)d_p_hist);
-    BBK_CHECK_LAUNCH("bh_hist_kernel");
     return BBK_OK;
 }
 

@@ -11,13 +11,10 @@
 void bbk_set_error(const char* fmt, ...);
 int bbk_num_sms();
 
-// K4 -> K5 hand-over (bbk_pvalues_bh / bbk_bh_qvalues_prepared): K4 leaves one bit per record, p < BBK_SMALL_P, so that
-// the q-value step finds its candidates from m/8 bytes instead of another pass over p.  Exact whatever the bound: when
+// K4 -> K5 hand-over (bbk_score_pairs / bbk_score_deferred -> bbk_bh_*_listed): K4 lists (key, row) of every p < BBK_SMALL_P,
+// so that the q-value step finds its candidates in that list instead of another pass over p.  Exact whatever the bound: when
 // the saturation bucket lies above it, K5 falls back to its own pass.
-// Layout: uint4 per 128 consecutive records; bit l of word e = record 128 j + 4 l + e.
 #define BBK_SMALL_P 0.03125
-// where K4 puts the bits inside K5's workspace (defined in bh.cu)
-unsigned* bbk_bh_mask_buffer(void* workspace, long long m);
 // the library's radix sort on its own (bh.cu): n (u64 key, u32 value) pairs in buffer `src` (0 / 1) of a workspace of
 // bbk_bh_workspace_bytes(capacity) bytes, stable, result left in the same buffer; n_host < 0: count at bbk_sort_count_ptr
 void bbk_sort_buffers(void* workspace, long long capacity, int which, unsigned long long** keys, unsigned** idx);

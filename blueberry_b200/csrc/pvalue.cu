@@ -258,10 +258,6 @@ struct PvParams {
     int n_chrom;
     double* p;
     long long* p_hist;
-    // hand-over to the q-value step (both NULL unless bbk_pvalues_bh): q pre-filled with 1.0 / NaN, and one bit per record
-    // (p < BBK_SMALL_P); the last n_pairs % 4 records have no bit, K5 looks at them itself
-    double* q;
-    unsigned* small_mask;
 };
 
 struct BiasRow { long long base, nloc, mid0; unsigned long long span; };     // span = nloc * R
@@ -377,10 +373,6 @@ __device__ __forceinline__ bool record_prior(const PvParams& P, int m1, int m2, 
 
 __device__ __forceinline__ double finish_p(double pv) {                  // fithic.py:434: rows with !(p <= 1) are dropped
     return (pv <= 1.0) ? pv : __longlong_as_double(0x7ff8000000000000ll);
-}
-
-__device__ __forceinline__ double prefill_q(double pv) {                 // q of a row that is not a candidate
-    return isnan(pv) ? pv : 1.0;
 }
 
 __device__ __forceinline__ void hist_p(unsigned* sh_hist, double pv, unsigned& ones, unsigned& nans) {
@@ -609,18 +601,6 @@ __global__ void __launch_bounds__(PV_THREADS, 3) pvalues_kernel(PvParams P) {
                 st_stream_double2(pv2 + 2 * g + 1, r23);
                 if (HIST) { hist_p(sh_hist, r01.x, ones, nans); hist_p(sh_hist, r01.y, ones, nans);
                             hist_p(sh_hist, r23.x, ones, nans); hist_p(sh_hist, r23.y, ones, nans); }
-                if (HIST && P.q) {
-                    double2* qv2 = reinterpret_cast<double2*>(P.q);
-                    st_stream_double2(qv2 + 2 * g, make_double2(prefill_q(r01.x), prefill_q(r01.y)));
-                    st_stream_double2(qv2 + 2 * g + 1, make_double2(prefill_q(r23.x), prefill_q(r23.y)));
-                }
-            }
-            if (HIST && P.q && (wt * groups_per_tile + it * 32) < n_groups) {
-                // one bit per record: p < BBK_SMALL_P.  Word e of the warp-iteration holds element e of every lane's group.
-                const bool in = g < n_groups;
-                const unsigned w0 = __ballot_sync(0xffffffffu, in && r01.x < BBK_SMALL_P), w1 = __ballot_sync(0xffffffffu, in && r01.y < BBK_SMALL_P);
-                const unsigned w2 = __ballot_sync(0xffffffffu, in && r23.x < BBK_SMALL_P), w3 = __ballot_sync(0xffffffffu, in && r23.y < BBK_SMALL_P);
-                if (lane == 0) reinterpret_cast<uint4*>(P.small_mask)[wt * WT_ITERS + it] = make_uint4(w0, w1, w2, w3);
             }
         }
         __syncwarp();      // the tile buffers are reused by the next warp tile
@@ -669,7 +649,6 @@ __global__ void pvalues_tail_kernel(PvParams P) {
         if (isnan(pv)) atomicAdd((unsigned long long*)&P.p_hist[BBK_PHIST_BINS + 1], 1ull);
         else if (pv == 1.0) atomicAdd((unsigned long long*)&P.p_hist[BBK_PHIST_BINS], 1ull);
         else atomicAdd((unsigned long long*)&P.p_hist[(unsigned)((unsigned long long)__double_as_longlong(pv) >> 51) & (BBK_PHIST_BINS - 1)], 1ull);
-        if (P.q) P.q[i] = prefill_q(pv);
     }
 }
 
@@ -711,25 +690,23 @@ int launch_pv(const PvParams& P, cudaStream_t st) {
 
 }  // namespace
 
-static int pvalues_impl(const int32_t* d_chr1, const int32_t* d_chr2, const int32_t* d_mid1, const int32_t* d_mid2,
-                        const int32_t* d_count, int64_t n_pairs, int32_t shard_chrom, int64_t resolution, int64_t min_dist,
-                        int64_t max_dist, const BbkFitResult* d_fit, const double* d_spline_y, const BbkBiasTable* bias,
-                        double* d_p, int64_t* d_p_hist, double* d_q, unsigned* small_mask, void* stream) {
+extern "C" int bbk_pvalues(const int32_t* d_chr1, const int32_t* d_chr2, const int32_t* d_mid1, const int32_t* d_mid2,
+                           const int32_t* d_count, int64_t n_pairs, int32_t shard_chrom, int64_t resolution, int64_t min_dist,
+                           int64_t max_dist, const BbkFitResult* d_fit, const double* d_spline_y, const BbkBiasTable* bias,
+                           double* d_p, int64_t* d_p_hist, void* stream) {
     BBK_REQUIRE(n_pairs >= 0, "bbk_pvalues: negative size");
     BBK_REQUIRE(resolution > 0 && resolution < (1ll << 32), "bbk_pvalues: resolution must be in [1, 2^32)");
     BBK_REQUIRE((d_chr1 == nullptr) == (d_chr2 == nullptr), "bbk_pvalues: chr1/chr2 must both be given or both NULL");
     BBK_REQUIRE(d_fit && d_spline_y, "bbk_pvalues: null fit");
     if (n_pairs == 0) return BBK_OK;
     BBK_REQUIRE(d_mid1 && d_mid2 && d_count && d_p, "bbk_pvalues: null column");
-    uintptr_t align = (uintptr_t)d_mid1 | (uintptr_t)d_mid2 | (uintptr_t)d_count | (uintptr_t)d_chr1 | (uintptr_t)d_chr2 | (uintptr_t)d_p |
-                      (uintptr_t)d_q;
+    uintptr_t align = (uintptr_t)d_mid1 | (uintptr_t)d_mid2 | (uintptr_t)d_count | (uintptr_t)d_chr1 | (uintptr_t)d_chr2 | (uintptr_t)d_p;
     BBK_REQUIRE((align & 15) == 0, "bbk_pvalues: columns must be 16-byte aligned");
     PvParams P = {};
     P.chr1 = d_chr1; P.chr2 = d_chr2; P.mid1 = d_mid1; P.mid2 = d_mid2; P.count = d_count;
     P.n_pairs = n_pairs; P.shard_chrom = shard_chrom; P.R = resolution; P.min_dist = min_dist; P.max_dist = max_dist;
     P.div = make_fastdiv((uint64_t)resolution);
     P.fit = d_fit; P.spline_y = d_spline_y; P.p = d_p; P.p_hist = (long long*)d_p_hist;
-    P.q = d_q; P.small_mask = small_mask;
     bool has_bias = bias && bias->d_bias;
     if (has_bias) {
         BBK_REQUIRE(bias->d_chrom_base && bias->d_mid0 && bias->n_chrom > 0, "bbk_pvalues: incomplete bias table");
@@ -752,31 +729,6 @@ static int pvalues_impl(const int32_t* d_chr1, const int32_t* d_chr2, const int3
     BBK_PV_CASE(true, true, false)   BBK_PV_CASE(true, true, true)
 #undef BBK_PV_CASE
     return BBK_E_INVALID;
-}
-
-extern "C" int bbk_pvalues(const int32_t* d_chr1, const int32_t* d_chr2, const int32_t* d_mid1, const int32_t* d_mid2,
-                           const int32_t* d_count, int64_t n_pairs, int32_t shard_chrom, int64_t resolution, int64_t min_dist,
-                           int64_t max_dist, const BbkFitResult* d_fit, const double* d_spline_y, const BbkBiasTable* bias,
-                           double* d_p, int64_t* d_p_hist, void* stream) {
-    return pvalues_impl(d_chr1, d_chr2, d_mid1, d_mid2, d_count, n_pairs, shard_chrom, resolution, min_dist, max_dist, d_fit,
-                        d_spline_y, bias, d_p, d_p_hist, nullptr, nullptr, stream);
-}
-
-extern "C" int bbk_pvalues_bh(const int32_t* d_chr1, const int32_t* d_chr2, const int32_t* d_mid1, const int32_t* d_mid2,
-                              const int32_t* d_count, int64_t n_pairs, int32_t shard_chrom, int64_t resolution, int64_t min_dist,
-                              int64_t max_dist, const BbkFitResult* d_fit, const double* d_spline_y, const BbkBiasTable* bias,
-                              double* d_p, int64_t* d_p_hist, double* d_q, void* d_bh_workspace, size_t workspace_bytes,
-                              void* stream) {
-    BBK_REQUIRE(n_pairs >= 0 && n_pairs < (1ll << 32), "bbk_pvalues_bh: n_pairs must be in [0, 2^32)");
-    BBK_REQUIRE(d_p_hist && d_bh_workspace, "bbk_pvalues_bh: the histogram and the q-value workspace are required");
-    BBK_REQUIRE(n_pairs == 0 || d_q, "bbk_pvalues_bh: null q");
-    BBK_REQUIRE(((uintptr_t)d_bh_workspace & 255) == 0, "bbk_pvalues_bh: workspace must be 256-byte aligned");
-    if (workspace_bytes < bbk_bh_workspace_bytes(n_pairs)) {
-        bbk_set_error("bbk_pvalues_bh: workspace too small (%zu < %zu bytes)", workspace_bytes, bbk_bh_workspace_bytes(n_pairs));
-        return BBK_E_WORKSPACE;
-    }
-    return pvalues_impl(d_chr1, d_chr2, d_mid1, d_mid2, d_count, n_pairs, shard_chrom, resolution, min_dist, max_dist, d_fit,
-                        d_spline_y, bias, d_p, d_p_hist, d_q, bbk_bh_mask_buffer(d_bh_workspace, n_pairs), stream);
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -150,11 +150,11 @@ class GenomePass(object):
                 self.c_rows = torch.empty(ccap, dtype=torch.int32, device=dev)
                 self.cands = _lib.Candidates(self.c_keys.data_ptr(), self.c_rows.data_ptr(), ccap)
         if self.q_values:
-            if self.world == 1 or not self.listed:
+            if self.world == 1:
                 need = int(self.lib.bbk_bh_workspace_bytes(m))
                 if getattr(self, "bh_ws", None) is None or self.bh_ws.numel() < need:
                     self.bh_ws = torch.empty(need, dtype=torch.uint8, device=dev)
-            if self.world > 1 and self.listed and getattr(self, "sel_ws", None) is None:
+            elif getattr(self, "sel_ws", None) is None:
                 self.sel_ws = torch.empty(int(self.lib.bbk_bh_workspace_bytes(0)), dtype=torch.uint8, device=dev)
                 self._alloc_gather()
         return self
@@ -260,18 +260,20 @@ class GenomePass(object):
                 eng.launches += 6          # init, threshold, candidate filter, compact (returns at once), rank, ones fix
             else:
                 eng.bh_ws = self.bh_ws
-                eng.qvalues(self.p[:m], self.q[:m], n_tests=self.n_tests, use_hist=True)
-            return
-        if not self.listed:
-            eng.qvalues_global(self.p[:m], self.q[:m], n_tests=self.n_tests, group=self.group, hist=eng.p_hist)
+                eng.qvalues(self.p[:m], self.q[:m], n_tests=self.n_tests)
             return
         # genome-wide: global histogram -> common saturation bucket -> candidates below it -> one fixed-capacity all-gather
         dist.all_reduce(eng.p_hist, op=dist.ReduceOp.SUM, group=self.group)
         cap = self.gather_cap
-        _lib.check(lib.bbk_bh_select_listed(_lib.ptr(self.p), m, self.n_tests, _lib.ptr(eng.p_hist), _lib.ptr(self.q),
-                                            ctypes.byref(self.cands), _lib.ptr(self.score_state),
-                                            ctypes.c_void_p(self.send.data_ptr() + 8), _lib.ptr(self.send_idx), cap,
-                                            _lib.ptr(self.bh_state), _lib.ptr(self.sel_ws), self.sel_ws.numel(), st), "bbk_bh_select_listed")
+        keys = ctypes.c_void_p(self.send.data_ptr() + 8)
+        if self.listed:
+            _lib.check(lib.bbk_bh_select_listed(_lib.ptr(self.p), m, self.n_tests, _lib.ptr(eng.p_hist), _lib.ptr(self.q),
+                                                ctypes.byref(self.cands), _lib.ptr(self.score_state), keys, _lib.ptr(self.send_idx), cap,
+                                                _lib.ptr(self.bh_state), _lib.ptr(self.sel_ws), self.sel_ws.numel(), st), "bbk_bh_select_listed")
+        else:
+            _lib.check(lib.bbk_bh_select(_lib.ptr(self.p), m, self.n_tests, _lib.ptr(eng.p_hist), _lib.ptr(self.q), keys,
+                                         _lib.ptr(self.send_idx), cap, _lib.ptr(self.bh_state), _lib.ptr(self.sel_ws), self.sel_ws.numel(),
+                                         st), "bbk_bh_select")
         _lib.check(lib.bbk_bh_pack_count(_lib.ptr(self.bh_state), _lib.ptr(self.send), st), "bbk_bh_pack_count")
         dist.all_gather_into_tensor(self.recv, self.send, group=self.group)
         _lib.check(lib.bbk_bh_rank_gathered_padded(_lib.ptr(self.recv), self.world, cap, self.rank, _lib.ptr(self.bh_state),
@@ -279,7 +281,8 @@ class GenomePass(object):
                                                    _lib.ptr(self.gather_overflow), _lib.ptr(self.gat_ws), self.gat_ws.numel(), st),
                    "bbk_bh_rank_gathered_padded")
         _lib.check(lib.bbk_bh_fix_ones_dev(_lib.ptr(self.p), m, _lib.ptr(self.q_ones), _lib.ptr(self.q), st), "bbk_bh_fix_ones_dev")
-        eng.launches += 12   # init, threshold, filter, compact, export, pack | prepare, compact, rank, export, scatter | ones fix
+        # init, threshold, [candidate filter], compact, export, pack | prepare, compact, rank, export, scatter | ones fix
+        eng.launches += 12 if self.listed else 11
 
     def read_state(self):
         """(FitResult bytes, ScoreState, gather overflow) after ONE synchronisation."""
@@ -312,7 +315,7 @@ class GenomePass(object):
             if self.listed and score.overflow:
                 self.attach(self.shards, self.p, self.q, list_capacity=max(self.rows, 4))
                 again = True
-            if self.world > 1 and self.q_values and self.listed:
+            if self.world > 1 and self.q_values:
                 flags = torch.tensor([ov, 1 if again else 0, self.rows], dtype=torch.int64, device=self.device)
                 dist.all_reduce(flags, op=dist.ReduceOp.MAX, group=self.group)
                 ov_any, again, max_rows = int(flags[0].item()), bool(int(flags[1].item())), int(flags[2].item())

@@ -1,4 +1,5 @@
-"""Device-side driver of one Fit-Hi-C significance pass (the reference's fithic(), fithic.py:110-133).
+"""Device-side stages of one Fit-Hi-C significance pass (the reference's fithic(), fithic.py:110-133); distributed.GenomePass
+enqueues them.
 
     K1 hist_pairs  ->  [allreduce of the distance table across ranks]  ->  K2/K3 fit (one CTA)
     ->  K4 pvalues  ->  K5 Benjamini-Hochberg q-values (opt-in; the reference writes -1, fithic.py:435)
@@ -243,102 +244,22 @@ class PassEngine(object):
             self.bh_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         return self.bh_ws
 
-    def pvalues(self, shard, p_out, with_hist=False, q_out=None):
-        """K4.  with_hist: also fill self.p_hist (zero it first).  q_out (with with_hist): the hand-over of
-        bbk_pvalues_bh - q pre-filled and the small p listed for qvalues(..., prepared=True) right after."""
+    def pvalues(self, shard, p_out, with_hist=False):
+        """K4.  with_hist: also fill self.p_hist (zero it first)."""
         bias = ctypes.byref(self.bias.struct) if self.bias is not None else None
-        args = (_lib.ptr(shard.chr1), _lib.ptr(shard.chr2), _lib.ptr(shard.mid1), _lib.ptr(shard.mid2),
-                _lib.ptr(shard.count), shard.n, shard.chrom, self.R, self.min_dist, self.max_dist,
-                _lib.ptr(self.fit_result), _lib.ptr(self.spline_y), bias, _lib.ptr(p_out))
-        if q_out is not None:
-            if not with_hist:
-                raise ValueError("the K4 -> K5 hand-over needs the histogram (with_hist=True)")
-            ws = self._bh_workspace(shard.n)
-            _lib.check(self.lib.bbk_pvalues_bh(*args, _lib.ptr(self.p_hist), _lib.ptr(q_out), _lib.ptr(ws), ws.numel(),
-                                               _lib.stream_ptr()), "bbk_pvalues_bh")
-        else:
-            _lib.check(self.lib.bbk_pvalues(*args, _lib.ptr(self.p_hist) if with_hist else None, _lib.stream_ptr()), "bbk_pvalues")
+        _lib.check(self.lib.bbk_pvalues(_lib.ptr(shard.chr1), _lib.ptr(shard.chr2), _lib.ptr(shard.mid1), _lib.ptr(shard.mid2),
+                                        _lib.ptr(shard.count), shard.n, shard.chrom, self.R, self.min_dist, self.max_dist,
+                                        _lib.ptr(self.fit_result), _lib.ptr(self.spline_y), bias, _lib.ptr(p_out),
+                                        _lib.ptr(self.p_hist) if with_hist else None, _lib.stream_ptr()), "bbk_pvalues")
         self.launches += 1
 
-    def qvalues(self, p, q, n_tests=-1, use_hist=False, rank=None, mode=_lib.BH_UNSORTED, prepared=False):
+    def qvalues(self, p, q, n_tests=-1):
+        """K5 over p, with the histogram K4 left in self.p_hist."""
         m = int(p.numel())
         ws = self._bh_workspace(m)
-        if prepared:
-            if rank is not None or mode != _lib.BH_UNSORTED or not use_hist:
-                raise ValueError("prepared q-values: unsorted mode with the K4 histogram, no ranks")
-            _lib.check(self.lib.bbk_bh_qvalues_prepared(_lib.ptr(p), m, int(n_tests), _lib.ptr(self.p_hist), _lib.ptr(q),
-                                                        _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "bbk_bh_qvalues_prepared")
-            self.launches += 6       # init, threshold, list filter, compact (returns at once), rank, ones fix
-            return
-        _lib.check(self.lib.bbk_bh_qvalues(_lib.ptr(p), m, int(n_tests), mode, _lib.ptr(self.p_hist) if use_hist else None,
-                                           _lib.ptr(q), _lib.ptr(rank), _lib.ptr(ws), ws.numel(),
-                                           _lib.stream_ptr()), "bbk_bh_qvalues")
-        # init, [coarse histogram], threshold, compact, rank (one cooperative launch), ones fix
-        self.launches += (4 if mode == _lib.BH_POSITIONAL else 6 - (1 if use_hist else 0))
-
-    def qvalues_global(self, p, q, n_tests=-1, group=None, hist=None, prepared=False):
-        """Genome-wide Benjamini-Hochberg across the ranks of `group`: every rank passes its shard's p and gets
-        the q-values its rows would have if all shards had been ranked together (the reference's q-value step,
-        utils.py:31-90 -> blueberry.pyx:40).  Two collectives: all-reduce of the 4096-bucket p histogram and
-        all-gather of the candidate keys below the common saturation bucket.  `hist`: this shard's coarse
-        histogram when K4 already filled it (self.p_hist), else it is computed here.  prepared: K4 ran with q_out=q
-        (bbk_pvalues_bh), so q is pre-filled and the candidates come from its flag bits.  Synchronises the host once
-        (candidate counts).  With one rank the result equals qvalues() bit for bit."""
-        import torch.distributed as dist
-        lib, dev = self.lib, self.device
-        st = _lib.stream_ptr()
-        m = int(p.numel())
-        world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
-        rank = dist.get_rank(group) if world > 1 else 0
-        if hist is None:
-            hist = torch.zeros(_lib.PHIST_LEN, dtype=torch.int64, device=dev)
-            _lib.check(lib.bbk_p_hist(_lib.ptr(p), m, _lib.ptr(hist), st), "bbk_p_hist")
-        ghist = hist.clone()
-        if world > 1:
-            dist.all_reduce(ghist, op=dist.ReduceOp.SUM, group=group)
-        keys = torch.empty(max(m, 1), dtype=torch.int64, device=dev)
-        idx = torch.empty(max(m, 1), dtype=torch.int32, device=dev)
-        state = torch.zeros(4, dtype=torch.int64, device=dev)
-        if prepared:
-            ws0 = self._bh_workspace(m)          # holds K4's flag bits
-            _lib.check(lib.bbk_bh_select_prepared(_lib.ptr(p), m, int(n_tests), _lib.ptr(ghist), _lib.ptr(q), _lib.ptr(keys),
-                                                  _lib.ptr(idx), _lib.ptr(state), _lib.ptr(ws0), ws0.numel(), st), "bbk_bh_select_prepared")
-        else:
-            ws0 = torch.empty(int(lib.bbk_bh_workspace_bytes(0)), dtype=torch.uint8, device=dev)
-            _lib.check(lib.bbk_bh_select(_lib.ptr(p), m, int(n_tests), _lib.ptr(ghist), _lib.ptr(q), _lib.ptr(keys), _lib.ptr(idx),
-                                         _lib.ptr(state), _lib.ptr(ws0), ws0.numel(), st), "bbk_bh_select")
-        # candidate counts of all ranks with ONE host synchronisation
-        if world > 1:
-            counts_dev = torch.empty(world, dtype=torch.int64, device=dev)
-            dist.all_gather_into_tensor(counts_dev, state[0:1].contiguous(), group=group)
-            all_counts = counts_dev.cpu().tolist()
-        else:
-            all_counts = [int(state[0].item())]
-        n_local = int(all_counts[rank])
-        n_all = int(sum(all_counts))
-        if world > 1:
-            cap = max(max(all_counts), 1)
-            recv = torch.empty(world * cap, dtype=torch.int64, device=dev)
-            dist.all_gather_into_tensor(recv, keys[:cap].contiguous() if cap <= keys.numel() else
-                                        torch.cat([keys, torch.zeros(cap - keys.numel(), dtype=torch.int64, device=dev)]), group=group)
-            keys_all = torch.cat([recv[r * cap:r * cap + c] for r, c in enumerate(all_counts)]) if n_all else \
-                torch.empty(0, dtype=torch.int64, device=dev)
-        else:
-            keys_all = keys[:n_local]
-        q_all = torch.empty(max(n_all, 1), dtype=torch.float64, device=dev)
-        q_ones = torch.zeros(2, dtype=torch.float64, device=dev)
-        need = int(lib.bbk_bh_workspace_bytes(n_all))
-        if self.bh_ws is None or self.bh_ws.numel() < need:
-            self.bh_ws = torch.empty(need, dtype=torch.uint8, device=dev)
-        _lib.check(lib.bbk_bh_rank_gathered(_lib.ptr(keys_all), n_all, _lib.ptr(state), _lib.ptr(q_all), _lib.ptr(q_ones),
-                                            _lib.ptr(self.bh_ws), self.bh_ws.numel(), st), "bbk_bh_rank_gathered")
-        off = int(sum(all_counts[:rank]))
-        if n_local:
-            _lib.check(lib.bbk_bh_scatter(_lib.ptr(q_all[off:off + n_local]), _lib.ptr(idx), n_local, _lib.ptr(q), st), "bbk_bh_scatter")
-        # rare: q of the p == 1.0 group below 1 - decided and applied on the device (no host round trip)
-        _lib.check(lib.bbk_bh_fix_ones_dev(_lib.ptr(p), m, _lib.ptr(q_ones), _lib.ptr(q), st), "bbk_bh_fix_ones_dev")
-        self.launches += 10       # select (4 kernels) + rank_gathered (4) + scatter + ones fix
-        return n_all
+        _lib.check(self.lib.bbk_bh_qvalues(_lib.ptr(p), m, int(n_tests), _lib.BH_UNSORTED, _lib.ptr(self.p_hist), _lib.ptr(q), None,
+                                           _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "bbk_bh_qvalues")
+        self.launches += 5       # init, threshold, compact, rank (one cooperative launch), ones fix
 
     # ------------------------------------------------------------------ results
     @staticmethod
@@ -365,47 +286,10 @@ class PassEngine(object):
         """Copy the fit status back (synchronises) and raise what the reference would raise."""
         return self.decode_fit(self.fit_result.cpu().numpy().tobytes())
 
-    def run_second_pass(self, shards, p_first, p_outs, p_outlier, q_outs=None, n_tests=-1, group=None, smoothing=None):
-        """Refit after outlier removal (BASELINE config 4; definition in include/bbk.h): statistics from the records
-        with first-pass p > p_outlier, then ALL records are scored again with the refitted S and spline."""
-        self.hist_excluding(shards, p_first, p_outlier)
-        self.allreduce_stats(group)
-        self.fit(smoothing)
-        fuse_hist = q_outs is not None and len(shards) == 1
-        if fuse_hist:
-            self.p_hist.zero_()
-        for i, (sh, p) in enumerate(zip(shards, p_outs)):
-            if sh.n:
-                self.pvalues(sh, p, with_hist=fuse_hist, q_out=q_outs[i] if fuse_hist else None)
-        if q_outs is not None:
-            for p, q in zip(p_outs, q_outs):
-                if p.numel():
-                    self.qvalues(p, q, n_tests=n_tests, use_hist=fuse_hist, prepared=fuse_hist)
-
-    def run(self, shards, p_outs, q_outs=None, n_tests=-1, group=None, smoothing=None):
-        """The whole pass over `shards`; p_outs[i] (float64, len shards[i].n) receives the p-values.
-
-        q_outs (optional): per-shard q buffers.  Each shard's q-values are ranked on their own (one Benjamini-Hochberg step
-        and one default N per shard - the per-chromosome result files of datatypes.pyx:26); for ONE ranking over several
-        shards or ranks use distributed.GenomePass, which is what fithic.fit_transform_arrays runs.
-        """
-        self.hist(shards)
-        self.allreduce_stats(group)
-        self.fit(smoothing)
-        fuse_hist = q_outs is not None and len(shards) == 1
-        if fuse_hist:
-            self.p_hist.zero_()
-        for i, (sh, p) in enumerate(zip(shards, p_outs)):
-            if sh.n:
-                self.pvalues(sh, p, with_hist=fuse_hist, q_out=q_outs[i] if fuse_hist else None)
-        if q_outs is not None:
-            for p, q in zip(p_outs, q_outs):
-                if p.numel():
-                    self.qvalues(p, q, n_tests=n_tests, use_hist=fuse_hist, prepared=fuse_hist)
-
 
 class HostPipeline(object):
-    """Successive single-shard passes (one library each) streamed from pinned host memory.
+    """Successive single-shard passes (one library each, a distributed.GenomePass on this GPU alone) streamed from pinned
+    host memory.
 
     A pass cannot start scoring before all of its records are on the device (S and the spline need the whole
     distance table, fithic.py:110-133), so inside one pass the inbound and the outbound copies never overlap.
@@ -419,30 +303,33 @@ class HostPipeline(object):
         pass
 
     def __init__(self, engine, max_pairs, chrom=0, slots=2):
+        from .distributed import GenomePass
         self.eng = engine
         self.chrom = int(chrom)
         self.max_pairs = int(max_pairs)
         dev = engine.device
-        padded = (self.max_pairs + 1) & ~1
+        rows = max((self.max_pairs + 3) & ~3, 4)          # GenomePass.attach: a shard's p / q rows in whole groups of 4
         self.slots = []
         for _ in range(int(slots)):
             s = HostPipeline._Slot()
             s.mid1, s.mid2, s.count = (torch.empty(self.max_pairs, dtype=torch.int32, device=dev) for _ in range(3))
-            s.p, s.q = (torch.empty(padded, dtype=torch.float64, device=dev) for _ in range(2))
+            s.p, s.q = (torch.empty(rows, dtype=torch.float64, device=dev) for _ in range(2))
             s.in_ready, s.run_done, s.out_done = (torch.cuda.Event() for _ in range(3))
             s.fit = torch.zeros_like(engine.fit_result)                      # this pass' BbkFitResult (the engine's is overwritten by the next pass)
             s.h_fit = torch.zeros(engine.fit_result.numel(), dtype=torch.uint8).pin_memory()
             s.index = -1
             self.slots.append(s)
+        # Nothing here synchronises, so nothing would see BbkScoreState.overflow: the deferred list has a place for every row
+        # of a slot (and later attaches keep it, being no larger).
+        self.gp = GenomePass(engine, group=False)
+        self.gp.attach([Shard(s.mid1, s.mid2, s.count, chrom=self.chrom)], s.p, s.q, list_capacity=rows)
         self.s_in, self.s_run, self.s_out = (torch.cuda.Stream(dev) for _ in range(3))
         self.s_run.wait_stream(torch.cuda.current_stream(dev))      # the engine's tables were filled there
         self.submitted = 0
 
-    def submit(self, h_mid1, h_mid2, h_count, h_p, h_q=None, n_tests=-1, run=None):
+    def submit(self, h_mid1, h_mid2, h_count, h_p, h_q=None, n_tests=-1):
         """Enqueue one pass: pinned int32 host columns in, p (and q when h_q is given) back into pinned float64
-        host buffers.  Returns the event that fires when the outputs are on the host.
-        run (optional): callable(shard, p, q) that enqueues the pass on the current stream instead of engine.run -
-        e.g. the multi-GPU sequence with its all-reduce and genome-wide q-values."""
+        host buffers.  Returns the event that fires when the outputs are on the host."""
         n = int(h_mid1.numel())
         if n > self.max_pairs or h_mid2.numel() != n or h_count.numel() != n or h_p.numel() != n:
             raise ValueError("library larger than the pipeline's slots, or columns differ in length")
@@ -460,11 +347,9 @@ class HostPipeline(object):
         self.s_run.wait_event(s.in_ready)
         self.s_run.wait_event(s.out_done)       # this slot's previous p/q have left the device
         with torch.cuda.stream(self.s_run):
-            sh = Shard(s.mid1[:n], s.mid2[:n], s.count[:n], chrom=self.chrom)
-            if run is not None:
-                run(sh, s.p[:n], s.q[:n] if h_q is not None else None)
-            else:
-                self.eng.run([sh], [s.p[:n]], [s.q[:n]] if h_q is not None else None, n_tests=n_tests)
+            self.gp.q_values = h_q is not None
+            self.gp.attach([Shard(s.mid1[:n], s.mid2[:n], s.count[:n], chrom=self.chrom)], s.p, s.q)
+            self.gp.enqueue(n_tests)
             s.fit.copy_(self.eng.fit_result, non_blocking=True)
             s.run_done.record()
         self.s_out.wait_event(s.run_done)

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BBK_VERSION 100 /* 0.1.0 */
+#define BBK_VERSION 200 /* 0.2.0 */
 
 /* error codes */
 #define BBK_OK 0
@@ -167,20 +167,6 @@ int bbk_pvalues(const int32_t* d_chr1, const int32_t* d_chr2, const int32_t* d_m
                 int64_t max_dist, const BbkFitResult* d_fit, const double* d_spline_y, const BbkBiasTable* bias,
                 double* d_p, int64_t* d_p_hist, void* stream);
 
-/* K4 with the hand-over to K5 (one shard whose q-values are wanted, ranked on its own): besides p and the histogram,
- * K4 stores q = 1.0 (NaN where p is NaN) for every record and lists (key, index) of the records with p < 2^-5 inside
- * the q-value workspace.  bbk_bh_qvalues_prepared then ranks from that list - a few MB - instead of re-reading p
- * and re-writing q (16 B/pair); K4 is not bound by DRAM, so the extra 8 B/pair it writes are free.  If the
- * saturation bucket lies at or above 2^-5 (a large share of significant rows) the prepared call falls back to the
- * full pass by itself: results are identical to bbk_pvalues + bbk_bh_qvalues in every case.
- * d_p_hist must be zeroed (all BBK_PHIST_LEN entries) before the call; d_bh_workspace: bbk_bh_workspace_bytes(n_pairs),
- * and it must reach bbk_bh_qvalues_prepared untouched. */
-int bbk_pvalues_bh(const int32_t* d_chr1, const int32_t* d_chr2, const int32_t* d_mid1, const int32_t* d_mid2,
-                   const int32_t* d_count, int64_t n_pairs, int32_t shard_chrom, int64_t resolution, int64_t min_dist,
-                   int64_t max_dist, const BbkFitResult* d_fit, const double* d_spline_y, const BbkBiasTable* bias,
-                   double* d_p, int64_t* d_p_hist, double* d_q, void* d_bh_workspace, size_t workspace_bytes,
-                   void* stream);
-
 /* ---------------------------------------------------------------------------------------------
  * K4 as one streaming pass + a patch pass       replaces the scoring loop of fit_spline, fithic.py:413-435
  *
@@ -301,49 +287,36 @@ int bbk_pack_scores(const double* d_p, const double* d_q, int64_t m, uint32_t* d
 size_t bbk_bh_workspace_bytes(int64_t m);
 int bbk_bh_qvalues(const double* d_p, int64_t m, int64_t n_tests, int32_t mode, const int64_t* d_p_hist,
                    double* d_q, int64_t* d_rank, void* d_workspace, size_t workspace_bytes, void* stream);
-/* after bbk_pvalues_bh on the same d_p / d_p_hist / d_q / workspace: BBK_BH_UNSORTED without ranks */
-int bbk_bh_qvalues_prepared(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist, double* d_q,
-                            void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K5, genome-wide across ranks: the reference's q-value step ranks the p-values of ALL chromosomes
  * together (utils.py:31-90 gathers them per chromosome for blueberry.pyx:40).  Shards live on different
- * GPUs, so the ranking is split around two host-side collectives (NCCL through torch.distributed):
- *   bbk_p_hist (or K4's d_p_hist)  ->  all-reduce(sum) of the histogram
- *   bbk_bh_select        : common saturation bucket from the GLOBAL histogram; writes q = 1.0 / NaN for
+ * GPUs, so the ranking is split around two host-side collectives (NCCL through torch.distributed), with no
+ * candidate count ever reaching the host:
+ *   K4's d_p_hist        ->  all-reduce(sum) of the histogram
+ *   bbk_bh_select[_listed] : common saturation bucket from the GLOBAL histogram; writes q = 1.0 / NaN for
  *                          everything that is not a candidate, candidates' keys / row indices to d_keys /
- *                          d_idx (capacity m), d_state[4] = {n_candidates, tau_key, N, n_ones}
- *   all-gather of the candidate keys (order: rank 0's, rank 1's, ...)
- *   bbk_bh_rank_gathered : sorts the gathered keys, forward running max; d_q_all[i] = q of gathered key i;
- *                          d_q_ones[2] = {q of the p == 1.0 group, 1.0 if it is below 1}
- *   bbk_bh_scatter       : d_q_dst[d_idx[i]] = d_q_src[i] for this rank's slice of d_q_all
- *   bbk_bh_fix_ones      : only when d_q_ones[1] != 0: q = q_ones wherever p == 1.0
- * Workspaces: bbk_bh_workspace_bytes(0) for select, bbk_bh_workspace_bytes(n_all) for rank_gathered.
- * With one rank this reproduces bbk_bh_qvalues bit for bit.
+ *                          d_idx, d_state[4] = {n_candidates, tau_key, N, n_ones}
+ *   bbk_bh_pack_count    : puts n_candidates in front of the keys (d_keys = d_send + 1)
+ *   all-gather of the fixed-capacity blocks (order: rank 0's, rank 1's, ...)
+ *   bbk_bh_rank_gathered_padded : ranks all gathered keys, scatters this rank's q-values back
+ *   bbk_bh_fix_ones_dev  : only when q of the p == 1.0 group is below 1: q = q_ones wherever p == 1.0
+ * Workspace of select: bbk_bh_workspace_bytes(0).  With one rank this reproduces bbk_bh_qvalues bit for bit.
+ * d_keys / d_idx hold keys_capacity entries (a fixed-capacity send block); candidates beyond it are counted in
+ * d_state[0] but not stored - bbk_bh_rank_gathered_padded then reports the overflow.
  * ------------------------------------------------------------------------------------------- */
-int bbk_p_hist(const double* d_p, int64_t m, int64_t* d_p_hist, void* stream);
 int bbk_bh_select(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
-                  uint64_t* d_keys, uint32_t* d_idx, uint64_t* d_state, void* d_workspace, size_t workspace_bytes,
-                  void* stream);
-/* bbk_bh_select after bbk_pvalues_bh on the same d_p / d_q: q is already pre-filled and the candidates come from K4's flag
- * bits (d_workspace = the workspace given to bbk_pvalues_bh, untouched since); falls back to the full pass by itself when the
- * GLOBAL saturation bucket lies at or above 2^-5.  Same outputs as bbk_bh_select. */
-int bbk_bh_select_prepared(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
-                           uint64_t* d_keys, uint32_t* d_idx, uint64_t* d_state, void* d_workspace, size_t workspace_bytes,
-                           void* stream);
-int bbk_bh_rank_gathered(const uint64_t* d_keys_all, int64_t n_all, const uint64_t* d_state, double* d_q_all,
-                         double* d_q_ones, void* d_workspace, size_t workspace_bytes, void* stream);
-int bbk_bh_scatter(const double* d_q_src, const uint32_t* d_idx, int64_t n, double* d_q_dst, void* stream);
-int bbk_bh_fix_ones(const double* d_p, int64_t m, double q_ones, double* d_q, void* stream);
-/* the same, decided on the device from d_q_ones[2] of bbk_bh_rank_gathered (no host round trip) */
+                  uint64_t* d_keys, uint32_t* d_idx, int64_t keys_capacity, uint64_t* d_state, void* d_workspace,
+                  size_t workspace_bytes, void* stream);
+/* q = d_q_ones[0] wherever p == 1.0, decided on the device from d_q_ones[2] of bbk_bh_rank_gathered_padded (nothing to do
+ * when d_q_ones[1] == 0) */
 int bbk_bh_fix_ones_dev(const double* d_p, int64_t m, const double* d_q_ones, double* d_q, void* stream);
 
-/* listed mode: after bbk_pvalues_listed on the same d_p / d_p_hist / d_q, ranking from its candidate list */
+/* listed mode: after bbk_score_pairs / bbk_score_deferred on the same d_p / d_p_hist / d_q, ranking from their candidate list */
 int bbk_bh_qvalues_listed(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist, double* d_q,
                           const BbkCandidates* cands, const BbkScoreState* d_state, void* d_workspace, size_t workspace_bytes,
                           void* stream);
-/* d_keys / d_idx hold keys_capacity entries (a fixed-capacity send block); candidates beyond it are counted in d_state[0] but
- * not stored - bbk_bh_rank_gathered_padded then reports the overflow */
+/* bbk_bh_select from that candidate list */
 int bbk_bh_select_listed(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
                          const BbkCandidates* cands, const BbkScoreState* d_score, uint64_t* d_keys, uint32_t* d_idx,
                          int64_t keys_capacity, uint64_t* d_state, void* d_workspace, size_t workspace_bytes, void* stream);
@@ -351,10 +324,10 @@ int bbk_bh_select_listed(const double* d_p, int64_t m, int64_t n_tests, const in
 /* Genome-wide ranking with the gather left on the device (no candidate count ever reaches the host): every rank sends a
  * fixed-capacity block [count | keys[0 .. cap)] - d_keys of bbk_bh_select* written at send + 1, the count put in front by
  * bbk_bh_pack_count - and one all-gather delivers `world` such blocks (d_recv: world * (cap + 1) u64).
- * bbk_bh_rank_gathered_padded prefixes the counts, compacts the blocks, ranks them (forward running max, as
- * bbk_bh_rank_gathered) and scatters THIS rank's slice back: d_q_dst[d_idx_local[i]] = q of this rank's candidate i.
+ * bbk_bh_rank_gathered_padded prefixes the counts, compacts the blocks, ranks them (forward running max) and scatters
+ * THIS rank's slice back: d_q_dst[d_idx_local[i]] = q of this rank's candidate i.
  * A count above cap puts the largest count of any rank into *d_overflow (int32, never cleared here); the host checks it when it reads the results and repeats
- * the q-value step with a larger capacity.  d_q_ones[2] as bbk_bh_rank_gathered.  Workspace:
+ * the q-value step with a larger capacity.  d_q_ones[2] = {q of the p == 1.0 group, 1.0 if it is below 1}.  Workspace:
  * bbk_bh_gathered_workspace_bytes(world, cap). */
 size_t bbk_bh_gathered_workspace_bytes(int32_t world, int64_t cap);
 int bbk_bh_pack_count(const uint64_t* d_state, uint64_t* d_send, void* stream);

@@ -34,11 +34,11 @@ def test_library_exports_every_declared_symbol(lib):
         assert hasattr(lib, name), "libbbk.so does not export %s" % name
 
 
-def test_ctypes_signatures_cover_the_header(lib):
+def test_ctypes_signatures_and_version_match_the_header(lib):
     from blueberry_b200 import _lib
     assert sorted(_lib.SIGNATURES) == _declared_functions()
     lib.bbk_version.restype = ctypes.c_int
-    assert lib.bbk_version() == 100
+    assert lib.bbk_version() == 200
 
 
 def test_fit_result_struct_matches_header():

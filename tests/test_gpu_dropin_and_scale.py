@@ -87,10 +87,11 @@ def test_stage_functions_drop_in(tmp_path):
     assert ok, nbad
 
 
-def test_full_size_properties_config2():
+def test_full_size_properties_config2_genome_pass():
     """BASELINE config 2 (chr1 @ 5 kb, 97,750,851 records) generated on the device: properties that need no oracle."""
     import torch
     from blueberry_b200 import _lib
+    from blueberry_b200.distributed import GenomePass
     from blueberry_b200.engine import BiasTables, PassEngine, Shard
     lib = _lib.load()
     dev = torch.device("cuda:0")
@@ -108,9 +109,10 @@ def test_full_size_properties_config2():
     eng = PassEngine(R, 100, 0, max_dist, nb, dev)
     eng.set_fragments([nb], [(nb - 1) * R])
     eng.set_bias(BiasTables([np.where((bias_host < 0.5) | (bias_host > 2), -1.0, bias_host)], [R // 2], dev))
-    p = torch.empty(P + 1, dtype=torch.float64, device=dev)[:P]
-    q = torch.empty(P + 1, dtype=torch.float64, device=dev)[:P]
-    eng.run([Shard(mid1, mid2, count)], [p], [q])
+    gp = GenomePass(eng, group=False)
+    gp.attach([Shard(mid1, mid2, count)])
+    gp.run()
+    p, q = gp.shard_p(0), gp.shard_q(0)
     fit = eng.read_fit()
     d = (mid2 - mid1).long()
     # K1: a checksum of checksums - the table must hold exactly the in-range counts, distance by distance
@@ -273,11 +275,12 @@ def test_bias_loci_off_the_fragment_grid(shift):
     assert len(np.unique(ref.p[np.isin(m2, bm[moved])])) > 1    # the moved loci were really used
 
 
-def test_host_pipeline_matches_serial_passes():
+def test_host_pipeline_matches_serial_genome_passes():
     """engine.HostPipeline: five different libraries (different sizes and seeds) streamed through two device slots
     give bit-for-bit the p and q of the same libraries run one at a time on the default stream."""
     import torch
     from blueberry_b200 import _lib
+    from blueberry_b200.distributed import GenomePass
     from blueberry_b200.engine import BiasTables, HostPipeline, PassEngine, Shard
     lib = _lib.load()
     dev = torch.device("cuda:0")
@@ -296,11 +299,11 @@ def test_host_pipeline_matches_serial_passes():
                                           _lib.ptr(cols[1]), _lib.ptr(cols[2]), _lib.stream_ptr()), "synth")
         n = P - 1000 * i - (i & 1)                    # ragged sizes, odd and even
         cols = [c[:n].contiguous() for c in cols]
-        p = torch.empty(n + 1, dtype=torch.float64, device=dev)[:n]
-        q = torch.empty(n + 1, dtype=torch.float64, device=dev)[:n]
-        eng.run([Shard(*cols)], [p], [q])
+        gp = GenomePass(eng, group=False)
+        gp.attach([Shard(*cols)])
+        gp.run()
         fit = eng.read_fit()
-        want.append((p.cpu(), q.cpu(), (fit.S, fit.n_knots, fit.smoothing, fit.y_min)))
+        want.append((gp.shard_p(0).cpu(), gp.shard_q(0).cpu(), (fit.S, fit.n_knots, fit.smoothing, fit.y_min)))
         libs.append([c.cpu().pin_memory() for c in cols])
     torch.cuda.synchronize()
     pipe = HostPipeline(eng, P, slots=2)
@@ -334,57 +337,6 @@ def test_host_pipeline_matches_serial_passes():
     assert torch.equal(outs[1][0].view(torch.int64), want[1][0].view(torch.int64))
     with pytest.raises(ValueError):
         pipe.submit(libs[0][0], libs[0][1], libs[0][2], torch.empty(libs[0][0].numel(), dtype=torch.float64))
-
-
-@pytest.mark.parametrize("n_tests", [-1, 25])
-def test_k4_handover_matches_two_pass_qvalues(n_tests):
-    """bbk_pvalues_bh + bbk_bh_qvalues_prepared (K4 pre-fills q and lists the small p) against bbk_pvalues +
-    bbk_bh_qvalues, bit for bit.  n_tests = 25 pushes the saturation bucket above 2^-5, so the prepared call has
-    to fall back to the full pass on its own (and q of the p == 1.0 rows drops below 1)."""
-    import torch
-    from blueberry_b200 import _lib
-    from blueberry_b200.engine import BiasTables, PassEngine, Shard
-    lib = _lib.load()
-    dev = torch.device("cuda:0")
-    R, nb, K = 5000, 7001, 300
-    P = int(lib.bbk_synth_n_pairs(nb, K))
-    assert P % 4 != 0                                 # the last records go through the tail kernel
-    rng = np.random.default_rng(9)
-    bias_host = np.exp(rng.normal(0.0, 0.25, size=nb))
-    bias_dev = torch.from_numpy(bias_host).to(dev)
-    cols = [torch.empty(P, dtype=torch.int32, device=dev) for _ in range(3)]
-    _lib.check(lib.bbk_synth_contacts(nb, K, R, 120.0, 1.08, 77, _lib.ptr(bias_dev), _lib.ptr(cols[0]), _lib.ptr(cols[1]),
-                                      _lib.ptr(cols[2]), _lib.stream_ptr()), "synth")
-    eng = PassEngine(R, 100, 0, K * R, nb, dev)
-    eng.set_fragments([nb], [(nb - 1) * R])
-    eng.set_bias(BiasTables([np.where((bias_host < 0.5) | (bias_host > 2), -1.0, bias_host)], [R // 2], dev))
-    sh = Shard(*cols)
-    eng.hist([sh]); eng.allreduce_stats(None); eng.fit()
-    p0, q0, p1, q1 = (torch.empty(P + 3, dtype=torch.float64, device=dev)[:P] for _ in range(4))
-    eng.p_hist.zero_()
-    eng.pvalues(sh, p0, with_hist=True)
-    eng.qvalues(p0, q0, n_tests=n_tests, use_hist=True)
-    hist0 = eng.p_hist.clone()
-    eng.p_hist.zero_()
-    q1.fill_(-7.0)
-    eng.pvalues(sh, p1, with_hist=True, q_out=q1)
-    eng.qvalues(p1, q1, n_tests=n_tests, use_hist=True, prepared=True)
-    torch.cuda.synchronize()
-    assert torch.equal(p0.view(torch.int64), p1.view(torch.int64))
-    assert torch.equal(hist0[:4098], eng.p_hist[:4098])
-    assert torch.equal(q0.view(torch.int64), q1.view(torch.int64))
-    use_list = int(eng.bh_ws[100:104].view(torch.int32)[0])
-    # the genome-wide (multi-GPU) pipeline with one rank, fed by the same hand-over
-    q2 = torch.full((P + 3,), -7.0, dtype=torch.float64, device=dev)[:P]
-    eng.p_hist.zero_()
-    eng.pvalues(sh, p1, with_hist=True, q_out=q2)
-    eng.qvalues_global(p1, q2, n_tests=n_tests, hist=eng.p_hist, prepared=True)
-    torch.cuda.synchronize()
-    assert torch.equal(q0.view(torch.int64), q2.view(torch.int64))
-    assert use_list == (1 if n_tests < 0 else 0)
-    if n_tests > 0:
-        assert float(q1[p1 == 1.0][0]) < 1.0
-    assert int((q1 < 1.0).sum()) > 1000
 
 
 def test_decimate_matches_reference_golden_and_oracle(tmp_path):

@@ -435,6 +435,47 @@ def test_list_overflow_is_detected_and_repaired():
     assert _same(gp.q.cpu().numpy()[:gp.rows], _bh_of(gp.p.cpu().numpy()[:gp.rows]))     # the candidate overflow falls back to the full pass: still exact
 
 
+@pytest.mark.parametrize("n_tests", [-1, 25])
+def test_k4_handover_matches_two_pass_qvalues(n_tests):
+    """The streaming K4's hand-over to K5 (q pre-filled, the small p listed, bbk_bh_qvalues_listed) against bbk_bh_qvalues on
+    the pass's own p, bit for bit.  n_tests = 25 pushes the saturation bucket above 2^-5, so the listed call has to fall back
+    to the full pass on its own (and q of the p == 1.0 rows drops below 1)."""
+    import torch
+    from blueberry_b200 import _lib
+    from blueberry_b200.distributed import GenomePass
+    from blueberry_b200.engine import BiasTables, PassEngine, Shard
+    lib = _lib.load()
+    dev = torch.device("cuda:0")
+    R, nb, K = 5000, 7001, 300
+    P = int(lib.bbk_synth_n_pairs(nb, K))
+    assert P % 4 != 0                                 # the shard ends inside a group of four rows
+    rng = np.random.default_rng(9)
+    bias_host = np.exp(rng.normal(0.0, 0.25, size=nb))
+    bias_dev = torch.from_numpy(bias_host).to(dev)
+    cols = [torch.empty(P, dtype=torch.int32, device=dev) for _ in range(3)]
+    _lib.check(lib.bbk_synth_contacts(nb, K, R, 120.0, 1.08, 77, _lib.ptr(bias_dev), _lib.ptr(cols[0]), _lib.ptr(cols[1]),
+                                      _lib.ptr(cols[2]), _lib.stream_ptr()), "synth")
+    eng = PassEngine(R, 100, 0, K * R, nb, dev)
+    eng.set_fragments([nb], [(nb - 1) * R])
+    eng.set_bias(BiasTables([np.where((bias_host < 0.5) | (bias_host > 2), -1.0, bias_host)], [R // 2], dev))
+    gp = GenomePass(eng, group=False, q_values=True)
+    gp.attach([Shard(*cols)])
+    assert gp.listed
+    gp.run(n_tests=n_tests)
+    use_list = int(gp.bh_ws[100:104].view(torch.int32)[0])          # BhState::use_list of the q-value step
+    p1, q1 = gp.shard_p(0), gp.shard_q(0)
+    q0 = torch.full((P + 3,), -7.0, dtype=torch.float64, device=dev)[:P]
+    ws = torch.empty(int(lib.bbk_bh_workspace_bytes(P)), dtype=torch.uint8, device=dev)
+    _lib.check(lib.bbk_bh_qvalues(_lib.ptr(p1), P, n_tests, _lib.BH_UNSORTED, None, _lib.ptr(q0), None, _lib.ptr(ws), ws.numel(),
+                                  _lib.stream_ptr()), "bbk_bh_qvalues")
+    torch.cuda.synchronize()
+    assert torch.equal(q0.view(torch.int64), q1.view(torch.int64))
+    assert use_list == (1 if n_tests < 0 else 0)
+    if n_tests > 0:
+        assert float(q1[p1 == 1.0][0]) < 1.0
+    assert int((q1 < 1.0).sum()) > 1000
+
+
 def test_fit_transform_arrays_pinned_and_wide_inputs():
     """The drop-in array call: pinned int32 torch columns, int64 numpy columns and a value beyond int32 (OverflowError)."""
     import torch

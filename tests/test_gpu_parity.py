@@ -348,26 +348,57 @@ def test_error_behaviour_matches_reference(torch_cuda):
 
 
 @pytest.mark.parametrize("m,frac_ones,n_scale", [(300_001, 0.6, 1.0), (300_001, 0.3, 0.01), (50_000, 0.0, 40.0)])
-def test_bh_genome_wide_path_single_rank_equals_local(m, frac_ones, n_scale, torch_cuda):
-    """The split select / gather / rank / scatter pipeline used across GPUs, run with one rank, against the oracle."""
-    from blueberry_b200.engine import PassEngine
+def test_bh_fixed_capacity_gather_single_rank_equals_local(m, frac_ones, n_scale, torch_cuda):
+    """The select / fixed-capacity gather / rank / scatter pipeline used across GPUs, run with one rank (the all-gather then
+    delivers the send block itself), against the oracle; then with a capacity below the candidate count, which must be
+    reported."""
+    import ctypes
+    from blueberry_b200 import _lib
     from oracle import fithic_oracle as fo
     torch = torch_cuda
+    lib = _lib.load()
+    dev = torch.device("cuda:0")
     rng = np.random.default_rng(m + 3)
     p = rng.random(m) ** 3
     p[rng.random(m) < frac_ones] = 1.0
     p[rng.integers(0, m, m // 10)] = p[rng.integers(0, m, m // 10)]
     p[rng.integers(0, m, m // 50)] = np.nan
     n_tests = max(1, int(m * n_scale))
-    eng = PassEngine(1, 100, 0, 10, 16, torch.device("cuda:0"))
-    dp = torch.empty((m + 1) & ~1, dtype=torch.float64, device="cuda:0")[:m].copy_(torch.from_numpy(p))
-    dq = torch.full(((m + 1) & ~1,), -7.0, dtype=torch.float64, device="cuda:0")[:m]
-    eng.qvalues_global(dp, dq, n_tests=n_tests)
-    torch.cuda.synchronize()
+    dp = torch.empty((m + 1) & ~1, dtype=torch.float64, device=dev)[:m].copy_(torch.from_numpy(p))
+    dq = torch.full(((m + 1) & ~1,), -7.0, dtype=torch.float64, device=dev)[:m]
+    # K4's coarse histogram: bucket (bits >> 51) & 4095 of a p in [0, 1), p == 1.0 in slot 4096, NaN in slot 4097
+    nan, one = torch.isnan(dp), dp == 1.0
+    hist = torch.zeros(_lib.PHIST_LEN, dtype=torch.int64, device=dev)
+    hist[:_lib.PHIST_BINS] = torch.bincount(((dp.view(torch.int64) >> 51) & 4095)[~nan & ~one], minlength=_lib.PHIST_BINS)
+    hist[_lib.PHIST_BINS] = one.sum()
+    hist[_lib.PHIST_BINS + 1] = nan.sum()
+    st = _lib.stream_ptr()
+
+    def gathered(cap):
+        send = torch.zeros(cap + 1, dtype=torch.int64, device=dev)
+        idx = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+        state = torch.zeros(4, dtype=torch.int64, device=dev)
+        q_ones = torch.zeros(2, dtype=torch.float64, device=dev)
+        overflow = torch.zeros(1, dtype=torch.int32, device=dev)
+        sel_ws = torch.empty(int(lib.bbk_bh_workspace_bytes(0)), dtype=torch.uint8, device=dev)
+        gat_ws = torch.empty(int(lib.bbk_bh_gathered_workspace_bytes(1, cap)), dtype=torch.uint8, device=dev)
+        _lib.check(lib.bbk_bh_select(_lib.ptr(dp), m, n_tests, _lib.ptr(hist), _lib.ptr(dq), ctypes.c_void_p(send.data_ptr() + 8),
+                                     _lib.ptr(idx), cap, _lib.ptr(state), _lib.ptr(sel_ws), sel_ws.numel(), st), "bbk_bh_select")
+        _lib.check(lib.bbk_bh_pack_count(_lib.ptr(state), _lib.ptr(send), st), "bbk_bh_pack_count")
+        recv = send
+        _lib.check(lib.bbk_bh_rank_gathered_padded(_lib.ptr(recv), 1, cap, 0, _lib.ptr(state), _lib.ptr(idx), _lib.ptr(dq), _lib.ptr(q_ones),
+                                                   _lib.ptr(overflow), _lib.ptr(gat_ws), gat_ws.numel(), st), "bbk_bh_rank_gathered_padded")
+        _lib.check(lib.bbk_bh_fix_ones_dev(_lib.ptr(dp), m, _lib.ptr(q_ones), _lib.ptr(dq), st), "bbk_bh_fix_ones_dev")
+        torch.cuda.synchronize()
+        return int(state[0].item()), int(overflow.item())
+
+    n_cand, ov = gathered(m)
     q = dq.cpu().numpy()
     valid = ~np.isnan(p)
     assert np.isnan(q[~valid]).all()
     assert np.array_equal(q[valid], fo.benjamini_hochberg_correction(p[valid], n_tests))
+    assert ov == 0 and n_cand > 0
+    assert gathered(n_cand - 1) == (n_cand, n_cand)
 
 
 def test_second_pass_against_composed_reference_golden(torch_cuda):
