@@ -259,8 +259,9 @@ class GenomePass(object):
                                                      self.bh_ws.numel(), st), "bbk_bh_qvalues_listed")
                 eng.launches += 6          # init, threshold, candidate filter, compact (returns at once), rank, ones fix
             else:
-                eng.bh_ws = self.bh_ws
-                eng.qvalues(self.p[:m], self.q[:m], n_tests=self.n_tests)
+                _lib.check(lib.bbk_bh_qvalues(_lib.ptr(self.p), m, self.n_tests, _lib.BH_UNSORTED, _lib.ptr(eng.p_hist), _lib.ptr(self.q),
+                                              None, _lib.ptr(self.bh_ws), self.bh_ws.numel(), st), "bbk_bh_qvalues")
+                eng.launches += 5          # init, threshold, compact, rank (one cooperative launch), ones fix
             return
         # genome-wide: global histogram -> common saturation bucket -> candidates below it -> one fixed-capacity all-gather
         dist.all_reduce(eng.p_hist, op=dist.ReduceOp.SUM, group=self.group)
@@ -352,13 +353,15 @@ class HostStream(object):
         pass
 
     def __init__(self, genome_pass, sizes, chroms, slots=2, packed=False, cap_p=None, cap_q=None):
-        """packed: results cross the host link as two bits per row + the values that are not 1.0 / NaN (bbk_pack_scores);
+        """sizes / chroms: records and chromosome of every shard; the slots hold layout_rows(sizes) rows.
+        packed: results cross the host link as two bits per row + the values that are not 1.0 / NaN (bbk_pack_scores);
         submit_packed() returns a PackedScores whose dense() rebuilds the float64 columns bit for bit.  cap_p / cap_q: rows
         the packed value lists can hold (default rows / 2 and rows / 16; a pass that needs more comes back dense)."""
         self.gp = genome_pass
         self.sizes, self.chroms = [int(x) for x in sizes], [int(x) for x in chroms]
-        self.starts = layout_rows(self.sizes)[0]
-        self.rows = max(layout_rows(self.sizes)[1], 4)
+        self.starts, rows = layout_rows(self.sizes)
+        self.rows = max(rows, 4)
+        self.packed = bool(packed)
         dev = genome_pass.device
         self.slots = []
         for _ in range(int(slots)):
@@ -366,105 +369,98 @@ class HostStream(object):
             s.mid1, s.mid2, s.count = (torch.empty(self.rows, dtype=torch.int32, device=dev) for _ in range(3))
             s.p = torch.full((self.rows,), float("nan"), dtype=torch.float64, device=dev)
             s.q = torch.full((self.rows,), float("nan"), dtype=torch.float64, device=dev) if genome_pass.q_values else None
-            s.shards = [Shard(s.mid1[a:a + n], s.mid2[a:a + n], s.count[a:a + n], chrom=c)
-                        for a, n, c in zip(self.starts, self.sizes, self.chroms)]
-            s.in_ready, s.run_done, s.out_done = (torch.cuda.Event() for _ in range(3))
+            s.shards = self._shards(s, self.starts, self.sizes)
+            s.in_ready, s.run_done, s.out_done, s.counts_ready = (torch.cuda.Event() for _ in range(4))
             s.fit = torch.zeros_like(genome_pass.eng.fit_result)
             s.h_fit = torch.zeros(genome_pass.eng.fit_result.numel(), dtype=torch.uint8).pin_memory()
+            if self.packed:
+                s.pack = DevicePack(self.rows, dev, genome_pass.q_values, cap_p, cap_q)
+                s.h_pack_state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8).pin_memory()
             s.index = -1
             self.slots.append(s)
+        # Nothing here synchronises, so nothing would see BbkScoreState.overflow: the deferred list has a place for every row
+        # of a slot (and later attaches keep it, being no larger).
+        genome_pass.attach(s.shards, s.p, s.q, list_capacity=self.rows)
         self.s_in, self.s_run, self.s_out = (torch.cuda.Stream(dev) for _ in range(3))
         self.s_run.wait_stream(torch.cuda.current_stream(dev))
         self.submitted = 0
-        self.packed = bool(packed)
         self._pending = None
-        if self.packed:
-            lib = genome_pass.lib
-            self.cap_p = int(cap_p) if cap_p else max(self.rows // 2, 1024)
-            self.cap_q = int(cap_q) if cap_q else max(self.rows // 16, 1024)
-            self.n_words, self.n_chunks = int(lib.bbk_pack_code_words(self.rows)), int(lib.bbk_pack_chunks(self.rows))
-            for s in self.slots:
-                s.codes = torch.empty(self.n_words, dtype=torch.int32, device=dev)
-                s.chunks = torch.empty(self.n_chunks * 24, dtype=torch.uint8, device=dev)
-                s.vals_p = torch.empty(self.cap_p, dtype=torch.float64, device=dev)
-                s.vals_q = torch.empty(self.cap_q, dtype=torch.float64, device=dev) if genome_pass.q_values else None
-                s.pack_state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8, device=dev)
-                s.h_pack_state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8).pin_memory()
-                s.counts_ready = torch.cuda.Event()
 
-    def submit(self, h_mid1, h_mid2, h_count, h_p, h_q=None, n_tests=-1):
-        """Enqueue one pass over the host table; returns the event that fires when p (and q) are on the host."""
-        for t in (h_mid1, h_mid2, h_count, h_p, h_q):
-            if t is not None and (not t.is_pinned() or t.numel() < self.rows):
-                raise ValueError("host columns must be pinned and hold at least %d rows" % self.rows)
+    def _shards(self, s, starts, sizes):
+        return [Shard(s.mid1[a:a + n], s.mid2[a:a + n], s.count[a:a + n], chrom=c) for a, n, c in zip(starts, sizes, self.chroms)]
+
+    def _run(self, h_mid1, h_mid2, h_count, h_out, n_tests, sizes, q_values, pack=False):
+        """What submit() and submit_packed() share: check the host columns, copy the records into the next slot (stream in)
+        and run the pass there (stream run), packing p / q after it when `pack`.  Returns (slot, rows the pass covers)."""
         s = self.slots[self.submitted % len(self.slots)]
+        sizes = self.sizes if sizes is None else [int(x) for x in sizes]
+        starts, rows = layout_rows(sizes)
+        if len(sizes) != len(self.chroms) or rows > self.rows:
+            raise ValueError("sizes must give one shard per chromosome of the stream and fit its %d rows" % self.rows)
+        n = starts[-1] + sizes[-1] if sizes else 0
+        for t in (h_mid1, h_mid2, h_count) + h_out:
+            if t is not None and (not t.is_pinned() or t.numel() < n):
+                raise ValueError("host columns must be pinned and hold at least %d rows" % n)
+        if q_values and s.q is None:
+            raise ValueError("the stream's GenomePass was made with q_values=False")
+        shards = s.shards if sizes is self.sizes else self._shards(s, starts, sizes)
         self.submitted += 1
-        n = self.rows
+        s.index = self.submitted - 1
         self.s_in.wait_event(s.run_done)        # the pass that last read this slot's records has finished
         with torch.cuda.stream(self.s_in):
-            s.mid1.copy_(h_mid1[:n], non_blocking=True)
-            s.mid2.copy_(h_mid2[:n], non_blocking=True)
-            s.count.copy_(h_count[:n], non_blocking=True)
+            s.mid1[:n].copy_(h_mid1[:n], non_blocking=True)
+            s.mid2[:n].copy_(h_mid2[:n], non_blocking=True)
+            s.count[:n].copy_(h_count[:n], non_blocking=True)
             s.in_ready.record()
+        # the previous packed pass' value lists: their sizes are on the host by now (or soon); their copies overlap these inbound ones
+        self._finalize_pending()
         self.s_run.wait_event(s.in_ready)
         self.s_run.wait_event(s.out_done)       # this slot's previous p / q have left the device
+        gp = self.gp
         with torch.cuda.stream(self.s_run):
-            self.gp.attach(s.shards, s.p, s.q)
-            self.gp.enqueue(n_tests)
-            s.fit.copy_(self.gp.eng.fit_result, non_blocking=True)
+            keep_q, gp.q_values = gp.q_values, q_values
+            gp.attach(shards, s.p, s.q)
+            gp.enqueue(n_tests)
+            gp.q_values = keep_q
+            s.fit.copy_(gp.eng.fit_result, non_blocking=True)
+            if pack:
+                s.pack.pack(s.p, s.q, self.s_run)
+                gp.eng.launches += 2
             s.run_done.record()
+        return s, n
+
+    def submit(self, h_mid1, h_mid2, h_count, h_p, h_q=None, n_tests=-1, sizes=None):
+        """Enqueue one pass over the host table; returns the event that fires when p (and q) are on the host.
+        sizes: this pass' shard sizes, one per chromosome of the stream (default: the sizes it was made with); their
+        layout_rows total must fit the slots.  The host columns hold at least the rows the pass covers (up to the end of its
+        last shard), and exactly those rows come back.  Without h_q the pass skips the q-value step; at N > 1 that step is
+        collective, so every rank must pass or omit h_q alike."""
+        s, n = self._run(h_mid1, h_mid2, h_count, (h_p, h_q), n_tests, sizes, h_q is not None)
         self.s_out.wait_event(s.run_done)
         with torch.cuda.stream(self.s_out):
-            h_p[:n].copy_(s.p, non_blocking=True)
-            if h_q is not None and s.q is not None:
-                h_q[:n].copy_(s.q, non_blocking=True)
+            h_p[:n].copy_(s.p[:n], non_blocking=True)
+            if h_q is not None:
+                h_q[:n].copy_(s.q[:n], non_blocking=True)
             s.h_fit.copy_(s.fit, non_blocking=True)
             s.out_done.record()
-        s.index = self.submitted - 1
         return s.out_done
 
     # ------------------------------------------------------------------ packed results
     def submit_packed(self, h_mid1, h_mid2, h_count, out, n_tests=-1):
         """Like submit(), but p / q come back packed into `out` (a PackedScores made by packed_buffers()).  The sizes of the two
-        value lists are only known once the pass has run, so their copies are issued lazily: by the NEXT submit_packed() (after
+        value lists are only known once the pass has run, so their copies are issued lazily: by the NEXT submission (after
         it has put its own inbound copies on the wire) or by drain().  Returns `out`; out.done fires when it is complete."""
         if not self.packed:
             raise ValueError("this stream was not created with packed=True")
-        for t in (h_mid1, h_mid2, h_count):
-            if not t.is_pinned() or t.numel() < self.rows:
-                raise ValueError("host columns must be pinned and hold at least %d rows" % self.rows)
-        s = self.slots[self.submitted % len(self.slots)]
-        self.submitted += 1
-        n = self.rows
-        gp = self.gp
-        self.s_in.wait_event(s.run_done)
-        with torch.cuda.stream(self.s_in):
-            s.mid1.copy_(h_mid1[:n], non_blocking=True)
-            s.mid2.copy_(h_mid2[:n], non_blocking=True)
-            s.count.copy_(h_count[:n], non_blocking=True)
-            s.in_ready.record()
-        # the previous pass' value lists: their sizes are on the host by now (or soon); their copies overlap this pass' inbound ones
-        self._finalize_pending()
-        self.s_run.wait_event(s.in_ready)
-        self.s_run.wait_event(s.out_done)
-        with torch.cuda.stream(self.s_run):
-            gp.attach(s.shards, s.p, s.q)
-            gp.enqueue(n_tests)
-            s.fit.copy_(gp.eng.fit_result, non_blocking=True)
-            _lib.check(gp.lib.bbk_pack_scores(_lib.ptr(s.p), _lib.ptr(s.q), n, _lib.ptr(s.codes), _lib.ptr(s.chunks), _lib.ptr(s.vals_p),
-                                              self.cap_p, _lib.ptr(s.vals_q), self.cap_q if s.vals_q is not None else 0,
-                                              _lib.ptr(s.pack_state), _lib.stream_ptr(self.s_run)), "bbk_pack_scores")
-            gp.eng.launches += 2
-            s.run_done.record()
+        s, _ = self._run(h_mid1, h_mid2, h_count, (), n_tests, None, self.gp.q_values, pack=True)
         self.s_out.wait_event(s.run_done)
         with torch.cuda.stream(self.s_out):
-            s.h_pack_state.copy_(s.pack_state, non_blocking=True)
+            s.h_pack_state.copy_(s.pack.state, non_blocking=True)
             s.counts_ready.record()
-            out.codes.copy_(s.codes, non_blocking=True)
-            out.chunks.copy_(s.chunks, non_blocking=True)
+            out.codes.copy_(s.pack.codes, non_blocking=True)
+            out.chunks.copy_(s.pack.chunks, non_blocking=True)
             s.h_fit.copy_(s.fit, non_blocking=True)
-        s.index = self.submitted - 1
-        out.rows, out.want_q = n, s.q is not None
+        out.rows, out.want_q = self.rows, s.q is not None
         out.done = None
         self._pending = (s, out)
         return out
@@ -486,19 +482,21 @@ class HostStream(object):
                     out.dense_q.copy_(s.q, non_blocking=True)
             else:
                 if out.n_p:
-                    out.vals_p[:out.n_p].copy_(s.vals_p[:out.n_p], non_blocking=True)
-                if out.n_q and s.vals_q is not None:
-                    out.vals_q[:out.n_q].copy_(s.vals_q[:out.n_q], non_blocking=True)
+                    out.vals_p[:out.n_p].copy_(s.pack.vals_p[:out.n_p], non_blocking=True)
+                if out.n_q and s.pack.vals_q is not None:
+                    out.vals_q[:out.n_q].copy_(s.pack.vals_q[:out.n_q], non_blocking=True)
             s.out_done.record()
         out.done = s.out_done
 
     def packed_buffers(self):
         """Pinned host buffers for one packed result."""
-        return PackedScores(self.rows, self.n_words, self.n_chunks, self.cap_p, self.cap_q if self.gp.q_values else 0)
+        pk = self.slots[0].pack
+        return PackedScores(self.rows, pk.codes.numel(), pk.chunks.numel() // 24, pk.cap_p, pk.cap_q)
 
     def fit_of(self, index):
         """Fit result of submission `index` once its outputs are on the host (raises the reference's exception for a failed
-        fit); PassEngine.reference_smoothing(result) tells whether that pass must be repeated with the reference's own s."""
+        fit); PassEngine.reference_smoothing(result) tells whether that pass must be repeated with the reference's own s.
+        Only the last `slots` submissions are held."""
         s = self.slots[int(index) % len(self.slots)]
         if s.index != int(index):
             raise KeyError("submission %d is no longer (or not yet) held by the stream" % int(index))
@@ -508,6 +506,29 @@ class HostStream(object):
     def drain(self):
         self._finalize_pending()
         self.s_out.synchronize()
+
+
+class DevicePack(object):
+    """Device buffers of one pass' p / q columns in the form that crosses the host link (bbk_pack_scores): the code words,
+    the chunk table, the p and q value lists and the pack state.  cap_p / cap_q: values the lists hold (default rows / 2 and
+    rows / 16, at least 1024); a pass with more raises PackState.overflow, and the caller decides what comes back instead."""
+
+    def __init__(self, rows, device, want_q, cap_p=None, cap_q=None):
+        self.lib = _lib.load()
+        self.rows = int(rows)
+        self.cap_p = int(cap_p) if cap_p else max(self.rows // 2, 1024)
+        self.cap_q = (int(cap_q) if cap_q else max(self.rows // 16, 1024)) if want_q else 0
+        self.codes = torch.empty(int(self.lib.bbk_pack_code_words(self.rows)), dtype=torch.int32, device=device)
+        self.chunks = torch.empty(int(self.lib.bbk_pack_chunks(self.rows)) * 24, dtype=torch.uint8, device=device)
+        self.vals_p = torch.empty(self.cap_p, dtype=torch.float64, device=device)
+        self.vals_q = torch.empty(self.cap_q, dtype=torch.float64, device=device) if want_q else None
+        self.state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8, device=device)
+
+    def pack(self, p, q, stream=None):
+        """bbk_pack_scores over the first `rows` rows of p and q (None without q-values); two launches on `stream`."""
+        _lib.check(self.lib.bbk_pack_scores(_lib.ptr(p), _lib.ptr(q), self.rows, _lib.ptr(self.codes), _lib.ptr(self.chunks),
+                                            _lib.ptr(self.vals_p), self.cap_p, _lib.ptr(self.vals_q), self.cap_q, _lib.ptr(self.state),
+                                            _lib.stream_ptr(stream)), "bbk_pack_scores")
 
 
 class PackedScores(object):

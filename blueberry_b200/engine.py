@@ -1,11 +1,11 @@
-"""Device-side stages of one Fit-Hi-C significance pass (the reference's fithic(), fithic.py:110-133); distributed.GenomePass
-enqueues them.
+"""Device-side stages of one Fit-Hi-C significance pass (the reference's fithic(), fithic.py:110-133): the tables a pass
+shares (Shard, BiasTables, PassEngine's possible pairs, distance table and fit buffers) and the launches of its stages.
+distributed.GenomePass enqueues them and adds the streaming K4 and K5, the Benjamini-Hochberg q-values (opt-in; the
+reference writes -1, fithic.py:435).
 
-    K1 hist_pairs  ->  [allreduce of the distance table across ranks]  ->  K2/K3 fit (one CTA)
-    ->  K4 pvalues  ->  K5 Benjamini-Hochberg q-values (opt-in; the reference writes -1, fithic.py:435)
+    K1 hist_pairs  ->  [allreduce of the distance table across ranks]  ->  K2/K3 fit (one CTA)  ->  K4 pvalues (direct)
 
-Everything between the first and last kernel is enqueued on one CUDA stream with no host
-synchronisation; S, the spline range and the candidate count of the q-value step stay on the device.
+Nothing here synchronises the host except read_fit(): S and the spline range stay on the device.
 PyTorch is used for device memory, streams and torch.distributed only.
 """
 import ctypes
@@ -121,7 +121,6 @@ class PassEngine(object):
         self.fit_ws = torch.zeros(ws, dtype=torch.uint8, device=dev)
         self.p_hist = torch.zeros(_lib.PHIST_LEN, dtype=torch.int64, device=dev)
         self.bias = None
-        self.bh_ws = None
         self.launches = 0
 
     def grow_bins(self):
@@ -238,12 +237,6 @@ class PassEngine(object):
                    "bbk_fit")
         self.launches += 1
 
-    def _bh_workspace(self, m):
-        need = int(self.lib.bbk_bh_workspace_bytes(int(m)))
-        if self.bh_ws is None or self.bh_ws.numel() < need:
-            self.bh_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
-        return self.bh_ws
-
     def pvalues(self, shard, p_out, with_hist=False):
         """K4.  with_hist: also fill self.p_hist (zero it first)."""
         bias = ctypes.byref(self.bias.struct) if self.bias is not None else None
@@ -252,14 +245,6 @@ class PassEngine(object):
                                         _lib.ptr(self.fit_result), _lib.ptr(self.spline_y), bias, _lib.ptr(p_out),
                                         _lib.ptr(self.p_hist) if with_hist else None, _lib.stream_ptr()), "bbk_pvalues")
         self.launches += 1
-
-    def qvalues(self, p, q, n_tests=-1):
-        """K5 over p, with the histogram K4 left in self.p_hist."""
-        m = int(p.numel())
-        ws = self._bh_workspace(m)
-        _lib.check(self.lib.bbk_bh_qvalues(_lib.ptr(p), m, int(n_tests), _lib.BH_UNSORTED, _lib.ptr(self.p_hist), _lib.ptr(q), None,
-                                           _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "bbk_bh_qvalues")
-        self.launches += 5       # init, threshold, compact, rank (one cooperative launch), ones fix
 
     # ------------------------------------------------------------------ results
     @staticmethod
@@ -285,93 +270,3 @@ class PassEngine(object):
     def read_fit(self):
         """Copy the fit status back (synchronises) and raise what the reference would raise."""
         return self.decode_fit(self.fit_result.cpu().numpy().tobytes())
-
-
-class HostPipeline(object):
-    """Successive single-shard passes (one library each, a distributed.GenomePass on this GPU alone) streamed from pinned
-    host memory.
-
-    A pass cannot start scoring before all of its records are on the device (S and the spline need the whole
-    distance table, fithic.py:110-133), so inside one pass the inbound and the outbound copies never overlap.
-    Across passes they do: while library k is being scored and its p/q travel back, library k+1 is already
-    arriving.  `slots` device copies of the record columns and of p/q make that legal; three streams (in, run,
-    out) and per-slot events order them.  Nothing here synchronises the host; call drain() (or wait on the event
-    submit() returns) before reading the host outputs.
-    """
-
-    class _Slot(object):
-        pass
-
-    def __init__(self, engine, max_pairs, chrom=0, slots=2):
-        from .distributed import GenomePass
-        self.eng = engine
-        self.chrom = int(chrom)
-        self.max_pairs = int(max_pairs)
-        dev = engine.device
-        rows = max((self.max_pairs + 3) & ~3, 4)          # GenomePass.attach: a shard's p / q rows in whole groups of 4
-        self.slots = []
-        for _ in range(int(slots)):
-            s = HostPipeline._Slot()
-            s.mid1, s.mid2, s.count = (torch.empty(self.max_pairs, dtype=torch.int32, device=dev) for _ in range(3))
-            s.p, s.q = (torch.empty(rows, dtype=torch.float64, device=dev) for _ in range(2))
-            s.in_ready, s.run_done, s.out_done = (torch.cuda.Event() for _ in range(3))
-            s.fit = torch.zeros_like(engine.fit_result)                      # this pass' BbkFitResult (the engine's is overwritten by the next pass)
-            s.h_fit = torch.zeros(engine.fit_result.numel(), dtype=torch.uint8).pin_memory()
-            s.index = -1
-            self.slots.append(s)
-        # Nothing here synchronises, so nothing would see BbkScoreState.overflow: the deferred list has a place for every row
-        # of a slot (and later attaches keep it, being no larger).
-        self.gp = GenomePass(engine, group=False)
-        self.gp.attach([Shard(s.mid1, s.mid2, s.count, chrom=self.chrom)], s.p, s.q, list_capacity=rows)
-        self.s_in, self.s_run, self.s_out = (torch.cuda.Stream(dev) for _ in range(3))
-        self.s_run.wait_stream(torch.cuda.current_stream(dev))      # the engine's tables were filled there
-        self.submitted = 0
-
-    def submit(self, h_mid1, h_mid2, h_count, h_p, h_q=None, n_tests=-1):
-        """Enqueue one pass: pinned int32 host columns in, p (and q when h_q is given) back into pinned float64
-        host buffers.  Returns the event that fires when the outputs are on the host."""
-        n = int(h_mid1.numel())
-        if n > self.max_pairs or h_mid2.numel() != n or h_count.numel() != n or h_p.numel() != n:
-            raise ValueError("library larger than the pipeline's slots, or columns differ in length")
-        for t in (h_mid1, h_mid2, h_count, h_p, h_q):
-            if t is not None and not t.is_pinned():
-                raise ValueError("host buffers must be pinned (torch.Tensor.pin_memory)")
-        s = self.slots[self.submitted % len(self.slots)]
-        self.submitted += 1
-        self.s_in.wait_event(s.run_done)        # the pass that last read this slot's records has finished
-        with torch.cuda.stream(self.s_in):
-            s.mid1[:n].copy_(h_mid1, non_blocking=True)
-            s.mid2[:n].copy_(h_mid2, non_blocking=True)
-            s.count[:n].copy_(h_count, non_blocking=True)
-            s.in_ready.record()
-        self.s_run.wait_event(s.in_ready)
-        self.s_run.wait_event(s.out_done)       # this slot's previous p/q have left the device
-        with torch.cuda.stream(self.s_run):
-            self.gp.q_values = h_q is not None
-            self.gp.attach([Shard(s.mid1[:n], s.mid2[:n], s.count[:n], chrom=self.chrom)], s.p, s.q)
-            self.gp.enqueue(n_tests)
-            s.fit.copy_(self.eng.fit_result, non_blocking=True)
-            s.run_done.record()
-        self.s_out.wait_event(s.run_done)
-        with torch.cuda.stream(self.s_out):
-            h_p.copy_(s.p[:n], non_blocking=True)
-            if h_q is not None:
-                h_q.copy_(s.q[:n], non_blocking=True)
-            s.h_fit.copy_(s.fit, non_blocking=True)
-            s.out_done.record()
-        s.index = self.submitted - 1
-        return s.out_done
-
-    def fit_of(self, index):
-        """Fit result of submission `index` (0-based), once its outputs are on the host: raises what the reference would
-        raise for that library (ZeroDivisionError, ...), else returns the FitResult - PassEngine.reference_smoothing(result)
-        then tells whether the pass has to be submitted again with the reference's own s.  Only the last `slots`
-        submissions are kept."""
-        s = self.slots[int(index) % len(self.slots)]
-        if s.index != int(index):
-            raise KeyError("submission %d is no longer (or not yet) held by the pipeline" % int(index))
-        s.out_done.synchronize()
-        return PassEngine.decode_fit(s.h_fit.numpy().tobytes())
-
-    def drain(self):
-        self.s_out.synchronize()

@@ -20,7 +20,6 @@ as in the reference (fithic.py:121-133 runs one pass).  No PNG is drawn.
 
 There is no CPU fallback: without libbbk.so and a CUDA device these functions raise.
 """
-import ctypes
 import gzip
 import sys
 
@@ -306,7 +305,7 @@ def _pinned_cache(dev, name, nbytes):
 def _scores_to_host(p_rows, q_rows, dev):
     """The pass' p / q columns as numpy arrays, plus keep = (p <= 1): packed on the device (bbk_pack_scores: two bits per row +
     the values that are not 1.0 / NaN), moved through pinned buffers that are allocated once, unpacked by all host cores."""
-    lib = _lib.load()
+    from .distributed import DevicePack
     n = int(p_rows.numel())
     p = np.empty(n, dtype=np.float64)
     q = np.empty(n, dtype=np.float64) if q_rows is not None else None
@@ -316,32 +315,24 @@ def _scores_to_host(p_rows, q_rows, dev):
     if p_rows.data_ptr() & 15 or (q_rows is not None and q_rows.data_ptr() & 15):
         p_rows = p_rows.clone()
         q_rows = q_rows.clone() if q_rows is not None else None
-    words, nch = int(lib.bbk_pack_code_words(n)), int(lib.bbk_pack_chunks(n))
-    st = _lib.stream_ptr()
-    cap_p, cap_q = max(n // 2, 1024), (max(n // 16, 1024) if q_rows is not None else 0)
-    for attempt in range(2):
-        codes = torch.empty(words, dtype=torch.int32, device=dev)
-        chunks = torch.empty(nch * 24, dtype=torch.uint8, device=dev)
-        vals_p = torch.empty(cap_p, dtype=torch.float64, device=dev)
-        vals_q = torch.empty(max(cap_q, 1), dtype=torch.float64, device=dev)
-        state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8, device=dev)
-        _lib.check(lib.bbk_pack_scores(_lib.ptr(p_rows), _lib.ptr(q_rows), n, _lib.ptr(codes), _lib.ptr(chunks), _lib.ptr(vals_p), cap_p,
-                                       _lib.ptr(vals_q) if q_rows is not None else None, cap_q, _lib.ptr(state), st), "bbk_pack_scores")
-        ps = _lib.PackState.from_buffer_copy(state.cpu().numpy().tobytes())
+    for caps in ((None, None), (n, n)):          # on overflow: every row carries a value, lists as long as the columns
+        pk = DevicePack(n, dev, q_rows is not None, *caps)
+        pk.pack(p_rows, q_rows)
+        ps = _lib.PackState.from_buffer_copy(pk.state.cpu().numpy().tobytes())
         if not ps.overflow:
             break
-        cap_p, cap_q = n, (n if q_rows is not None else 0)       # every row carries a value: lists as long as the columns
     n_p, n_q = int(ps.n_p), int(ps.n_q)
+    words, nch = pk.codes.numel(), pk.chunks.numel() // 24
     h_codes = _pinned_cache(dev, "codes", 4 * words)[:4 * words].view(torch.int32)
     h_chunks = _pinned_cache(dev, "chunks", 24 * nch)[:24 * nch]
     h_vp = _pinned_cache(dev, "vals_p", 8 * max(n_p, 1))[:8 * max(n_p, 1)].view(torch.float64)
     h_vq = _pinned_cache(dev, "vals_q", 8 * max(n_q, 1))[:8 * max(n_q, 1)].view(torch.float64)
-    h_codes.copy_(codes, non_blocking=True)
-    h_chunks.copy_(chunks, non_blocking=True)
+    h_codes.copy_(pk.codes, non_blocking=True)
+    h_chunks.copy_(pk.chunks, non_blocking=True)
     if n_p:
-        h_vp[:n_p].copy_(vals_p[:n_p], non_blocking=True)
+        h_vp[:n_p].copy_(pk.vals_p[:n_p], non_blocking=True)
     if n_q:
-        h_vq[:n_q].copy_(vals_q[:n_q], non_blocking=True)
+        h_vq[:n_q].copy_(pk.vals_q[:n_q], non_blocking=True)
     torch.cuda.current_stream(dev).synchronize()
     _io.unpack_scores(h_codes.numpy(), h_chunks.numpy(), h_vp.numpy(), h_vq.numpy() if q_rows is not None else None, n, p, q,
                       want_q=q_rows is not None, keep_out=keep.view(np.uint8))

@@ -275,70 +275,6 @@ def test_bias_loci_off_the_fragment_grid(shift):
     assert len(np.unique(ref.p[np.isin(m2, bm[moved])])) > 1    # the moved loci were really used
 
 
-def test_host_pipeline_matches_serial_genome_passes():
-    """engine.HostPipeline: five different libraries (different sizes and seeds) streamed through two device slots
-    give bit-for-bit the p and q of the same libraries run one at a time on the default stream."""
-    import torch
-    from blueberry_b200 import _lib
-    from blueberry_b200.distributed import GenomePass
-    from blueberry_b200.engine import BiasTables, HostPipeline, PassEngine, Shard
-    lib = _lib.load()
-    dev = torch.device("cuda:0")
-    R, nb, K = 5000, 6000, 400
-    P = int(lib.bbk_synth_n_pairs(nb, K))
-    rng = np.random.default_rng(5)
-    bias_host = np.exp(rng.normal(0.0, 0.25, size=nb))
-    bias_dev = torch.from_numpy(bias_host).to(dev)
-    eng = PassEngine(R, 100, 0, K * R, nb, dev)
-    eng.set_fragments([nb], [(nb - 1) * R])
-    eng.set_bias(BiasTables([np.where((bias_host < 0.5) | (bias_host > 2), -1.0, bias_host)], [R // 2], dev))
-    libs, want = [], []
-    for i in range(5):
-        cols = [torch.empty(P, dtype=torch.int32, device=dev) for _ in range(3)]
-        _lib.check(lib.bbk_synth_contacts(nb, K, R, 40.0 + 25 * i, 1.08, 100 + i, _lib.ptr(bias_dev), _lib.ptr(cols[0]),
-                                          _lib.ptr(cols[1]), _lib.ptr(cols[2]), _lib.stream_ptr()), "synth")
-        n = P - 1000 * i - (i & 1)                    # ragged sizes, odd and even
-        cols = [c[:n].contiguous() for c in cols]
-        gp = GenomePass(eng, group=False)
-        gp.attach([Shard(*cols)])
-        gp.run()
-        fit = eng.read_fit()
-        want.append((gp.shard_p(0).cpu(), gp.shard_q(0).cpu(), (fit.S, fit.n_knots, fit.smoothing, fit.y_min)))
-        libs.append([c.cpu().pin_memory() for c in cols])
-    torch.cuda.synchronize()
-    pipe = HostPipeline(eng, P, slots=2)
-    outs = []
-    for cols in libs:
-        n = cols[0].numel()
-        h_p, h_q = torch.empty(n, dtype=torch.float64).pin_memory(), torch.empty(n, dtype=torch.float64).pin_memory()
-        outs.append((h_p, h_q, pipe.submit(cols[0], cols[1], cols[2], h_p, h_q)))
-    outs[0][2].synchronize()                          # the event of the first library alone makes its outputs readable
-    assert torch.equal(outs[0][0].view(torch.int64), want[0][0].view(torch.int64))
-    pipe.drain()
-    for (h_p, h_q, _), (p, q, _fit) in zip(outs, want):
-        assert torch.equal(h_p.view(torch.int64), p.view(torch.int64))
-        assert torch.equal(h_q.view(torch.int64), q.view(torch.int64))
-    assert (want[0][0][:100000] != want[1][0][:100000]).any()
-    # every pass leaves its own fit result (the engine's is overwritten by the next pass); the last `slots` are held
-    for k in (3, 4):
-        fit = pipe.fit_of(k)
-        assert (fit.S, fit.n_knots, fit.smoothing, fit.y_min) == want[k][2]
-        assert fit.y_min > 0 and PassEngine.reference_smoothing(fit) in (None, fit.y_min ** 2)
-    with pytest.raises(KeyError):
-        pipe.fit_of(0)
-    # a library without a single contact: the reference divides by S == 0 (fithic.py:216); the pipeline reports it per pass
-    zero = torch.zeros(libs[0][2].numel(), dtype=torch.int32).pin_memory()
-    h_p = torch.empty(zero.numel(), dtype=torch.float64).pin_memory()
-    pipe.submit(libs[0][0], libs[0][1], zero, h_p)
-    with pytest.raises(ZeroDivisionError):
-        pipe.fit_of(5)
-    pipe.submit(libs[1][0], libs[1][1], libs[1][2], outs[1][0], outs[1][1])      # and the next pass is not affected
-    assert pipe.fit_of(6).S == want[1][2][0]
-    assert torch.equal(outs[1][0].view(torch.int64), want[1][0].view(torch.int64))
-    with pytest.raises(ValueError):
-        pipe.submit(libs[0][0], libs[0][1], libs[0][2], torch.empty(libs[0][0].numel(), dtype=torch.float64))
-
-
 def test_decimate_matches_reference_golden_and_oracle(tmp_path):
     """K7 (bbk_decimate through FithicContactMap.decimate) against the golden output of the reference's own method
     (tests/golden/decimate.npz), bit for bit including the order-dependent sum and product, then against the oracle on

@@ -586,6 +586,105 @@ def test_host_stream_packed_results_equal_dense():
             assert outs[0].nbytes() < 16 * rows + 4096
 
 
+def test_host_stream_matches_serial_genome_passes():
+    """distributed.HostStream: five different libraries (different sizes and seeds) streamed through two device slots
+    give bit-for-bit the p and q of the same libraries run one at a time on the default stream."""
+    import torch
+    from blueberry_b200 import _lib
+    from blueberry_b200.distributed import GenomePass, HostStream
+    from blueberry_b200.engine import BiasTables, PassEngine, Shard
+    lib = _lib.load()
+    dev = torch.device("cuda:0")
+    R, nb, K = 5000, 6000, 400
+    P = int(lib.bbk_synth_n_pairs(nb, K))
+    rng = np.random.default_rng(5)
+    bias_host = np.exp(rng.normal(0.0, 0.25, size=nb))
+    bias_dev = torch.from_numpy(bias_host).to(dev)
+    eng = PassEngine(R, 100, 0, K * R, nb, dev)
+    eng.set_fragments([nb], [(nb - 1) * R])
+    eng.set_bias(BiasTables([np.where((bias_host < 0.5) | (bias_host > 2), -1.0, bias_host)], [R // 2], dev))
+    libs, want = [], []
+    for i in range(5):
+        cols = [torch.empty(P, dtype=torch.int32, device=dev) for _ in range(3)]
+        _lib.check(lib.bbk_synth_contacts(nb, K, R, 40.0 + 25 * i, 1.08, 100 + i, _lib.ptr(bias_dev), _lib.ptr(cols[0]),
+                                          _lib.ptr(cols[1]), _lib.ptr(cols[2]), _lib.stream_ptr()), "synth")
+        n = P - 1000 * i - (i & 1)                    # ragged sizes, odd and even
+        cols = [c[:n].contiguous() for c in cols]
+        gp = GenomePass(eng, group=False)
+        gp.attach([Shard(*cols)])
+        gp.run()
+        fit = eng.read_fit()
+        want.append((gp.shard_p(0).cpu(), gp.shard_q(0).cpu(), (fit.S, fit.n_knots, fit.smoothing, fit.y_min)))
+        libs.append([c.cpu().pin_memory() for c in cols])
+    torch.cuda.synchronize()
+    pipe = HostStream(GenomePass(eng, group=False), [P], [0], slots=2)
+    outs = []
+    for cols in libs:
+        n = cols[0].numel()
+        h_p, h_q = torch.empty(n, dtype=torch.float64).pin_memory(), torch.empty(n, dtype=torch.float64).pin_memory()
+        outs.append((h_p, h_q, pipe.submit(cols[0], cols[1], cols[2], h_p, h_q, sizes=[n])))
+    outs[0][2].synchronize()                          # the event of the first library alone makes its outputs readable
+    assert torch.equal(outs[0][0].view(torch.int64), want[0][0].view(torch.int64))
+    pipe.drain()
+    for (h_p, h_q, _), (p, q, _fit) in zip(outs, want):
+        assert torch.equal(h_p.view(torch.int64), p.view(torch.int64))
+        assert torch.equal(h_q.view(torch.int64), q.view(torch.int64))
+    assert (want[0][0][:100000] != want[1][0][:100000]).any()
+    # every pass leaves its own fit result (the engine's is overwritten by the next pass); the last `slots` are held
+    for k in (3, 4):
+        fit = pipe.fit_of(k)
+        assert (fit.S, fit.n_knots, fit.smoothing, fit.y_min) == want[k][2]
+        assert fit.y_min > 0 and PassEngine.reference_smoothing(fit) in (None, fit.y_min ** 2)
+    with pytest.raises(KeyError):
+        pipe.fit_of(0)
+    # a library without a single contact: the reference divides by S == 0 (fithic.py:216); the stream reports it per pass
+    zero = torch.zeros(libs[0][2].numel(), dtype=torch.int32).pin_memory()
+    h_p = torch.empty(zero.numel(), dtype=torch.float64).pin_memory()
+    pipe.submit(libs[0][0], libs[0][1], zero, h_p, sizes=[zero.numel()])           # without h_q: no q-value step
+    assert pipe.gp.q_values
+    with pytest.raises(ZeroDivisionError):
+        pipe.fit_of(5)
+    pipe.submit(libs[1][0], libs[1][1], libs[1][2], outs[1][0], outs[1][1], sizes=[libs[1][0].numel()])     # and the next pass is not affected
+    assert pipe.fit_of(6).S == want[1][2][0]
+    assert torch.equal(outs[1][0].view(torch.int64), want[1][0].view(torch.int64))
+    with pytest.raises(ValueError):
+        pipe.submit(libs[0][0], libs[0][1], libs[0][2], torch.empty(libs[0][0].numel(), dtype=torch.float64), sizes=[libs[0][0].numel()])
+
+
+def test_host_stream_deferred_list_holds_every_row():
+    """A slot of more than 2^20 rows, nearly all of them deferred by the streaming K4 (counts above 64 go to its patch pass).
+    Nothing in the stream synchronises, so nothing would see a deferred-list overflow: the stream's list has a place for every
+    row of a slot, and p and q equal those of GenomePass.run (which repeats a pass whose list overflowed) bit for bit."""
+    import torch
+    from blueberry_b200 import _lib
+    from blueberry_b200.distributed import GenomePass, HostStream
+    from blueberry_b200.engine import PassEngine, Shard
+    lib = _lib.load()
+    dev = torch.device("cuda:0")
+    R, nb, K = 5000, 20050, 100
+    n = int(lib.bbk_synth_n_pairs(nb, K))
+    assert n > 1 << 20 and n % 4 == 0
+    cols = [torch.empty(n, dtype=torch.int32, device=dev) for _ in range(3)]
+    _lib.check(lib.bbk_synth_contacts(nb, K, R, 20000.0, 1.08, 3, None, _lib.ptr(cols[0]), _lib.ptr(cols[1]), _lib.ptr(cols[2]),
+                                      _lib.stream_ptr()), "synth")
+    eng = PassEngine(R, 100, 0, K * R, nb, dev)
+    eng.set_fragments([nb], [(nb - 1) * R])
+    gp = GenomePass(eng, group=False)
+    gp.attach([Shard(*cols)])
+    assert gp.listed
+    fit = gp.run()
+    assert gp.last_score.n_list > max(1 << 20, n // 4)            # more rows deferred than a default-size list holds
+    want_p, want_q = gp.shard_p(0).cpu(), gp.shard_q(0).cpu()
+    h = [c.cpu().pin_memory() for c in cols]
+    h_p, h_q = (torch.empty(n, dtype=torch.float64).pin_memory() for _ in range(2))
+    pipe = HostStream(GenomePass(eng, group=False), [n], [0], slots=2)
+    pipe.submit(h[0], h[1], h[2], h_p, h_q)
+    pipe.drain()
+    assert (pipe.fit_of(0).S, pipe.fit_of(0).smoothing) == (fit.S, fit.smoothing)
+    assert torch.equal(h_p.view(torch.int64), want_p.view(torch.int64))
+    assert torch.equal(h_q.view(torch.int64), want_q.view(torch.int64))
+
+
 def _torchrun(world, script, timeout=900):
     env = dict(os.environ)
     env["MASTER_ADDR"] = "127.0.0.1"
