@@ -21,6 +21,7 @@ FIT_STATUS = {
     -14: (ZeroDivisionError, "float division by zero (no in-range contacts: observedIntraInRangeSum == 0; fithic.py:216)"),
     -15: (ValueError, "x must be increasing if s > 0"),
     -16: (ValueError, "no genomic distance lies inside [min(x), max(x)]; nothing to evaluate the spline on"),
+    -17: (RuntimeError, "the fit problem's sizes, pointers or workspace do not allow the fit (bbk_fit_batched)"),
 }
 
 
@@ -36,6 +37,14 @@ class FitResult(ctypes.Structure):
         ("fp", ctypes.c_double), ("smoothing", ctypes.c_double), ("phase_cycles", ctypes.c_int64 * 6),
         ("spline_diag", ctypes.c_int64 * 8), ("y_min", ctypes.c_double),
     ]
+
+
+class FitProblem(ctypes.Structure):
+    _fields_ = [("d_possible", ctypes.c_void_p), ("d_obs_sum", ctypes.c_void_p), ("d_totals", ctypes.c_void_p),
+                ("d_result", ctypes.c_void_p), ("d_x", ctypes.c_void_p), ("d_y", ctypes.c_void_p), ("d_bin_of_key", ctypes.c_void_p),
+                ("d_spline_y", ctypes.c_void_p), ("d_spline_raw", ctypes.c_void_p), ("d_knots", ctypes.c_void_p),
+                ("d_coefs", ctypes.c_void_p), ("d_workspace", ctypes.c_void_p), ("workspace_bytes", ctypes.c_uint64),
+                ("nkeys", ctypes.c_int32), ("max_bins", ctypes.c_int32)]
 
 
 class BiasTable(ctypes.Structure):
@@ -65,6 +74,10 @@ class Candidates(ctypes.Structure):
     _fields_ = [("d_keys", ctypes.c_void_p), ("d_rows", ctypes.c_void_p), ("capacity", ctypes.c_int64)]
 
 
+class BhSegment(ctypes.Structure):
+    _fields_ = [("d_p_hist", ctypes.c_void_p), ("d_state", ctypes.c_void_p), ("cands", Candidates), ("n_tests", ctypes.c_int64)]
+
+
 _vp, _i32, _i64, _f64, _sz = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_double, ctypes.c_size_t
 
 # name -> (restype, argtypes); exactly the prototypes of include/bbk.h
@@ -79,6 +92,7 @@ SIGNATURES = {
     "bbk_fit_workspace_bytes": (_sz, [_i32, _i32]),
     "bbk_fit": (ctypes.c_int, [_vp, _vp, _i32, _vp, _i32, _i64, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                _vp, _sz, _vp]),
+    "bbk_fit_batched": (ctypes.c_int, [_vp, _i32, _i32, _i64, _i64, _i64, _vp]),
     "bbk_fit_from_bins": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "bbk_pvalues": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _i64, _i64, _i64, _vp, _vp,
                                    ctypes.POINTER(BiasTable), _vp, _vp, _vp]),
@@ -106,6 +120,8 @@ SIGNATURES = {
     "bbk_pack_code_words": (_i64, [_i64]),
     "bbk_pack_scores": (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp]),
     "bbk_bh_qvalues_listed": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, ctypes.POINTER(Candidates), _vp, _vp, _sz, _vp]),
+    "bbk_bh_segmented_workspace_bytes": (_sz, [_i64, _i32]),
+    "bbk_bh_qvalues_segmented": (ctypes.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, _vp, _sz, _vp]),
     "bbk_bh_select_listed": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, ctypes.POINTER(Candidates), _vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "bbk_bh_gathered_workspace_bytes": (_sz, [_i32, _i64]),
     "bbk_bh_pack_count": (ctypes.c_int, [_vp, _vp, _vp]),

@@ -120,8 +120,7 @@ __global__ void __launch_bounds__(BH_THREADS) bh_hist_kernel(const double* p, lo
 }
 
 // one CTA of 1024 threads (4 buckets each): totals, N, and the saturation bucket
-__global__ void __launch_bounds__(1024) bh_threshold_kernel(BhState* st, const long long* phist, int prune, int listed,
-                                                            const BbkScoreState* ss = nullptr) {
+__device__ __forceinline__ void bh_threshold_body(BhState* st, const long long* phist, int prune, int listed, const BbkScoreState* ss) {
     __shared__ long long part[1024];
     __shared__ int first_bucket;
     const int t = threadIdx.x;
@@ -167,6 +166,11 @@ __global__ void __launch_bounds__(1024) bh_threshold_kernel(BhState* st, const l
         // (a candidate list that overflowed is no list: the full pass over p takes over)
         st->use_list = (listed && tau <= bbk_key_of(BBK_SMALL_P) && !(ss && ss->cand_overflow)) ? 1 : 0;
     }
+}
+
+__global__ void __launch_bounds__(1024) bh_threshold_kernel(BhState* st, const long long* phist, int prune, int listed,
+                                                            const BbkScoreState* ss = nullptr) {
+    bh_threshold_body(st, phist, prune, listed, ss);
 }
 
 // the 16 B/pair pass: q = 1.0 for saturated / p == 1.0 rows, NaN for NaN rows, candidates appended.  A CTA takes chunks of
@@ -505,7 +509,30 @@ struct RankParams {
     long long* rank;         // optional
     long long n_host;        // >= 0: number of (key, index) pairs, known to the host; < 0: BhState::n_cand
     int src;                 // buffer (0 / 1) the pairs start in; a sort-only launch leaves the result there
+    // segmented ranking (bbk_bh_qvalues_segmented): the index is a row, row r belongs to the segment s with
+    // seg_off[s] <= r < seg_off[s + 1]; seg[s] is that segment's state, seg_start[s] where its candidates start once sorted
+    const long long* seg_off;
+    BhState* seg;
+    unsigned long long* seg_start;
+    int n_seg;
+    int seg_passes;          // extra stable digit passes keyed on the segment: 1 up to 256 segments, 2 above
 };
+
+__device__ __forceinline__ int seg_of(const long long* off, int n_seg, unsigned row) {     // last s with off[s] <= row
+    int lo = 0, hi = n_seg - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(off + mid) <= (long long)row) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// radix digit of pass `pass`: the 8 bytes of the key, then (segmented) the bytes of the row's segment
+template <bool SEG>
+__device__ __forceinline__ unsigned rk_digit(const RankParams& R, unsigned long long key, unsigned val, int pass) {
+    if (SEG && pass >= NPASS) return ((unsigned)seg_of(R.seg_off, R.n_seg, val) >> (8 * (pass - NPASS))) & 255u;
+    return (unsigned)(key >> (8 * pass)) & 255u;
+}
 
 __device__ __forceinline__ int rk_eff_blocks(long long n, int G) {
     long long g = (n + RK_TILE - 1) / RK_TILE;
@@ -532,6 +559,30 @@ __device__ __forceinline__ MaxHead mh_combine(const MaxHead& a, const MaxHead& b
     r.h = a.h > b.h ? a.h : b.h;
     return r;
 }
+// segmented: h = where the element's segment starts; a later segment discards what came before it
+__device__ __forceinline__ MaxHead mh_combine_seg(const MaxHead& a, const MaxHead& b) {
+    if (b.h > a.h) return b;
+    MaxHead r;
+    r.v = (a.v > b.v) ? a.v : b.v;
+    r.h = a.h;
+    return r;
+}
+template <bool SEG>
+__device__ __forceinline__ MaxHead mh_comb(const MaxHead& a, const MaxHead& b) { return SEG ? mh_combine_seg(a, b) : mh_combine(a, b); }
+// element i of the sorted candidates of a segmented ranking: rank and N are its segment's, and a tie group never spans a segment
+// boundary (fithic.py:473-485 inside every segment)
+__device__ __forceinline__ MaxHead mh_elem_seg(const RankParams& R, const unsigned long long* keys, const unsigned* idx, long long i) {
+    const int s = seg_of(R.seg_off, R.n_seg, idx[i]);
+    const long long start = (long long)R.seg_start[s];
+    const unsigned long long k = keys[i];
+    MaxHead e;
+    e.h = start;
+    if (i == start || keys[i - 1] != k) {
+        double bh = (value_of(k) * (double)R.seg[s].n_tests) / (double)(i - start + 1);
+        e.v = (1.0 < bh) ? 1.0 : bh;
+    } else e.v = -INFINITY;
+    return e;
+}
 __device__ __forceinline__ MaxHead mh_elem(const unsigned long long* keys, long long i, double N) {
     MaxHead e;
     const unsigned long long k = keys[i];
@@ -543,7 +594,7 @@ __device__ __forceinline__ MaxHead mh_elem(const unsigned long long* keys, long 
     return e;
 }
 
-template <bool SCAN>
+template <bool SCAN, bool SEG>
 __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
     cg::grid_group grid = cg::this_grid();
     __shared__ unsigned base[256];                   // digit counts of the chunk, then the running output cursor per digit
@@ -565,14 +616,18 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
     unsigned* table = R.L.block_hist;                // [Ge][256]
     int par = R.src;
-    for (int pass = 0; pass < NPASS; ++pass) {
-        const int shift = 8 * pass;
+    if (SEG && b == 0 && t == 0) {                   // where every segment's candidates start once sorted (published by the first grid.sync)
+        unsigned long long run = 0;
+        for (int s = 0; s < R.n_seg; ++s) { R.seg_start[s] = run; run += R.seg[s].n_cand; }
+    }
+    for (int pass = 0; pass < NPASS + (SEG ? R.seg_passes : 0); ++pass) {
         const unsigned long long* kin = R.L.keys[par];
         if (active) {
             if (t < 256) base[t] = 0;
             if (t == 0) sh_skip = 0;
             __syncthreads();
-            for (long long i = c.lo + t; i < c.hi; i += RK_THREADS) atomicAdd(&base[(unsigned)(kin[i] >> shift) & 255u], 1u);
+            for (long long i = c.lo + t; i < c.hi; i += RK_THREADS)
+                atomicAdd(&base[rk_digit<SEG>(R, kin[i], SEG ? R.L.idx[par][i] : 0u, pass)], 1u);
             __syncthreads();
             if (t < 256) table[(size_t)b * 256 + t] = base[t];
         }
@@ -607,7 +662,7 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
             }
             __syncthreads();
             const bool skip = sh_skip != 0;
-            if (t == 0 && b == 0) st->skip[pass] = skip ? 1 : 0;
+            if (t == 0 && b == 0 && (!SEG || pass < NPASS)) st->skip[pass] = skip ? 1 : 0;
             if (!skip) {
                 const unsigned* iin = R.L.idx[par];
                 unsigned long long* kout = R.L.keys[par ^ 1];
@@ -628,7 +683,7 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
 #pragma unroll
                     for (int it = 0; it < RK_IPT; ++it) {
                         const bool live = wbase + it * 32 + lane < c.hi;
-                        const unsigned dg = live ? ((unsigned)(key[it] >> shift) & 255u) : 256u;
+                        const unsigned dg = live ? rk_digit<SEG>(R, key[it], val[it], pass) : 256u;
                         const unsigned peers = __match_any_sync(0xffffffffu, dg);
                         const unsigned rk = __popc(peers & ((1u << lane) - 1));
                         const unsigned before = live ? whist[warp][dg] : 0;
@@ -663,7 +718,7 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
 #pragma unroll
                     for (int it = 0; it < RK_IPT; ++it) {
                         if (wbase + it * 32 + lane < c.hi) {
-                            const unsigned dg = (unsigned)(key[it] >> shift) & 255u;
+                            const unsigned dg = rk_digit<SEG>(R, key[it], val[it], pass);
                             const unsigned lp = tstart[dg] + whist[warp][dg] + loc[it];
                             skeys[lp] = key[it];
                             svals[lp] = val[it];
@@ -674,10 +729,11 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
                     const int n_tile = left < RK_TILE ? (int)left : RK_TILE;
                     for (int k = t; k < n_tile; k += RK_THREADS) {
                         const unsigned long long kk = skeys[k];
-                        const unsigned dg = (unsigned)(kk >> shift) & 255u;
+                        const unsigned vv = svals[k];
+                        const unsigned dg = rk_digit<SEG>(R, kk, vv, pass);
                         const unsigned pos = gstart[dg] + ((unsigned)k - tstart[dg]);
                         kout[pos] = kk;
-                        iout[pos] = svals[k];
+                        iout[pos] = vv;
                     }
                     __syncthreads();
                 }
@@ -711,14 +767,14 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
         if (lo > c.hi) lo = c.hi;
         if (hi > c.hi) hi = c.hi;
         MaxHead acc = ident;
-        for (long long i = lo; i < hi; ++i) acc = mh_combine(acc, mh_elem(keys, i, N));
+        for (long long i = lo; i < hi; ++i) acc = mh_comb<SEG>(acc, SEG ? mh_elem_seg(R, keys, idx, i) : mh_elem(keys, i, N));
         MaxHead inc = acc;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
             MaxHead up;
             up.v = __shfl_up_sync(0xffffffffu, inc.v, o);
             up.h = __shfl_up_sync(0xffffffffu, inc.h, o);
-            if (lane >= o) inc = mh_combine(up, inc);
+            if (lane >= o) inc = mh_comb<SEG>(up, inc);
         }
         if (lane == 31) { wv[warp] = inc.v; wh[warp] = inc.h; }
         excl.v = __shfl_up_sync(0xffffffffu, inc.v, 1);
@@ -726,10 +782,10 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
         if (lane == 0) excl = ident;
         __syncthreads();
         MaxHead wpre = ident;
-        for (int w = 0; w < warp; ++w) { MaxHead e = {wv[w], wh[w]}; wpre = mh_combine(wpre, e); }
-        excl = mh_combine(wpre, excl);
+        for (int w = 0; w < warp; ++w) { MaxHead e = {wv[w], wh[w]}; wpre = mh_comb<SEG>(wpre, e); }
+        excl = mh_comb<SEG>(wpre, excl);
         if (t == RK_THREADS - 1) {
-            MaxHead all = mh_combine(excl, acc);
+            MaxHead all = mh_comb<SEG>(excl, acc);
             R.L.part_max[b] = all.v;
             R.L.part_head[b] = all.h;
         }
@@ -737,23 +793,39 @@ __global__ void __launch_bounds__(RK_THREADS, 1) bh_rank_kernel(RankParams R) {
     grid.sync();
     if (active) {
         MaxHead run = ident;                         // chunks of the earlier CTAs
-        for (int bb = lane; bb < b; bb += 32) { MaxHead e = {R.L.part_max[bb], R.L.part_head[bb]}; run = mh_combine(run, e); }
+        if (SEG) {      // CTAs in order: the lanes' strided partials are combined in CTA order below
+            MaxHead ordered = ident;
+            if (lane == 0)
+                for (int bb = 0; bb < b; ++bb) { MaxHead e = {R.L.part_max[bb], R.L.part_head[bb]}; ordered = mh_combine_seg(ordered, e); }
+            run.v = __shfl_sync(0xffffffffu, ordered.v, 0);
+            run.h = __shfl_sync(0xffffffffu, ordered.h, 0);
+        } else {
+            for (int bb = lane; bb < b; bb += 32) { MaxHead e = {R.L.part_max[bb], R.L.part_head[bb]}; run = mh_combine(run, e); }
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            MaxHead other;
-            other.v = __shfl_xor_sync(0xffffffffu, run.v, o);
-            other.h = __shfl_xor_sync(0xffffffffu, run.h, o);
-            run = mh_combine(run, other);
+            for (int o = 16; o > 0; o >>= 1) {
+                MaxHead other;
+                other.v = __shfl_xor_sync(0xffffffffu, run.v, o);
+                other.h = __shfl_xor_sync(0xffffffffu, run.h, o);
+                run = mh_combine(run, other);
+            }
         }
-        run = mh_combine(run, excl);
+        run = mh_comb<SEG>(run, excl);
         for (long long i = lo; i < hi; ++i) {
-            run = mh_combine(run, mh_elem(keys, i, N));
-            const unsigned o = idx[i];
-            R.q[o] = run.v;
-            if (R.rank) R.rank[o] = run.h + 1;
+            if (SEG) {
+                run = mh_combine_seg(run, mh_elem_seg(R, keys, idx, i));
+                const unsigned o = idx[i];
+                R.q[o] = run.v;
+                const int s = seg_of(R.seg_off, R.n_seg, o);
+                if ((unsigned long long)i + 1 == R.seg_start[s] + R.seg[s].n_cand) R.seg[s].total_max = run.v;   // the segment's last candidate
+            } else {
+                run = mh_combine(run, mh_elem(keys, i, N));
+                const unsigned o = idx[i];
+                R.q[o] = run.v;
+                if (R.rank) R.rank[o] = run.h + 1;
+            }
         }
     }
-    if (b == 0 && warp == 0) {                       // the p == 1.0 group: one tie group after every candidate
+    if (!SEG && b == 0 && warp == 0) {                       // the p == 1.0 group: one tie group after every candidate
         MaxHead all = ident;
         for (int bb = lane; bb < Ge; bb += 32) { MaxHead e = {R.L.part_max[bb], R.L.part_head[bb]}; all = mh_combine(all, e); }
 #pragma unroll
@@ -779,9 +851,11 @@ int rank_grid() {            // CTAs of bh_rank_kernel that are resident togethe
     static int g = 0;
     if (g == 0) {
         int per_sm = 0;
-        if (cudaFuncSetAttribute(bh_rank_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_DYN_SMEM) != cudaSuccess) return 0;
-        if (cudaFuncSetAttribute(bh_rank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_DYN_SMEM) != cudaSuccess) return 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bh_rank_kernel<true>, RK_THREADS, RK_DYN_SMEM) != cudaSuccess || per_sm < 1) return 0;
+        if (cudaFuncSetAttribute(bh_rank_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_DYN_SMEM) != cudaSuccess) return 0;
+        if (cudaFuncSetAttribute(bh_rank_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_DYN_SMEM) != cudaSuccess) return 0;
+        if (cudaFuncSetAttribute(bh_rank_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_DYN_SMEM) != cudaSuccess) return 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bh_rank_kernel<true, false>, RK_THREADS, RK_DYN_SMEM) != cudaSuccess || per_sm < 1) return 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bh_rank_kernel<true, true>, RK_THREADS, RK_DYN_SMEM) != cudaSuccess || per_sm < 1) return 0;
         g = bbk_num_sms();
     }
     return g;
@@ -790,10 +864,10 @@ int rank_grid() {            // CTAs of bh_rank_kernel that are resident togethe
 int launch_rank(const BhLayout& L, double* q, long long* rank, cudaStream_t st) {
     int g = rank_grid();
     if (g <= 0 || g > L.G) { bbk_set_error("bh_rank_kernel: cooperative launch not possible on this device"); return BBK_E_CUDA; }
-    RankParams R;
+    RankParams R = {};
     R.L = L; R.q = q; R.rank = rank; R.n_host = -1; R.src = 0;
     void* args[] = {&R};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)bh_rank_kernel<true>, dim3(g), dim3(RK_THREADS), args, RK_DYN_SMEM, st);
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)bh_rank_kernel<true, false>, dim3(g), dim3(RK_THREADS), args, RK_DYN_SMEM, st);
     if (e != cudaSuccess) { bbk_set_error("bh_rank_kernel: %s", cudaGetErrorString(e)); return BBK_E_CUDA; }
     return BBK_OK;
 }
@@ -815,10 +889,10 @@ int bbk_sort_pairs(void* workspace, long long capacity, long long n_host, int sr
     BhLayout L;
     bh_layout(workspace, capacity, bbk_num_sms() * 4 > 1024 ? 1024 : bbk_num_sms() * 4, &L);
     if (g <= 0 || g > L.G) { bbk_set_error("bbk_sort_pairs: cooperative launch not possible on this device"); return BBK_E_CUDA; }
-    RankParams R;
+    RankParams R = {};
     R.L = L; R.q = nullptr; R.rank = nullptr; R.n_host = n_host; R.src = src;
     void* args[] = {&R};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)bh_rank_kernel<false>, dim3(g), dim3(RK_THREADS), args, RK_DYN_SMEM, st);
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)bh_rank_kernel<false, false>, dim3(g), dim3(RK_THREADS), args, RK_DYN_SMEM, st);
     if (e != cudaSuccess) { bbk_set_error("bbk_sort_pairs: %s", cudaGetErrorString(e)); return BBK_E_CUDA; }
     return BBK_OK;
 }
@@ -945,6 +1019,173 @@ extern "C" int bbk_bh_qvalues_listed(const double* d_p, int64_t m, int64_t n_tes
     if (rc != BBK_OK) return rc;
     ones_fix_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, m, d_q, L.st);
     BBK_CHECK_LAUNCH("ones_fix_kernel");
+    return BBK_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Per-segment q-values in one step (bbk_bh_qvalues_segmented): segment s = rows [off[s], off[s+1]) of one p / q pair, each with
+// its own histogram, candidate list, score state and N.  Five launches whatever the number of segments:
+//   threshold (one CTA per segment, the body of bh_threshold_kernel on the segment's histogram)
+//   -> candidate filter over every list (segments whose list holds every candidate)
+//   -> the 16 B/row pass over the rows of the other segments only
+//   -> one cooperative rank launch: the key passes plus stable digit passes keyed on the row's segment, so the candidates end
+//      up ordered by (segment, p); the forward running max restarts at every segment with that segment's N
+//   -> ones fix, with a q_ones per segment
+// ---------------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int BH_SEG_MAX = 1 << 16;      // two segment digits
+
+__device__ void bh_state_init(BhState* st, long long n_tests) {
+    st->n_cand = 0; st->n_ones = 0; st->n_nan = 0; st->n_valid = 0; st->tau_key = ~0ull;
+    st->n_tests = n_tests; st->q_ones = 1.0; st->total_max = -INFINITY; st->need_ones_fix = 0;
+    for (int p = 0; p < NPASS; ++p) st->skip[p] = 0;
+    st->use_list = 0;
+}
+
+__global__ void __launch_bounds__(1024) bh_threshold_seg_kernel(const BbkBhSegment* segs, BhState* seg_st, BhState* st) {
+    const BbkBhSegment& sg = segs[blockIdx.x];
+    BhState* ss = seg_st + blockIdx.x;
+    if (threadIdx.x == 0) {
+        bh_state_init(ss, sg.n_tests);
+        if (blockIdx.x == 0) bh_state_init(st, -1);
+    }
+    __syncthreads();
+    bh_threshold_body(ss, (const long long*)sg.d_p_hist, 1, 1, sg.d_state);
+}
+
+// appends the lanes' candidates of one warp step: one atomic on the shared count, one on the segment's
+__device__ __forceinline__ void seg_append(bool cand, unsigned long long k, unsigned row, BhState* st, BhState* ss,
+                                           unsigned long long* keys, unsigned* idx) {
+    const unsigned bal = __ballot_sync(0xffffffffu, cand);
+    if (!bal) return;
+    const int lane = threadIdx.x & 31, leader = __ffs(bal) - 1;
+    unsigned long long base = 0;
+    if (lane == leader) {
+        base = atomicAdd(&st->n_cand, (unsigned long long)__popc(bal));
+        atomicAdd(&ss->n_cand, (unsigned long long)__popc(bal));
+    }
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (cand) {
+        const unsigned long long pos = base + __popc(bal & ((1u << lane) - 1));
+        keys[pos] = k;
+        idx[pos] = row;
+    }
+}
+
+__global__ void __launch_bounds__(BH_THREADS) bh_cand_filter_seg_kernel(const BbkBhSegment* segs, int n_seg, BhState* seg_st, BhState* st,
+                                                                        unsigned long long* keys, unsigned* idx) {
+    const long long stride = (long long)gridDim.x * BH_THREADS;
+    for (int s = 0; s < n_seg; ++s) {
+        BhState* ss = seg_st + s;
+        if (!ss->use_list) continue;
+        const unsigned long long tau = ss->tau_key;
+        const unsigned long long* ck = (const unsigned long long*)segs[s].cands.d_keys;
+        const unsigned* cr = segs[s].cands.d_rows;
+        const long long n = (long long)segs[s].d_state->n_cand;
+        for (long long i0 = (long long)blockIdx.x * BH_THREADS; i0 < n; i0 += stride) {
+            const long long i = i0 + threadIdx.x;
+            const unsigned long long k = i < n ? ck[i] : ~0ull;
+            const bool cand = i < n && k < tau;
+            seg_append(cand, k, cand ? cr[i] : 0u, st, ss, keys, idx);
+        }
+    }
+}
+
+// bh_compact_kernel (keep_ones = 0, no rank) over the rows of the segments whose candidate list does not cover every candidate
+__global__ void __launch_bounds__(BH_THREADS) bh_compact_seg_kernel(const double* p, double* q, const long long* off, int n_seg,
+                                                                    BhState* seg_st, BhState* st, unsigned long long* keys, unsigned* idx) {
+    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    const long long stride = (long long)gridDim.x * BH_THREADS;
+    for (int s = 0; s < n_seg; ++s) {
+        BhState* ss = seg_st + s;
+        if (ss->use_list) continue;
+        const unsigned long long tau = ss->tau_key;
+        const long long hi = off[s + 1];
+        for (long long i0 = off[s] + (long long)blockIdx.x * BH_THREADS; i0 < hi; i0 += stride) {
+            const long long i = i0 + threadIdx.x;
+            const bool live = i < hi;
+            const double v = live ? ld_stream_double(p + i) : qnan;
+            const bool isn = isnan(v);
+            const unsigned long long k = key_of(v);
+            const bool cand = live && !isn && k < tau && v != 1.0;
+            if (live && !cand) st_stream_double(q + i, isn ? qnan : 1.0);
+            seg_append(cand, k, (unsigned)i, st, ss, keys, idx);
+        }
+    }
+}
+
+// q of every segment's p == 1.0 group: one tie group after the segment's candidates (the end of bh_rank_kernel, per segment)
+__global__ void __launch_bounds__(BH_THREADS) ones_fix_seg_kernel(const double* p, double* q, const long long* off, int n_seg, BhState* seg_st) {
+    const long long stride = (long long)gridDim.x * BH_THREADS;
+    for (int s = 0; s < n_seg; ++s) {
+        BhState* ss = seg_st + s;
+        if (ss->n_ones == 0) continue;
+        double bh = (1.0 * (double)ss->n_tests) / (double)(ss->n_cand + 1);
+        bh = (1.0 < bh) ? 1.0 : bh;
+        double qo = (ss->total_max > bh) ? ss->total_max : bh;
+        if (ss->tau_key != ~0ull) qo = 1.0;
+        if (qo == 1.0) continue;
+        if (blockIdx.x == 0 && threadIdx.x == 0) { ss->q_ones = qo; ss->need_ones_fix = 1; }
+        for (long long i = off[s] + (long long)blockIdx.x * BH_THREADS + threadIdx.x; i < off[s + 1]; i += stride)
+            if (p[i] == 1.0) q[i] = qo;
+    }
+}
+
+size_t bh_seg_layout(void* base, long long m, int n_seg, BhLayout* L, BhState** seg_st, unsigned long long** seg_start) {
+    size_t off = bh_layout(base, m, sort_blocks(), L);
+    char* b = (char*)base;
+    if (seg_st) *seg_st = b ? (BhState*)(b + off) : nullptr;
+    off = align256(off + sizeof(BhState) * (size_t)n_seg);
+    if (seg_start) *seg_start = b ? (unsigned long long*)(b + off) : nullptr;
+    off = align256(off + sizeof(unsigned long long) * (size_t)n_seg);
+    return off;
+}
+
+}  // namespace
+
+extern "C" size_t bbk_bh_segmented_workspace_bytes(int64_t m, int32_t n_segments) {
+    if (m < 0 || n_segments < 0) return 0;
+    return bh_seg_layout(nullptr, m, n_segments, nullptr, nullptr, nullptr) + 256;
+}
+
+extern "C" int bbk_bh_qvalues_segmented(const double* d_p, int64_t m, const int64_t* d_offsets, const BbkBhSegment* d_segments,
+                                        int32_t n_segments, double* d_q, void* d_workspace, size_t workspace_bytes, void* stream) {
+    BBK_REQUIRE(m >= 0 && m < (1ll << 32), "bbk_bh_qvalues_segmented: m must be in [0, 2^32)");
+    BBK_REQUIRE(n_segments >= 0 && n_segments <= BH_SEG_MAX, "bbk_bh_qvalues_segmented: n_segments must be in [0, 65536]");
+    if (n_segments == 0 || m == 0) return BBK_OK;
+    BBK_REQUIRE(d_p && d_q && d_offsets && d_segments && d_workspace, "bbk_bh_qvalues_segmented: null pointer");
+    BBK_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "bbk_bh_qvalues_segmented: workspace must be 256-byte aligned");
+    BhLayout L;
+    BhState* seg_st;
+    unsigned long long* seg_start;
+    size_t need = bh_seg_layout(d_workspace, m, n_segments, &L, &seg_st, &seg_start);
+    if (workspace_bytes < need) {
+        bbk_set_error("bbk_bh_qvalues_segmented: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+        return BBK_E_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int sms = bbk_num_sms();
+    const long long* off = (const long long*)d_offsets;
+    bh_threshold_seg_kernel<<<n_segments, 1024, 0, st>>>(d_segments, seg_st, L.st);
+    BBK_CHECK_LAUNCH("bh_threshold_seg_kernel");
+    bh_cand_filter_seg_kernel<<<sms * 2, BH_THREADS, 0, st>>>(d_segments, n_segments, seg_st, L.st, L.keys[0], L.idx[0]);
+    BBK_CHECK_LAUNCH("bh_cand_filter_seg_kernel");
+    long long want = (m + BH_THREADS - 1) / BH_THREADS;
+    const int grid = (int)(want < (long long)sms * 8 ? want : (long long)sms * 8);
+    bh_compact_seg_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, d_q, off, n_segments, seg_st, L.st, L.keys[0], L.idx[0]);
+    BBK_CHECK_LAUNCH("bh_compact_seg_kernel");
+    const int g = rank_grid();
+    if (g <= 0 || g > L.G) { bbk_set_error("bh_rank_kernel: cooperative launch not possible on this device"); return BBK_E_CUDA; }
+    RankParams R = {};
+    R.L = L; R.q = d_q; R.rank = nullptr; R.n_host = -1; R.src = 0;
+    R.seg_off = off; R.seg = seg_st; R.seg_start = seg_start; R.n_seg = n_segments;
+    R.seg_passes = n_segments <= 1 ? 0 : (n_segments <= 256 ? 1 : 2);
+    void* args[] = {&R};
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)bh_rank_kernel<true, true>, dim3(g), dim3(RK_THREADS), args, RK_DYN_SMEM, st);
+    if (e != cudaSuccess) { bbk_set_error("bh_rank_kernel: %s", cudaGetErrorString(e)); return BBK_E_CUDA; }
+    ones_fix_seg_kernel<<<grid, BH_THREADS, 0, st>>>(d_p, d_q, off, n_segments, seg_st);
+    BBK_CHECK_LAUNCH("ones_fix_seg_kernel");
     return BBK_OK;
 }
 

@@ -57,7 +57,19 @@ __device__ __forceinline__ double* pick(double* pool, size_t pool_doubles, size_
     return need <= pool_doubles ? pool : global_fallback;
 }
 
-__global__ void __launch_bounds__(FIT_THREADS, 1) fit_kernel(FitParams P) {
+// bytes of scratch one fit needs (bbk_fit_workspace_bytes); the batched kernel checks every problem's workspace with it
+BBK_HD size_t fit_workspace_bytes(int max_bins, int nkeys) {
+    size_t m = max_bins > 4 ? (size_t)max_bins : 4;
+    size_t a = (size_t)3 * nkeys + m + 2;
+    size_t b = bbk_coop_ws_doubles((int)m) + 2 * m;
+    size_t c = 3 * (m + 4) + (size_t)4 * nkeys + 8;
+    size_t mx = a > b ? a : b;
+    mx = mx > c ? mx : c;
+    return (mx + 16) * sizeof(double);
+}
+
+// the whole fit of one problem by one CTA of FIT_THREADS threads
+__device__ __forceinline__ void fit_body(const FitParams& P) {
     extern __shared__ double pool[];
     __shared__ FitShared sh;
     const int tid = threadIdx.x;
@@ -376,6 +388,36 @@ __global__ void __launch_bounds__(FIT_THREADS, 1) fit_kernel(FitParams P) {
     }
 }
 
+__global__ void __launch_bounds__(FIT_THREADS, 1) fit_kernel(FitParams P) { fit_body(P); }
+
+// bbk_fit_batched: CTA b runs problem b with the shared n_bins / R / distance limits.  A problem that cannot run (sizes, null
+// pointers, workspace below fit_workspace_bytes) gets BBK_FIT_BAD_PROBLEM in its own result and touches nothing else.
+__global__ void __launch_bounds__(FIT_THREADS, 1) fit_batched_kernel(const BbkFitProblem* problems, int n_bins, long long R,
+                                                                     long long min_dist, long long max_dist, size_t pool_doubles) {
+    const BbkFitProblem pr = problems[blockIdx.x];
+    if (!pr.d_result) return;
+    const bool ok = pr.d_possible && pr.d_obs_sum && pr.d_totals && pr.d_x && pr.d_y && pr.d_spline_y && pr.d_spline_raw &&
+                    pr.d_knots && pr.d_coefs && pr.d_workspace && pr.nkeys > 0 && pr.max_bins >= 4 &&
+                    pr.workspace_bytes >= fit_workspace_bytes(pr.max_bins, pr.nkeys);
+    if (!ok) {
+        if (threadIdx.x == 0) {
+            BbkFitResult* r = pr.d_result;
+            r->status = BBK_FIT_BAD_PROBLEM;
+            r->n_out = 0; r->k0 = 0; r->L = 0; r->n_knots = 0; r->ier = 0; r->S = 0;
+            r->residual = 0.0;
+        }
+        return;
+    }
+    FitParams P;
+    P.possible = (const long long*)pr.d_possible; P.observed = (const long long*)pr.d_obs_sum; P.totals = (const long long*)pr.d_totals;
+    P.x_in = nullptr; P.y_in = nullptr; P.m_in = 0;
+    P.nkeys = pr.nkeys; P.n_bins = n_bins; P.R = R; P.min_dist = min_dist; P.max_dist = max_dist; P.max_bins = pr.max_bins;
+    P.result = pr.d_result; P.x = pr.d_x; P.y = pr.d_y; P.bin_of_key = pr.d_bin_of_key; P.spline_y = pr.d_spline_y;
+    P.spline_raw = pr.d_spline_raw; P.knots = pr.d_knots; P.coefs = pr.d_coefs; P.gws = (double*)pr.d_workspace;
+    P.pool_doubles = pool_doubles;
+    fit_body(P);
+}
+
 __global__ void possible_pairs_kernel(const long long* n_frags, const long long* max_frag, int n_chrom, long long R,
                                       int nkeys, long long* possible) {
     int k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -404,15 +446,7 @@ int launch_fit(FitParams& P, size_t workspace_bytes, cudaStream_t st) {
 
 }  // namespace
 
-extern "C" size_t bbk_fit_workspace_bytes(int32_t max_bins, int32_t nkeys) {
-    size_t m = max_bins > 4 ? (size_t)max_bins : 4;
-    size_t a = (size_t)3 * nkeys + m + 2;
-    size_t b = bbk_coop_ws_doubles((int)m) + 2 * m;
-    size_t c = 3 * (m + 4) + (size_t)4 * nkeys + 8;
-    size_t mx = a > b ? a : b;
-    mx = mx > c ? mx : c;
-    return (mx + 16) * sizeof(double);
-}
+extern "C" size_t bbk_fit_workspace_bytes(int32_t max_bins, int32_t nkeys) { return fit_workspace_bytes(max_bins, nkeys); }
 
 extern "C" int bbk_possible_pairs(const int64_t* d_n_frags, const int64_t* d_max_frag, int32_t n_chrom, int64_t resolution,
                                   int32_t nkeys, int64_t* d_possible, void* stream) {
@@ -462,4 +496,17 @@ extern "C" int bbk_fit_from_bins(const double* d_x_in, const double* d_y_in, int
     P.bin_of_key = nullptr; P.spline_y = d_spline_y; P.spline_raw = d_spline_raw; P.knots = d_knots; P.coefs = d_coefs;
     P.gws = (double*)d_workspace;
     return launch_fit(P, bbk_fit_workspace_bytes(m, nkeys), (cudaStream_t)stream);
+}
+
+extern "C" int bbk_fit_batched(const BbkFitProblem* d_problems, int32_t n_problems, int32_t n_bins, int64_t resolution,
+                               int64_t min_dist, int64_t max_dist, void* stream) {
+    BBK_REQUIRE(n_problems >= 0 && resolution > 0, "bbk_fit_batched: bad sizes");
+    if (n_problems == 0) return BBK_OK;
+    BBK_REQUIRE(d_problems, "bbk_fit_batched: null pointer");
+    const size_t pool = fit_pool_bytes();
+    BBK_CHECK_CUDA(cudaFuncSetAttribute(fit_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pool));
+    fit_batched_kernel<<<n_problems, FIT_THREADS, pool, (cudaStream_t)stream>>>(d_problems, n_bins, resolution, min_dist, max_dist,
+                                                                               pool / sizeof(double));
+    BBK_CHECK_LAUNCH("fit_batched_kernel");
+    return BBK_OK;
 }

@@ -339,6 +339,239 @@ class GenomePass(object):
         return self.finish()
 
 
+class ChromosomePass(object):
+    """Fit-Hi-C once per chromosome, every chromosome in one pass on this GPU: the authors' workflow (one run per chromosome,
+    datatypes.pyx:26) without one fit launch, one q-value step and one host synchronisation per chromosome.
+
+    engines[i]: the PassEngine of chromosome i, set up with that chromosome's fragments only (its own possible pairs, distance
+    table, fit buffers and histogram); every engine has the same resolution / n_bins / distance limits and the same bias
+    tables (or none).  shards[i]: its records, one compact Shard (chrom = its id).  Chromosome i's result equals a GenomePass
+    over engines[i] and shards[i] alone, bit for bit.  Streaming K4 only: the conditions of GenomePass.listed must hold.
+
+        per chromosome (three streams): K1              ->  ONE bbk_fit_batched
+        ->  per chromosome (three streams): guard, streaming K4, patch pass  ->  ONE bbk_bh_qvalues_segmented
+    """
+
+    def __init__(self, engines, shards, q_values=True, list_capacity=None, cand_capacity=None):
+        if len(engines) != len(shards) or not engines:
+            raise ValueError("one engine per shard, at least one")
+        self.engs, self.shards = list(engines), list(shards)
+        e0 = self.engs[0]
+        self.lib, self.device = e0.lib, e0.device
+        for e in self.engs:
+            if (e.R, e.n_bins, e.min_dist, e.max_dist, e.bias) != (e0.R, e0.n_bins, e0.min_dist, e0.max_dist, e0.bias):
+                raise ValueError("every chromosome's engine needs the same resolution, n_bins, distance limits and bias tables")
+        if not (0 <= e0.min_dist <= e0.max_dist and e0.max_dist + e0.R < (1 << 31) and e0.R >= 2) or \
+                (e0.bias is not None and e0.bias.step == 1):
+            raise ValueError("ChromosomePass runs the streaming K4 only (GenomePass.listed)")
+        if any(sh.chr1 is not None for sh in self.shards):
+            raise ValueError("ChromosomePass takes one-chromosome shards (no chromosome columns)")
+        self.q_values = bool(q_values)
+        n = len(self.engs)
+        dev = self.device
+        self.offsets, self.rows = layout_rows([sh.n for sh in self.shards])
+        if self.rows >= (1 << 32):
+            raise ValueError("more than 2^32 records on one GPU")
+        m = max(self.rows, 4)
+        self.p = torch.full((m,), float("nan"), dtype=torch.float64, device=dev)
+        self.q = torch.full((m,), float("nan"), dtype=torch.float64, device=dev) if self.q_values else None
+        ns = ctypes.sizeof(_lib.ScoreState)
+        self.score_state = torch.zeros(n * ns, dtype=torch.uint8, device=dev)
+        self.p_hist = torch.zeros(n * _lib.PHIST_LEN, dtype=torch.int64, device=dev)
+        self.lists = [None] * n
+        self.cands = [None] * n
+        for i, sh in enumerate(self.shards):
+            mi = max((sh.n + 3) & ~3, 4)
+            self._alloc_list(i, int(list_capacity) if list_capacity else min(mi, max(1 << 20, mi // 4)))
+            if self.q_values:
+                cc = int(cand_capacity) if cand_capacity else min(mi, max(1 << 20, mi // 16))
+                keys = torch.empty(cc, dtype=torch.int64, device=dev)
+                rows = torch.empty(cc, dtype=torch.int32, device=dev)
+                self.cands[i] = (keys, rows, _lib.Candidates(keys.data_ptr(), rows.data_ptr(), cc))
+        if self.q_values:
+            self.seg_off = torch.tensor(self.offsets + [self.rows], dtype=torch.int64, device=dev)
+            segs = (_lib.BhSegment * n)()
+            for i in range(n):
+                segs[i].d_p_hist = self.p_hist[i * _lib.PHIST_LEN:].data_ptr()
+                segs[i].d_state = self.score_state[i * ns:].data_ptr()
+                segs[i].cands = self.cands[i][2]
+                segs[i].n_tests = -1
+            self._segs_host = segs
+            self.segs = torch.zeros(ctypes.sizeof(segs), dtype=torch.uint8, device=dev)
+            self.bh_ws = torch.empty(int(self.lib.bbk_bh_segmented_workspace_bytes(m, n)), dtype=torch.uint8, device=dev)
+            self.n_tests = None
+        self.problems = torch.zeros(n * ctypes.sizeof(_lib.FitProblem), dtype=torch.uint8, device=dev)
+        self._set_problems()
+        self.smoothing = [None] * n
+        nf = e0.fit_result.numel()
+        self._host = torch.zeros(n * (nf + ns), dtype=torch.uint8).pin_memory()
+        self._sides = [torch.cuda.Stream(dev) for _ in range(2)]
+        self._ev = [torch.cuda.Event() for _ in range(3)]
+        self.launches = 0
+
+    def _alloc_list(self, i, cap):
+        dev = self.device
+        row = torch.empty(cap, dtype=torch.int32, device=dev)
+        cnt = torch.empty(cap, dtype=torch.int32, device=dev)
+        prior = torch.empty(cap, dtype=torch.float64, device=dev)
+        self.lists[i] = (row, cnt, prior, _lib.DeferredList(row.data_ptr(), cnt.data_ptr(), prior.data_ptr(), cap))
+
+    def _set_problems(self):
+        """The device array of fit descriptors (again after grow_bins has replaced an engine's buffers)."""
+        probs = (_lib.FitProblem * len(self.engs))()
+        for pr, e in zip(probs, self.engs):
+            pr.d_possible, pr.d_obs_sum, pr.d_totals = e.possible.data_ptr(), e.obs_sum.data_ptr(), e.totals.data_ptr()
+            pr.d_result, pr.d_x, pr.d_y, pr.d_bin_of_key = e.fit_result.data_ptr(), e.x.data_ptr(), e.y.data_ptr(), e.bin_of_key.data_ptr()
+            pr.d_spline_y, pr.d_spline_raw = e.spline_y.data_ptr(), e.spline_raw.data_ptr()
+            pr.d_knots, pr.d_coefs = e.knots.data_ptr(), e.coefs.data_ptr()
+            pr.d_workspace, pr.workspace_bytes = e.fit_ws.data_ptr(), e.fit_ws.numel()
+            pr.nkeys, pr.max_bins = e.nkeys, e.max_bins
+        self.problems.copy_(torch.frombuffer(bytearray(bytes(probs)), dtype=torch.uint8))
+
+    def chrom_p(self, i):
+        return self.p[self.offsets[i]:self.offsets[i] + self.shards[i].n]
+
+    def chrom_q(self, i):
+        return self.q[self.offsets[i]:self.offsets[i] + self.shards[i].n]
+
+    def _lanes(self, main):
+        """Stream pointers of three lanes (main and two side streams that start after what main holds so far)."""
+        self._ev[0].record(main)
+        for sd in self._sides:
+            sd.wait_event(self._ev[0])
+        return [_lib.stream_ptr(x) for x in [main] + self._sides]
+
+    def _join(self, main):
+        for sd, ev in zip(self._sides, self._ev[1:]):
+            ev.record(sd)
+            main.wait_event(ev)
+
+    def enqueue(self, n_tests=None, marks=None):
+        """Enqueue the whole pass on the current stream; no host synchronisation.  n_tests: None (every chromosome's N is its
+        number of emitted rows) or one value per chromosome (-1 = that default).  marks: as GenomePass.enqueue."""
+        lib, R = self.lib, self.engs[0]
+        main = torch.cuda.current_stream(self.device)
+        st = _lib.stream_ptr(main)
+        ns = ctypes.sizeof(_lib.ScoreState)
+
+        def mark(name):
+            if marks is not None:
+                ev = torch.cuda.Event(enable_timing=True)
+                ev.record(main)
+                marks[name] = ev
+
+        want_q = self.q_values
+        if want_q:
+            nt = [-1] * len(self.engs) if n_tests is None else [int(x) for x in n_tests]
+            if nt != self.n_tests:
+                for i, v in enumerate(nt):
+                    self._segs_host[i].n_tests = v
+                self.segs.copy_(torch.frombuffer(bytearray(bytes(self._segs_host)), dtype=torch.uint8))
+                self.n_tests = nt
+        mark("start")
+        self.score_state.zero_()
+        self.launches += 1
+        if want_q:
+            self.p_hist.zero_()
+            self.launches += 1
+        lanes = self._lanes(main)
+        for i, (e, sh) in enumerate(zip(self.engs, self.shards)):
+            li = lanes[i % 3]
+            _lib.check(lib.bbk_hist_init(_lib.ptr(e.obs_sum), e.nkeys, _lib.ptr(e.totals), li), "bbk_hist_init")
+            _lib.check(lib.bbk_hist_pairs(None, None, _lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, e.R, e.min_dist,
+                                          e.max_dist, e.nkeys, _lib.ptr(e.obs_sum), _lib.ptr(e.totals), li), "bbk_hist_pairs")
+            self.launches += 2
+        self._join(main)
+        mark("hist")
+        for i, e in enumerate(self.engs):
+            if self.smoothing[i] is not None:         # this chromosome gets the reference's own s (PassEngine.reference_smoothing)
+                req = _lib.FitResult()
+                req.status = _lib.FIT_S_GIVEN
+                req.smoothing = float(self.smoothing[i])
+                e.fit_result.copy_(torch.frombuffer(bytearray(bytes(req)), dtype=torch.uint8))
+        _lib.check(lib.bbk_fit_batched(_lib.ptr(self.problems), len(self.engs), R.n_bins, R.R, R.min_dist, R.max_dist, st),
+                   "bbk_fit_batched")
+        self.launches += 1
+        mark("fit")
+        lanes = self._lanes(main)
+        for i, (e, sh) in enumerate(zip(self.engs, self.shards)):
+            li = lanes[i % 3]
+            state = ctypes.c_void_p(self.score_state.data_ptr() + i * ns)
+            hist = ctypes.c_void_p(self.p_hist.data_ptr() + i * 8 * _lib.PHIST_LEN) if want_q else None
+            cands = ctypes.byref(self.cands[i][2]) if want_q else None
+            q = _lib.ptr(self.q) if want_q else None
+            bias = ctypes.byref(e.bias.struct) if e.bias is not None else None
+            flags = _lib.ptr(e.bias.flags) if e.bias is not None else None
+            deferred = ctypes.byref(self.lists[i][3])
+            _lib.check(lib.bbk_score_guard(_lib.ptr(e.fit_result), _lib.ptr(e.spline_y), state, li), "bbk_score_guard")
+            self.launches += 1
+            if sh.n:
+                _lib.check(lib.bbk_score_pairs(_lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, sh.chrom, e.R, e.min_dist,
+                                               e.max_dist, _lib.ptr(e.fit_result), _lib.ptr(e.spline_y), bias, flags, self.offsets[i],
+                                               _lib.ptr(self.p), q, hist, cands, deferred, state, li), "bbk_score_pairs")
+                self.launches += 1
+            _lib.check(lib.bbk_score_deferred(deferred, _lib.ptr(e.fit_result), _lib.ptr(self.p), q, hist, cands, state, li),
+                       "bbk_score_deferred")
+            self.launches += 1
+        self._join(main)
+        mark("pvalues")
+        if want_q and self.rows:
+            _lib.check(lib.bbk_bh_qvalues_segmented(_lib.ptr(self.p), self.rows, _lib.ptr(self.seg_off), _lib.ptr(self.segs),
+                                                    len(self.engs), _lib.ptr(self.q), _lib.ptr(self.bh_ws), self.bh_ws.numel(), st),
+                       "bbk_bh_qvalues_segmented")
+            self.launches += 5          # threshold, candidate filter, pass over p (returns at once), rank, ones fix
+        mark("bh")
+
+    def read_state(self):
+        """[(FitResult bytes, ScoreState)] of every chromosome after ONE synchronisation."""
+        nf, ns, n = self.engs[0].fit_result.numel(), ctypes.sizeof(_lib.ScoreState), len(self.engs)
+        for i, e in enumerate(self.engs):
+            self._host[i * nf:(i + 1) * nf].copy_(e.fit_result, non_blocking=True)
+        self._host[n * nf:].copy_(self.score_state, non_blocking=True)
+        torch.cuda.current_stream(self.device).synchronize()
+        raw = self._host.numpy().tobytes()
+        return [(raw[i * nf:(i + 1) * nf], _lib.ScoreState.from_buffer_copy(raw[n * nf + i * ns:n * nf + (i + 1) * ns]))
+                for i in range(n)]
+
+    def finish(self):
+        """Wait for the pass and make it final, chromosome by chromosome as GenomePass.finish does: a chromosome with more bins
+        than its buffers hold gets room for one per key, one whose s is not the reference's own gets that s, one whose deferred
+        list overflowed gets a list as long as its rows, and the pass repeats (at most 6 times; the other chromosomes come out
+        the same, every stage being deterministic).  A failed fit raises what the reference would raise for that chromosome
+        alone, naming it; chromosomes are checked in ascending order.  Returns the FitResults."""
+        for _ in range(6):
+            state = self.read_state()
+            grown = [i for i, (raw, _) in enumerate(state)
+                     if _lib.FitResult.from_buffer_copy(raw).status == _lib.FIT_TOO_MANY_BINS and self.engs[i].grow_bins()]
+            if grown:
+                self._set_problems()
+                self.enqueue(self.n_tests if self.q_values else None)
+                continue
+            fits, again = [], False
+            for i in sorted(range(len(self.engs)), key=lambda j: self.shards[j].chrom):
+                raw, score = state[i]
+                try:
+                    fit = PassEngine.decode_fit(raw)
+                except Exception as e:
+                    from .fithic import naming_chromosome
+                    raise naming_chromosome(e, self.shards[i].chrom)
+                s_ref = PassEngine.reference_smoothing(fit)
+                if s_ref is not None:
+                    self.smoothing[i], again = s_ref, True
+                if score.overflow:
+                    self._alloc_list(i, max((self.shards[i].n + 3) & ~3, 4))
+                    again = True
+            if not again:
+                self.last_state = state
+                return [PassEngine.decode_fit(raw) for raw, _ in state]
+            self.enqueue(self.n_tests if self.q_values else None)
+        raise _lib.BbkError("the per-chromosome pass did not settle after 6 attempts")
+
+    def run(self, n_tests=None):
+        self.enqueue(n_tests)
+        return self.finish()
+
+
 class HostStream(object):
     """Successive passes streamed from pinned host memory through one GenomePass (the end-to-end call of this rank).
 

@@ -403,15 +403,21 @@ def _run_pass(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1
             p_rows = torch.cat([gp.shard_p(i) for i in range(len(shards))])
             q_rows = torch.cat([gp.shard_q(i) for i in range(len(shards))]) if want_q else None
 
+    out = _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows if want_q else None, first, dev)
+    out.rows = (lo, hi)
+    return out
+
+
+def _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows, first, dev):
+    """PassOutput of one finished pass: the engine's tables and fit, p / q / keep of the given rows."""
     out = PassOutput()
     out.fit = fit
     out.frag = info
-    out.rows = (lo, hi)
     host = {"x": _to_host(eng.x[:fit.n_out]), "y": _to_host(eng.y[:fit.n_out]),
             "spline_y": _to_host(eng.spline_y[:fit.L]), "spline_raw": _to_host(eng.spline_raw[:fit.L]),
             "possible": _to_host(eng.possible), "observed": _to_host(eng.obs_sum), "bin_of_key": _to_host(eng.bin_of_key),
             "totals": _to_host(eng.totals), "first": _to_host(first) if first is not None else None}
-    out.p, out.q, out.keep = _scores_to_host(p_rows, q_rows if want_q else None, dev)    # keep: fithic.py:434 (NaN = not scored or dropped)
+    out.p, out.q, out.keep = _scores_to_host(p_rows, q_rows, dev)    # keep: fithic.py:434 (NaN = not scored or dropped)
     torch.cuda.current_stream(dev).synchronize()
     out.x = host["x"].numpy()
     out.y = host["y"].numpy()
@@ -437,6 +443,149 @@ def _run_pass(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1
     return out
 
 
+def split_chromosomes(chr1, chr2, frag_chrom, n_tests=None, refit=False, group=None):
+    """The argument checks and the input split of fit_transform_arrays(per_chromosome=True), on the host alone.
+
+    Returns [(chrom, lo, hi, frag_rows, n_tests_c)] in ascending chromosome order: the chromosome's rows are rows [lo, hi)
+    of the record table, its fragments are frag_rows (indices into frag_chrom) and n_tests_c its N (None: its own number of
+    emitted rows).  n_tests: None, one value for every chromosome, or a mapping {chrom: n} (a chromosome it does not name
+    gets None).  Raises ValueError for inter-chromosomal rows or a chromosome whose rows are not contiguous, and
+    NotImplementedError for refit=True or a process group."""
+    if group is not None:
+        raise NotImplementedError("per_chromosome=True runs on one GPU (group must be None)")
+    if refit:
+        raise NotImplementedError("per_chromosome=True does not take refit=True")
+    if chr1 is None or chr2 is None:
+        raise ValueError("per_chromosome=True needs the chromosome columns chr1 and chr2")
+    c1, c2 = np.asarray(chr1), np.asarray(chr2)
+    if c1.shape != c2.shape or c1.ndim != 1:
+        raise ValueError("chr1 and chr2 must be one-dimensional and of the same length")
+    bad = np.flatnonzero(c1 != c2)
+    if bad.size:
+        raise ValueError("per_chromosome=True takes intra-chromosomal rows only; row %d has chr1 %d and chr2 %d"
+                         % (bad[0], c1[bad[0]], c2[bad[0]]))
+    n = int(c1.size)
+    if n == 0:
+        return []
+    cuts = np.flatnonzero(c1[1:] != c1[:-1]) + 1
+    starts = np.concatenate([[0], cuts]).astype(np.int64)
+    ends = np.concatenate([cuts, [n]]).astype(np.int64)
+    ids = c1[starts].astype(np.int64)
+    uniq, cnt = np.unique(ids, return_counts=True)
+    if (cnt > 1).any():
+        raise ValueError("the rows of chromosome %d are not contiguous: per_chromosome=True needs every chromosome's rows "
+                         "in one block" % uniq[cnt > 1][0])
+    fc = np.asarray(frag_chrom)
+    mapping = hasattr(n_tests, "keys")
+    if mapping:
+        n_tests = {int(k): v for k, v in n_tests.items()}
+    plan = []
+    for j in np.argsort(ids, kind="stable"):
+        c = int(ids[j])
+        nt = n_tests.get(c) if mapping else n_tests
+        plan.append((c, int(starts[j]), int(ends[j]), np.flatnonzero(fc == c), None if nt is None else int(nt)))
+    return plan
+
+
+def naming_chromosome(e, chrom):
+    """An exception of the type of e whose message starts with the chromosome it is about (e itself when its type does not
+    take a message); .chrom holds the id."""
+    try:
+        err = type(e)("chromosome %d: %s" % (chrom, e))
+    except Exception:
+        err = e
+    err.chrom = int(chrom)
+    return err
+
+
+def _own_bias_step(sub, resolution):
+    """The grid step _bias_tables would give a chromosome's bias loci on their own."""
+    mids = np.asarray(sub[0], dtype=np.int64)
+    off = mids - mids.min()
+    R = int(resolution)
+    return int(np.gcd.reduce(np.concatenate([[R], off[off > 0]]))) if (off > 0).any() else R
+
+
+def _run_per_chromosome(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1, mid1, chr2, mid2, count, bias,
+                        want_q, n_tests, refit, group):
+    """fit_transform_arrays(per_chromosome=True): {chrom: PassOutput}, each equal to the call for that chromosome alone.
+    Chromosomes go through one distributed.ChromosomePass when the streaming K4 applies to them (the distance limits allow it
+    and their bias loci lie on the fragment grid, as they would alone); the others, and every chromosome when the limits do
+    not allow it, through single calls."""
+    from .distributed import ChromosomePass
+    plan = split_chromosomes(chr1, chr2, frag_chrom, n_tests, refit, group)
+    if not plan:
+        return {}
+    R = int(resolution)
+    fc, fm = np.asarray(frag_chrom), np.asarray(frag_mid)
+    c1, c2 = np.asarray(chr1), np.asarray(chr2)
+    bias_all = _bias_dict_from_arrays(*bias) if bias is not None else {}
+
+    def bias_of(c):
+        return {c: bias_all[c]} if c in bias_all else None
+
+    def single(c, lo, hi, fsel, nt):
+        out = _run_pass(R, n_bins, min_dist, max_dist, fc[fsel], fm[fsel], c1[lo:hi], mid1[lo:hi], c2[lo:hi], mid2[lo:hi],
+                        count[lo:hi], bias_of(c), want_q=want_q, n_tests=nt)
+        out.rows = (lo, hi)
+        return out
+
+    listed = 0 <= min_dist <= max_dist and max_dist + R < (1 << 31) and R >= 2
+    batch = [x for x in plan if listed and len(x[3]) and (x[0] not in bias_all or _own_bias_step(bias_all[x[0]], R) == R)]
+    out, failed = {}, None
+    if batch:
+        dev = _device()
+        tables = None
+        if any(x[0] in bias_all for x in batch):
+            try:
+                tables = _bias_tables({x[0]: bias_all[x[0]] for x in batch if x[0] in bias_all}, R, dev)
+            except NotImplementedError:              # together the tables are too large: one chromosome at a time
+                batch = []
+    if batch:
+        engines, shards, infos = [], [], []
+        for c, lo, hi, fsel, nt in batch:
+            info = _frag_info(fc[fsel], fm[fsel], R)
+            eng = PassEngine(R, n_bins, min_dist, max_dist, info.nkeys, dev)
+            eng.set_fragments(info.n_frags, info.max_frag)
+            if tables is not None:
+                eng.set_bias(tables)
+            cols = []
+            for a in (mid1, mid2, count):
+                t = _to_device_i32(a, dev, lo, hi)
+                cols.append(t.clone() if t.data_ptr() & 15 else t)     # the streaming K4 reads 16-byte aligned columns
+            engines.append(eng)
+            shards.append(Shard(*cols, chrom=c))
+            infos.append(info)
+        cp = ChromosomePass(engines, shards, q_values=want_q)
+        try:
+            fits = cp.run([-1 if x[4] is None else x[4] for x in batch])
+        except Exception as e:
+            if getattr(e, "chrom", None) is None:
+                raise
+            failed = (e.chrom, e)
+        else:
+            launches = cp.launches + sum(e.launches for e in engines)
+            for i, (c, lo, hi, fsel, nt) in enumerate(batch):
+                o = _pass_output(engines[i], fits[i], infos[i], R, min_dist, max_dist, cp.chrom_p(i),
+                                 cp.chrom_q(i) if want_q else None, None, dev)
+                o.rows = (lo, hi)
+                o.gpu_launches = launches
+                out[c] = o
+    in_batch = set(x[0] for x in batch)
+    for c, lo, hi, fsel, nt in plan:
+        if c in in_batch:
+            continue
+        if failed is not None and c > failed[0]:
+            break
+        try:
+            out[c] = single(c, lo, hi, fsel, nt)
+        except Exception as e:
+            raise naming_chromosome(e, c)
+    if failed is not None:
+        raise failed[1]
+    return {c: out[c] for c, _, _, _, _ in plan}
+
+
 class FitHiC(object):
     """Fit-Hi-C transformer object (fithic.py:49-108) - same constructor, same fit_transform."""
 
@@ -454,7 +603,7 @@ class FitHiC(object):
                interactions, fragments, biases, verbose)
 
     def fit_transform_arrays(self, chr1, mid1, chr2, mid2, count, frag_chrom, frag_mid, bias=None,
-                             q_values=False, n_tests=None, refit=False, group=None):
+                             q_values=False, n_tests=None, refit=False, group=None, per_chromosome=False):
         """The same pass on in-memory records.
 
         chr1/chr2: integer chromosome ids per record (None: all records on one chromosome).
@@ -469,7 +618,18 @@ class FitHiC(object):
         shard_rows(n, world, r) of the table - PassOutput.rows says which, p / q / keep cover those rows only; the
         distance table, S, the bins and the spline are genome-wide (one all-reduce), and so are the q-values
         (distributed.GenomePass).  group=True: the default process group; or any ProcessGroup; None = this GPU alone.
+        per_chromosome: Fit-Hi-C once per chromosome, as the authors ran it (one run per chromosome, datatypes.pyx:26).
+        Returns {chrom id: PassOutput}; out[c] equals this call on c's rows, c's fragments and c's bias rows alone (every
+        field but gpu_launches, which counts the whole pass), and out[c].rows is the range of c's rows in the input.
+        n_tests may then also be a mapping {chrom: n}.  Every chromosome's rows must be one contiguous block and
+        intra-chromosomal (else ValueError); refit and group are not supported (NotImplementedError).  With the streaming
+        K4 (0 <= min_dist <= max_dist, max_dist + resolution < 2^31) every chromosome's fit runs in one launch and the
+        q-values in one step (distributed.ChromosomePass); otherwise it is the loop of single calls.  A chromosome whose
+        call alone would raise makes this call raise the same exception type, naming the chromosome (lowest id first).
         """
+        if per_chromosome:
+            return _run_per_chromosome(self.resolution, self.n_bins, self.min_dist, self.max_dist, frag_chrom, frag_mid, chr1,
+                                       mid1, chr2, mid2, count, bias, q_values, n_tests, refit, group)
         bias_dic = None
         if bias is not None:
             bias_dic = _bias_dict_from_arrays(*bias)

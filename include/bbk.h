@@ -43,6 +43,7 @@ extern "C" {
 #define BBK_FIT_S_ZERO (-14)           /* reference: ZeroDivisionError at fithic.py:216 */
 #define BBK_FIT_X_NOT_INCREASING (-15)
 #define BBK_FIT_EMPTY_GRID (-16)       /* no distance key inside [min(x), max(x)] */
+#define BBK_FIT_BAD_PROBLEM (-17)      /* bbk_fit_batched: a problem's sizes, pointers or workspace do not allow the fit */
 #define BBK_FIT_S_GIVEN 7777            /* INPUT value of BbkFitResult.status: use BbkFitResult.smoothing as s (see bbk_fit) */
 
 int bbk_version(void);
@@ -134,6 +135,32 @@ int bbk_fit(const int64_t* d_possible, const int64_t* d_obs_sum, int32_t nkeys, 
             BbkFitResult* d_result, double* d_x, double* d_y, int32_t* d_bin_of_key, double* d_spline_y,
             double* d_spline_raw, double* d_knots, double* d_coefs, void* d_workspace, size_t workspace_bytes,
             void* stream);
+/* Many independent fits in ONE launch (one CTA each, grid = n_problems), e.g. one per chromosome: the authors ran Fit-Hi-C
+ * once per chromosome (datatypes.pyx:26), each run with its own calculate_probabilities (fithic.py:160-227) and fit_spline
+ * (fithic.py:340-374).  Problem i is exactly bbk_fit with the tables and outputs of d_problems[i] and the shared n_bins,
+ * resolution, min_dist and max_dist; each result struct carries its own BBK_FIT_S_GIVEN input.  d_problems: a DEVICE array
+ * of n_problems descriptors owned by the caller.  A problem whose sizes, pointers or workspace (below
+ * bbk_fit_workspace_bytes(max_bins, nkeys)) do not allow the fit gets status BBK_FIT_BAD_PROBLEM and writes nothing else;
+ * the other problems are not affected. */
+typedef struct BbkFitProblem {
+    const int64_t* d_possible;
+    const int64_t* d_obs_sum;
+    const int64_t* d_totals;
+    BbkFitResult* d_result;
+    double* d_x;
+    double* d_y;
+    int32_t* d_bin_of_key;
+    double* d_spline_y;
+    double* d_spline_raw;
+    double* d_knots;
+    double* d_coefs;
+    void* d_workspace;
+    uint64_t workspace_bytes;
+    int32_t nkeys;
+    int32_t max_bins;
+} BbkFitProblem;
+int bbk_fit_batched(const BbkFitProblem* d_problems, int32_t n_problems, int32_t n_bins, int64_t resolution, int64_t min_dist,
+                    int64_t max_dist, void* stream);
 /* stage-injection entry for tests: the spline + antitonic part alone on given bin means x, y */
 int bbk_fit_from_bins(const double* d_x_in, const double* d_y_in, int32_t m, int32_t nkeys, int64_t resolution,
                       BbkFitResult* d_result, double* d_spline_y, double* d_spline_raw, double* d_knots,
@@ -316,6 +343,23 @@ int bbk_bh_fix_ones_dev(const double* d_p, int64_t m, const double* d_q_ones, do
 int bbk_bh_qvalues_listed(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist, double* d_q,
                           const BbkCandidates* cands, const BbkScoreState* d_state, void* d_workspace, size_t workspace_bytes,
                           void* stream);
+/* Per-chromosome q-values in one step: the authors ran Fit-Hi-C once per chromosome, so each chromosome's q-values come from its
+ * own benjamini_hochberg_correction (fithic.py:466-487) over its own p-values.  Segment s is rows [d_offsets[s], d_offsets[s+1])
+ * of d_p / d_q (d_offsets: DEVICE int64[n_segments + 1], non-decreasing, every start a multiple of 4 as layout_rows gives, the
+ * last <= m) scored by bbk_score_pairs / bbk_score_deferred with the segment's own histogram, candidate list and score state,
+ * given in d_segments (a DEVICE array of complete descriptors; candidate rows are rows of d_p).  q of every segment equals
+ * bbk_bh_qvalues_listed run on that segment alone, bit for bit, including segments that need the pass over p (saturation at or
+ * above 2^-5, or an overflowed candidate list: decided on the device, and only those segments' rows are read).  The number of
+ * launches does not depend on n_segments (<= 65536).  Workspace: bbk_bh_segmented_workspace_bytes(m, n_segments). */
+typedef struct BbkBhSegment {
+    const int64_t* d_p_hist;         /* BBK_PHIST_LEN: the segment's K4 histogram */
+    const BbkScoreState* d_state;    /* the segment's score state */
+    BbkCandidates cands;             /* the segment's candidate list */
+    int64_t n_tests;                 /* N of the segment; -1 = its number of non-NaN p */
+} BbkBhSegment;
+size_t bbk_bh_segmented_workspace_bytes(int64_t m, int32_t n_segments);
+int bbk_bh_qvalues_segmented(const double* d_p, int64_t m, const int64_t* d_offsets, const BbkBhSegment* d_segments,
+                             int32_t n_segments, double* d_q, void* d_workspace, size_t workspace_bytes, void* stream);
 /* bbk_bh_select from that candidate list */
 int bbk_bh_select_listed(const double* d_p, int64_t m, int64_t n_tests, const int64_t* d_p_hist_global, double* d_q,
                          const BbkCandidates* cands, const BbkScoreState* d_score, uint64_t* d_keys, uint32_t* d_idx,
