@@ -112,16 +112,37 @@ class GenomePass(object):
         self._host = torch.zeros(engine.fit_result.numel() + self.score_state.numel() + 8, dtype=torch.uint8).pin_memory()
         self.n_tests = -1
 
+    @property
+    def launches(self):
+        """Kernel launches counted so far (the engine's counter)."""
+        return self.eng.launches
+
+    @launches.setter
+    def launches(self, n):
+        self.eng.launches = n
+
+    def fit_results(self):
+        """The device BbkFitResult a pass leaves, as a list of one (HostStream copies it with each pass)."""
+        return [self.eng.fit_result]
+
+    def decode_fits(self, raw):
+        """fit_results() bytes -> FitResult; raises what the reference would raise for a failed fit."""
+        return PassEngine.decode_fit(raw)
+
     # ------------------------------------------------------------------ buffers
+    def check_sizes(self, sizes):
+        """Raise ValueError unless shards of these sizes can be attached."""
+        if layout_rows(sizes)[1] >= (1 << 32):
+            raise ValueError("more than 2^32 records on one rank")
+
     def attach(self, shards, p=None, q=None, list_capacity=None, cand_capacity=None):
         """Shards of this rank (engine.Shard).  Row r of shard i is row offsets[i] + r of the rank-local p / q buffers
         (offsets are multiples of 4; the few padding rows in between hold NaN).  p / q: optional caller buffers of
         at least `rows` float64 (16-byte aligned)."""
         dev = self.device
         self.shards = list(shards)
+        self.check_sizes([sh.n for sh in self.shards])
         self.offsets, self.rows = layout_rows([sh.n for sh in self.shards])
-        if self.rows >= (1 << 32):
-            raise ValueError("more than 2^32 records on one rank")
         m = max(self.rows, 4)
         self.p = p if p is not None else torch.empty(m, dtype=torch.float64, device=dev)
         self.q = (q if q is not None else torch.empty(m, dtype=torch.float64, device=dev)) if self.q_values else None
@@ -353,9 +374,10 @@ class ChromosomePass(object):
     """
 
     def __init__(self, engines, shards, q_values=True, list_capacity=None, cand_capacity=None):
+        """shards: the most records each chromosome can have; a later attach() may give any chromosome fewer (0 included)."""
         if len(engines) != len(shards) or not engines:
             raise ValueError("one engine per shard, at least one")
-        self.engs, self.shards = list(engines), list(shards)
+        self.engs = list(engines)
         e0 = self.engs[0]
         self.lib, self.device = e0.lib, e0.device
         for e in self.engs:
@@ -364,42 +386,29 @@ class ChromosomePass(object):
         if not (0 <= e0.min_dist <= e0.max_dist and e0.max_dist + e0.R < (1 << 31) and e0.R >= 2) or \
                 (e0.bias is not None and e0.bias.step == 1):
             raise ValueError("ChromosomePass runs the streaming K4 only (GenomePass.listed)")
-        if any(sh.chr1 is not None for sh in self.shards):
-            raise ValueError("ChromosomePass takes one-chromosome shards (no chromosome columns)")
         self.q_values = bool(q_values)
         n = len(self.engs)
         dev = self.device
-        self.offsets, self.rows = layout_rows([sh.n for sh in self.shards])
-        if self.rows >= (1 << 32):
-            raise ValueError("more than 2^32 records on one GPU")
-        m = max(self.rows, 4)
-        self.p = torch.full((m,), float("nan"), dtype=torch.float64, device=dev)
-        self.q = torch.full((m,), float("nan"), dtype=torch.float64, device=dev) if self.q_values else None
+        self.chroms = [sh.chrom for sh in shards]
+        self.max_sizes = [sh.n for sh in shards]
+        self.check_sizes(self.max_sizes)
         ns = ctypes.sizeof(_lib.ScoreState)
         self.score_state = torch.zeros(n * ns, dtype=torch.uint8, device=dev)
         self.p_hist = torch.zeros(n * _lib.PHIST_LEN, dtype=torch.int64, device=dev)
+        self.shards, self.offsets, self.rows = [], [], 0
+        self.p = self.q = None
         self.lists = [None] * n
         self.cands = [None] * n
-        for i, sh in enumerate(self.shards):
-            mi = max((sh.n + 3) & ~3, 4)
-            self._alloc_list(i, int(list_capacity) if list_capacity else min(mi, max(1 << 20, mi // 4)))
-            if self.q_values:
-                cc = int(cand_capacity) if cand_capacity else min(mi, max(1 << 20, mi // 16))
-                keys = torch.empty(cc, dtype=torch.int64, device=dev)
-                rows = torch.empty(cc, dtype=torch.int32, device=dev)
-                self.cands[i] = (keys, rows, _lib.Candidates(keys.data_ptr(), rows.data_ptr(), cc))
+        self.n_tests = None
         if self.q_values:
-            self.seg_off = torch.tensor(self.offsets + [self.rows], dtype=torch.int64, device=dev)
-            segs = (_lib.BhSegment * n)()
+            self.seg_off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+            self._seg_layout = None
+            self._segs_host = (_lib.BhSegment * n)()
             for i in range(n):
-                segs[i].d_p_hist = self.p_hist[i * _lib.PHIST_LEN:].data_ptr()
-                segs[i].d_state = self.score_state[i * ns:].data_ptr()
-                segs[i].cands = self.cands[i][2]
-                segs[i].n_tests = -1
-            self._segs_host = segs
-            self.segs = torch.zeros(ctypes.sizeof(segs), dtype=torch.uint8, device=dev)
-            self.bh_ws = torch.empty(int(self.lib.bbk_bh_segmented_workspace_bytes(m, n)), dtype=torch.uint8, device=dev)
-            self.n_tests = None
+                self._segs_host[i].d_p_hist = self.p_hist[i * _lib.PHIST_LEN:].data_ptr()
+                self._segs_host[i].d_state = self.score_state[i * ns:].data_ptr()
+            self.segs = torch.zeros(ctypes.sizeof(self._segs_host), dtype=torch.uint8, device=dev)
+            self._segs_nt = None                # the n_tests values self.segs holds (None: not uploaded yet)
         self.problems = torch.zeros(n * ctypes.sizeof(_lib.FitProblem), dtype=torch.uint8, device=dev)
         self._set_problems()
         self.smoothing = [None] * n
@@ -408,6 +417,66 @@ class ChromosomePass(object):
         self._sides = [torch.cuda.Stream(dev) for _ in range(2)]
         self._ev = [torch.cuda.Event() for _ in range(3)]
         self.launches = 0
+        self.attach(shards, list_capacity=list_capacity, cand_capacity=cand_capacity)
+
+    def check_sizes(self, sizes):
+        """Raise ValueError unless shards of these sizes can be attached: one per chromosome, none larger than it was built with."""
+        if len(sizes) != len(self.engs):
+            raise ValueError("one shard per chromosome of the pass (%d), got %d" % (len(self.engs), len(sizes)))
+        for c, n, most in zip(self.chroms, sizes, self.max_sizes):
+            if not 0 <= int(n) <= most:
+                raise ValueError("chromosome %d: %d rows, more than the %d the pass was built with" % (c, int(n), most))
+        if layout_rows(sizes)[1] >= (1 << 32):
+            raise ValueError("more than 2^32 records on one GPU")
+
+    def attach(self, shards, p=None, q=None, list_capacity=None, cand_capacity=None):
+        """Point the pass at other records (one compact Shard per chromosome, in the order and with the ids it was built with,
+        none larger than then) and other p / q buffers of at least `rows` float64 (laid out by layout_rows; the padding rows
+        between chromosomes are set to NaN), keeping the engines, the bias tables and the fit and q-value descriptors.
+        list_capacity / cand_capacity: given, every chromosome's deferred / candidate list is made anew with that many places
+        (at most its built size, which no pass can exceed: such a deferred list cannot overflow); omitted, the lists already
+        attached are kept (the first attach makes them at their default sizes, from the built sizes)."""
+        shards = list(shards)
+        self.check_sizes([sh.n for sh in shards])
+        if any(sh.chr1 is not None for sh in shards):
+            raise ValueError("ChromosomePass takes one-chromosome shards (no chromosome columns)")
+        if [sh.chrom for sh in shards] != self.chroms:
+            raise ValueError("the shards' chromosome ids differ from the pass' %s" % self.chroms)
+        dev = self.device
+        self.shards = shards
+        self.offsets, self.rows = layout_rows([sh.n for sh in shards])
+        m = max(self.rows, 4)
+        for t in (p, q):
+            if t is not None and t.numel() < m:
+                raise ValueError("p / q buffers need at least %d rows" % m)
+        self.p = p if p is not None else torch.full((m,), float("nan"), dtype=torch.float64, device=dev)
+        self.q = (q if q is not None else torch.full((m,), float("nan"), dtype=torch.float64, device=dev)) if self.q_values else None
+        for sh, o in zip(self.shards, self.offsets):
+            if sh.n & 3:
+                self.p[o + sh.n:o + ((sh.n + 3) & ~3)] = float("nan")
+                if self.q is not None:
+                    self.q[o + sh.n:o + ((sh.n + 3) & ~3)] = float("nan")
+        for i, most in enumerate(self.max_sizes):
+            mi = max((most + 3) & ~3, 4)
+            if list_capacity or self.lists[i] is None:
+                self._alloc_list(i, min(mi, int(list_capacity)) if list_capacity else min(mi, max(1 << 20, mi // 4)))
+            if self.q_values and (cand_capacity or self.cands[i] is None):
+                cc = min(mi, int(cand_capacity)) if cand_capacity else min(mi, max(1 << 20, mi // 16))
+                keys = torch.empty(cc, dtype=torch.int64, device=dev)
+                rows = torch.empty(cc, dtype=torch.int32, device=dev)
+                self.cands[i] = (keys, rows, _lib.Candidates(keys.data_ptr(), rows.data_ptr(), cc))
+                self._segs_host[i].cands = self.cands[i][2]
+                self._segs_nt = None
+        if self.q_values:
+            layout = self.offsets + [self.rows]
+            if layout != self._seg_layout:
+                # non_blocking: a pageable source is staged at once, and the stream is not synchronised
+                self.seg_off.copy_(torch.tensor(layout, dtype=torch.int64), non_blocking=True)
+                self._seg_layout = layout
+            need = int(self.lib.bbk_bh_segmented_workspace_bytes(m, len(self.engs)))
+            if getattr(self, "bh_ws", None) is None or self.bh_ws.numel() < need:
+                self.bh_ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        return self
 
     def _alloc_list(self, i, cap):
         dev = self.device
@@ -447,8 +516,10 @@ class ChromosomePass(object):
             main.wait_event(ev)
 
     def enqueue(self, n_tests=None, marks=None):
-        """Enqueue the whole pass on the current stream; no host synchronisation.  n_tests: None (every chromosome's N is its
-        number of emitted rows) or one value per chromosome (-1 = that default).  marks: as GenomePass.enqueue."""
+        """Enqueue the whole pass on the current stream; no host synchronisation.  n_tests: None or -1 (every chromosome's N is
+        its number of emitted rows) or one value per chromosome (-1 = that default).  marks: as GenomePass.enqueue.
+        Chromosome i's fit takes s = smoothing[i] when that is set (finish() sets it to PassEngine.reference_smoothing of the
+        chromosome's fit; a caller that streams passes sets it itself and submits the pass again)."""
         lib, R = self.lib, self.engs[0]
         main = torch.cuda.current_stream(self.device)
         st = _lib.stream_ptr(main)
@@ -460,14 +531,19 @@ class ChromosomePass(object):
                 ev.record(main)
                 marks[name] = ev
 
+        if n_tests is None or (np.ndim(n_tests) == 0 and int(n_tests) == -1):
+            nt = [-1] * len(self.engs)
+        else:
+            nt = [int(x) for x in n_tests]
+            if len(nt) != len(self.engs):
+                raise ValueError("n_tests: one value per chromosome (%d), got %d" % (len(self.engs), len(nt)))
+        self.n_tests = nt
         want_q = self.q_values
-        if want_q:
-            nt = [-1] * len(self.engs) if n_tests is None else [int(x) for x in n_tests]
-            if nt != self.n_tests:
-                for i, v in enumerate(nt):
-                    self._segs_host[i].n_tests = v
-                self.segs.copy_(torch.frombuffer(bytearray(bytes(self._segs_host)), dtype=torch.uint8))
-                self.n_tests = nt
+        if want_q and nt != self._segs_nt:
+            for i, v in enumerate(nt):
+                self._segs_host[i].n_tests = v
+            self.segs.copy_(torch.frombuffer(bytearray(bytes(self._segs_host)), dtype=torch.uint8), non_blocking=True)
+            self._segs_nt = nt
         mark("start")
         self.score_state.zero_()
         self.launches += 1
@@ -488,7 +564,7 @@ class ChromosomePass(object):
                 req = _lib.FitResult()
                 req.status = _lib.FIT_S_GIVEN
                 req.smoothing = float(self.smoothing[i])
-                e.fit_result.copy_(torch.frombuffer(bytearray(bytes(req)), dtype=torch.uint8))
+                e.fit_result.copy_(torch.frombuffer(bytearray(bytes(req)), dtype=torch.uint8), non_blocking=True)
         _lib.check(lib.bbk_fit_batched(_lib.ptr(self.problems), len(self.engs), R.n_bins, R.R, R.min_dist, R.max_dist, st),
                    "bbk_fit_batched")
         self.launches += 1
@@ -547,14 +623,9 @@ class ChromosomePass(object):
                 self._set_problems()
                 self.enqueue(self.n_tests if self.q_values else None)
                 continue
-            fits, again = [], False
-            for i in sorted(range(len(self.engs)), key=lambda j: self.shards[j].chrom):
-                raw, score = state[i]
-                try:
-                    fit = PassEngine.decode_fit(raw)
-                except Exception as e:
-                    from .fithic import naming_chromosome
-                    raise naming_chromosome(e, self.shards[i].chrom)
+            fits = self.decode_fits(b"".join(raw for raw, _ in state))
+            again = False
+            for i, (fit, (_, score)) in enumerate(zip(fits, state)):
                 s_ref = PassEngine.reference_smoothing(fit)
                 if s_ref is not None:
                     self.smoothing[i], again = s_ref, True
@@ -563,7 +634,7 @@ class ChromosomePass(object):
                     again = True
             if not again:
                 self.last_state = state
-                return [PassEngine.decode_fit(raw) for raw, _ in state]
+                return fits
             self.enqueue(self.n_tests if self.q_values else None)
         raise _lib.BbkError("the per-chromosome pass did not settle after 6 attempts")
 
@@ -571,31 +642,54 @@ class ChromosomePass(object):
         self.enqueue(n_tests)
         return self.finish()
 
+    def fit_results(self):
+        """The device BbkFitResult of every chromosome, in the pass' order (HostStream copies them with each pass)."""
+        return [e.fit_result for e in self.engs]
+
+    def decode_fits(self, raw):
+        """fit_results() bytes back to back -> [FitResult], in the pass' order.  A failed fit raises what the reference would
+        raise for that chromosome alone, naming it (fithic.naming_chromosome); the lowest failing id wins."""
+        nf = len(raw) // len(self.engs)
+        for i in sorted(range(len(self.engs)), key=lambda j: self.chroms[j]):
+            try:
+                PassEngine.decode_fit(raw[i * nf:(i + 1) * nf])
+            except Exception as e:
+                from .fithic import naming_chromosome
+                raise naming_chromosome(e, self.chroms[i])
+        return [PassEngine.decode_fit(raw[i * nf:(i + 1) * nf]) for i in range(len(self.engs))]
+
 
 class HostStream(object):
-    """Successive passes streamed from pinned host memory through one GenomePass (the end-to-end call of this rank).
+    """Successive passes streamed from pinned host memory through one GenomePass or ChromosomePass (the end-to-end call of
+    this rank).
 
     A pass cannot start scoring before all of its records are on the device (S and the spline need the whole distance
     table, fithic.py:110-133), so inside one pass the inbound and the outbound copies never overlap; across passes they do:
     `slots` device copies of the record columns and of p / q, three streams (in, run, out) and per-slot events.  The host
     table is three contiguous pinned int32 columns holding this rank's shards back to back (shard i = rows
     starts[i] .. starts[i] + sizes[i], starts = layout_rows(sizes): every start a multiple of 4); p / q come back as pinned
-    float64 columns over the same rows.  Nothing here synchronises the host: call drain() (or wait on the event submit() returns) before reading."""
+    float64 columns over the same rows.  Nothing here synchronises the host: call drain() (or wait on the event submit() returns) before reading.
+
+    With a ChromosomePass every shard is one chromosome (chroms = its ids, in its order; sizes at most those it was built
+    with), each gets its own fit and q-values, and fit_of(k) returns one FitResult per chromosome."""
 
     class _Slot(object):
         pass
 
     def __init__(self, genome_pass, sizes, chroms, slots=2, packed=False, cap_p=None, cap_q=None):
-        """sizes / chroms: records and chromosome of every shard; the slots hold layout_rows(sizes) rows.
-        packed: results cross the host link as two bits per row + the values that are not 1.0 / NaN (bbk_pack_scores);
-        submit_packed() returns a PackedScores whose dense() rebuilds the float64 columns bit for bit.  cap_p / cap_q: rows
-        the packed value lists can hold (default rows / 2 and rows / 16; a pass that needs more comes back dense)."""
+        """genome_pass: a GenomePass or a ChromosomePass.  sizes / chroms: records and chromosome of every shard; the slots hold
+        layout_rows(sizes) rows.  packed: results cross the host link as two bits per row + the values that are not 1.0 / NaN
+        (bbk_pack_scores); submit_packed() returns a PackedScores whose dense() rebuilds the float64 columns bit for bit, over
+        the slot's rows (the padding rows between shards hold NaN; shard i is rows starts[i] .. starts[i] + sizes[i]).
+        cap_p / cap_q: rows the packed value lists can hold (default rows / 2 and rows / 16; a pass that needs more comes back
+        dense)."""
         self.gp = genome_pass
         self.sizes, self.chroms = [int(x) for x in sizes], [int(x) for x in chroms]
         self.starts, rows = layout_rows(self.sizes)
         self.rows = max(rows, 4)
         self.packed = bool(packed)
         dev = genome_pass.device
+        nf = sum(f.numel() for f in genome_pass.fit_results())
         self.slots = []
         for _ in range(int(slots)):
             s = HostStream._Slot()
@@ -604,15 +698,16 @@ class HostStream(object):
             s.q = torch.full((self.rows,), float("nan"), dtype=torch.float64, device=dev) if genome_pass.q_values else None
             s.shards = self._shards(s, self.starts, self.sizes)
             s.in_ready, s.run_done, s.out_done, s.counts_ready = (torch.cuda.Event() for _ in range(4))
-            s.fit = torch.zeros_like(genome_pass.eng.fit_result)
-            s.h_fit = torch.zeros(genome_pass.eng.fit_result.numel(), dtype=torch.uint8).pin_memory()
+            s.fit = torch.zeros(nf, dtype=torch.uint8, device=dev)
+            s.h_fit = torch.zeros(nf, dtype=torch.uint8).pin_memory()
             if self.packed:
                 s.pack = DevicePack(self.rows, dev, genome_pass.q_values, cap_p, cap_q)
                 s.h_pack_state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8).pin_memory()
             s.index = -1
             self.slots.append(s)
         # Nothing here synchronises, so nothing would see BbkScoreState.overflow: the deferred list has a place for every row
-        # of a slot (and later attaches keep it, being no larger).
+        # of a slot (and later attaches keep it, being no larger).  A ChromosomePass caps each chromosome's list at the rows it
+        # was built with, which no pass can exceed.
         genome_pass.attach(s.shards, s.p, s.q, list_capacity=self.rows)
         self.s_in, self.s_run, self.s_out = (torch.cuda.Stream(dev) for _ in range(3))
         self.s_run.wait_stream(torch.cuda.current_stream(dev))
@@ -635,7 +730,8 @@ class HostStream(object):
             if t is not None and (not t.is_pinned() or t.numel() < n):
                 raise ValueError("host columns must be pinned and hold at least %d rows" % n)
         if q_values and s.q is None:
-            raise ValueError("the stream's GenomePass was made with q_values=False")
+            raise ValueError("the stream's pass was made with q_values=False")
+        self.gp.check_sizes(sizes)
         shards = s.shards if sizes is self.sizes else self._shards(s, starts, sizes)
         self.submitted += 1
         s.index = self.submitted - 1
@@ -652,13 +748,18 @@ class HostStream(object):
         gp = self.gp
         with torch.cuda.stream(self.s_run):
             keep_q, gp.q_values = gp.q_values, q_values
-            gp.attach(shards, s.p, s.q)
-            gp.enqueue(n_tests)
-            gp.q_values = keep_q
-            s.fit.copy_(gp.eng.fit_result, non_blocking=True)
+            try:
+                gp.attach(shards, s.p, s.q)
+                gp.enqueue(n_tests)
+            finally:
+                gp.q_values = keep_q
+            o = 0
+            for f in gp.fit_results():
+                s.fit[o:o + f.numel()].copy_(f, non_blocking=True)
+                o += f.numel()
             if pack:
                 s.pack.pack(s.p, s.q, self.s_run)
-                gp.eng.launches += 2
+                gp.launches += 2
             s.run_done.record()
         return s, n
 
@@ -729,12 +830,14 @@ class HostStream(object):
     def fit_of(self, index):
         """Fit result of submission `index` once its outputs are on the host (raises the reference's exception for a failed
         fit); PassEngine.reference_smoothing(result) tells whether that pass must be repeated with the reference's own s.
+        With a ChromosomePass: one FitResult per chromosome, in its order; a failed fit raises for the lowest failing id,
+        naming it, and a chromosome is repeated with its own s by setting pass.smoothing[i] and submitting again.
         Only the last `slots` submissions are held."""
         s = self.slots[int(index) % len(self.slots)]
         if s.index != int(index):
             raise KeyError("submission %d is no longer (or not yet) held by the stream" % int(index))
         s.out_done.synchronize()
-        return PassEngine.decode_fit(s.h_fit.numpy().tobytes())
+        return self.gp.decode_fits(s.h_fit.numpy().tobytes())
 
     def drain(self):
         self._finalize_pending()

@@ -1,12 +1,17 @@
 """Per-chromosome Fit-Hi-C on BASELINE config 3's genome (23 hg19 chromosomes @5kb, all pairs within 10 Mb), generated on the
-device as bench.py does, in three forms:
+device as bench.py does, in these forms:
 
   (a) distributed.ChromosomePass: every chromosome's fit in one launch, every chromosome's q-values in one step;
   (b) the loop the authors' workflow implies: one single-chromosome GenomePass per chromosome, each run to completion;
-  (c) the genome-wide GenomePass (one fit, one ranking over the genome), for reference.
+  (c) the genome-wide GenomePass (one fit, one ranking over the genome), for reference;
+  (d) (a) end to end from pinned host columns: distributed.HostStream(ChromosomePass, packed=True), two device slots, p / q
+      back as two bits per row + the values that are not 1.0 / NaN;
+  (e) the genome-wide pass through HostStream(GenomePass, packed=True) (bench.py's e2e leg), for reference.
 
 Prints one JSON line: the card and its power limit, ms per step, per-stage device times and launches per step of each form,
-and whether (a) equals (b) bit for bit (p, q and the fit of every chromosome).
+whether (a) equals (b) bit for bit (p, q and the fit of every chromosome), and for (d) / (e) the bytes in and out per step, the
+peak device memory allocated from the stream's construction on, and whether the last step's unpacked result equals (a)'s
+device columns (for (d)) bit for bit.
 
     python tools/bench_per_chromosome.py [--steps 5] [--warmup 2]
 """
@@ -55,9 +60,10 @@ def main():
     args = ap.parse_args()
     if args.steps < 1:
         ap.error("--steps must be at least 1")
+    import numpy as np
     import torch
     import bench
-    from blueberry_b200.distributed import ChromosomePass, GenomePass
+    from blueberry_b200.distributed import ChromosomePass, GenomePass, HostStream
     from blueberry_b200.engine import PassEngine
     if not torch.cuda.is_available():
         raise SystemExit("bench_per_chromosome.py needs a CUDA device")
@@ -137,6 +143,8 @@ def main():
         same &= fa[:72] == fb[:72] and fa[184:] == fb[184:]           # all but the SM cycle counters
     out["a_equals_b_bitwise"] = bool(same)
     out["rows"] = int(sum(sh.n for sh in W.shards))
+    a_p, a_q = cp.p.cpu().numpy(), cp.q.cpu().numpy()         # what (d) must give back
+    a_smoothing = list(cp.smoothing)                          # chromosomes (a) repeated with the reference's own s
     del singles, cp
     torch.cuda.empty_cache()
 
@@ -152,6 +160,64 @@ def main():
         _add(acc, _stages(marks), 1.0 / args.steps)
     out["c_genome_wide"] = {"ms_per_step": ms, "launches_per_step": n, "stages_ms": acc}
     out["fit_stage_a_over_c"] = out["a_batched"]["stages_ms"]["fit"] / out["c_genome_wide"]["stages_ms"]["fit"]
+    del gp
+    torch.cuda.empty_cache()
+
+    # (d) and (e): the records come from pinned host columns; the generator's device columns are freed, the slots take their place
+    h_in = [torch.empty(W.rows, dtype=torch.int32).pin_memory() for _ in range(3)]
+    for h, d in zip(h_in, (W.mid1, W.mid2, W.count)):
+        h.copy_(d)
+    cp = ChromosomePass(engines(), W.shards, q_values=True)   # built on the largest sizes a pass may have
+    cp.smoothing = a_smoothing
+    cp.shards, cp.p, cp.q = [], None, None                    # the stream attaches its own slots
+    W.mid1 = W.mid2 = W.count = None
+    W.shards = []
+    torch.cuda.synchronize()
+    torch.cuda.empty_cache()
+    in_rows = W.starts[-1] + W.sizes[-1]
+
+    def stream_leg(pas, launches, want=None):
+        torch.cuda.reset_peak_memory_stats(dev)
+        hs = HostStream(pas, W.sizes, W.chroms, slots=2, packed=True)
+        outs = [hs.packed_buffers() for _ in range(2)]
+
+        def step():
+            hs.submit_packed(h_in[0], h_in[1], h_in[2], outs[hs.submitted % 2])
+
+        for _ in range(args.warmup):
+            step()
+        hs.drain()
+        torch.cuda.synchronize()
+        n0 = launches()
+        step()
+        n = launches() - n0
+        hs.drain()
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        for _ in range(args.steps):          # the last value lists leave the device in drain(): inside the timed region
+            step()
+        hs.drain()
+        torch.cuda.synchronize()
+        ms = (time.perf_counter() - t0) * 1e3 / args.steps
+        peak = torch.cuda.max_memory_allocated(dev)
+        last = outs[(hs.submitted - 1) % 2]
+        fits = hs.fit_of(hs.submitted - 1)
+        fits = fits if isinstance(fits, list) else [fits]
+        res = {"ms_per_step": ms, "launches_per_step": n, "h2d_bytes_per_step": 12 * in_rows,
+               "d2h_bytes_per_step": last.nbytes() + hs.slots[0].h_fit.numel(), "dense_d2h_bytes_per_step": 16 * hs.rows,
+               "packed_values": {"p": last.n_p, "q": last.n_q, "overflow": last.overflow},
+               "peak_alloc_gib_from_stream_construction": peak / 2 ** 30,
+               "fits_needing_resubmission": sum(PassEngine.reference_smoothing(f) is not None for f in fits)}
+        if want is not None:
+            p, q = last.dense()
+            res["unpacked_equals_a_bitwise"] = bool(np.array_equal(p.view(np.uint64), want[0].view(np.uint64)) and
+                                                    np.array_equal(q.view(np.uint64), want[1].view(np.uint64)))
+        return res
+    out["d_chromosome_stream"] = stream_leg(cp, lambda: cp.launches, (a_p, a_q))
+    del cp
+    torch.cuda.empty_cache()
+    out["e_genome_stream"] = stream_leg(GenomePass(W.eng, group=False, q_values=True), lambda: W.eng.launches)
+    out["d_over_e_ms"] = out["d_chromosome_stream"]["ms_per_step"] / out["e_genome_stream"]["ms_per_step"]
     print(json.dumps(out))
 
 
