@@ -15,7 +15,7 @@ import os
 import numpy as np
 import pytest
 
-from helpers import PASS_CASES, golden_bias_dict, load_golden, log10_close
+from helpers import PASS_CASES, golden_bias_dict, load_golden, log10_close, score_table, truth
 
 pytestmark = pytest.mark.gpu
 
@@ -95,25 +95,6 @@ def test_bin_membership_bit_exact(name, torch_cuda):
     assert np.array_equal(out.bin_of_key, bok)
 
 
-def _score_table(torch, priors, counts, S, bias=None):
-    """Drive K4 directly: record i looks up priors[i] (mid1 = 0, mid2 = i, resolution 1)."""
-    from blueberry_b200 import _lib
-    from blueberry_b200.engine import PassEngine, Shard
-    n = len(priors)
-    eng = PassEngine(1, 100, 0, n, n, torch.device("cuda:0"))
-    eng.spline_y[:n] = torch.from_numpy(np.asarray(priors, dtype=np.float64)).cuda()
-    fr = _lib.FitResult(status=0, n_out=100, k0=0, L=n, n_knots=8, ier=0, S=int(S), min_x=0.0, max_x=float(n - 1),
-                        residual=0.0, fp=0.0, smoothing=0.0)
-    eng.fit_result.copy_(torch.frombuffer(bytearray(bytes(fr)), dtype=torch.uint8))
-    z = torch.zeros(n, dtype=torch.int32, device="cuda:0")
-    mid2 = torch.arange(n, dtype=torch.int32, device="cuda:0")
-    cnt = torch.from_numpy(np.asarray(counts, dtype=np.int32)).cuda()
-    p = torch.empty((n + 1) & ~1, dtype=torch.float64, device="cuda:0")[:n]
-    eng.pvalues(Shard(z, mid2, cnt), p)
-    torch.cuda.synchronize()
-    return p.cpu().numpy()
-
-
 def _random_tail_cases(rng, n, S):
     mu = 10 ** rng.uniform(-4, 3.3, n)
     mu = np.minimum(mu, S * 0.4)
@@ -131,7 +112,7 @@ def test_pvalue_kernel_against_scipy(S, torch_cuda):
     import scipy.special as sc
     rng = np.random.default_rng(S % 9973)
     q, c = _random_tail_cases(rng, 200_001, S)      # odd length: exercises the scalar tail of the kernel
-    got = _score_table(torch_cuda, q, c, S)
+    got = score_table(torch_cuda, q, c, S)
     with np.errstate(all="ignore"):
         ref = sc.bdtrc((c - 1).astype(np.float64), np.int64(S), q)
     assert not np.isnan(got).any() and not np.isnan(ref).any()
@@ -146,30 +127,11 @@ def test_pvalue_kernel_against_scipy(S, torch_cuda):
 
 def test_pvalue_kernel_against_60_digit_truth(torch_cuda):
     import mpmath as mp
-    mp.mp.dps = 60
     rng = np.random.default_rng(77)
     S = 1_234_567_891
     q, c = _random_tail_cases(rng, 600, S)
     c = np.maximum(c, 2)
-    got = _score_table(torch_cuda, q, c, S)
-
-    def truth(cc, n, qq):
-        qq = mp.mpf(float(qq))
-        lp = mp.loggamma(n + 1) - mp.loggamma(cc + 1) - mp.loggamma(n - cc + 1) + cc * mp.log(qq) + (n - cc) * mp.log(1 - qq)
-        qr = qq / (1 - qq)
-        if cc >= (n + 1) * qq:
-            term = mp.mpf(1); s = mp.mpf(1); j = cc
-            while j < n:
-                term *= mp.mpf(n - j) / (j + 1) * qr; s += term; j += 1
-                if term < mp.mpf(10) ** -45 * s:
-                    break
-            return mp.exp(lp) * s
-        term = mp.mpf(cc) / ((n - cc + 1) * qr); s = term; j = cc - 1
-        while j > 0:
-            term *= mp.mpf(j) / ((n - j + 1) * qr); s += term; j -= 1
-            if term < mp.mpf(10) ** -45 * s:
-                break
-        return 1 - mp.exp(lp) * s
+    got = score_table(torch_cuda, q, c, S)
 
     worst = 0.0
     for i in range(len(c)):
@@ -186,7 +148,7 @@ def test_pvalue_edge_semantics_match_bdtrc(torch_cuda):
     S = 100
     priors = np.array([-0.5, 1.5, 0.5, 0.5, 0.5, 0.0, 1.0, 0.0, 1.0, np.nan, 0.02, 0.005, 0.3, 0.3, -0.1, 0.5])
     counts = np.array([0, 0, 0, -3, 102, 1, 1, 2, 2, 3, 1, 1, 101, 100, 5, 7])
-    got = _score_table(torch_cuda, priors, counts, S)
+    got = score_table(torch_cuda, priors, counts, S)
     with np.errstate(all="ignore"):
         ref = sc.bdtrc((counts - 1).astype(np.float64), np.int64(S), priors)
     ref = np.where(ref <= 1, ref, np.nan)             # fithic.py:434 drops the row
