@@ -16,6 +16,10 @@ SIGNATURES = {
     "bbkio_unpack_scores": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _i32]),
     "bbkio_unpack_scores_keep": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _i32]),
     "bbkio_copy_bytes": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, _i32]),
+    "bbkio_pack_records_bound": (ctypes.c_uint64, [_i64]),
+    "bbkio_pack_records": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(_i64), _i32, _vp,
+                                          ctypes.c_uint64, ctypes.POINTER(ctypes.c_uint64), _i32]),
+    "bbkio_check_records": (ctypes.c_int, [_vp, ctypes.c_uint64, _i64]),
     "bbkio_read_interactions": (ctypes.c_int, [ctypes.c_char_p, _i32, ctypes.POINTER(_vp)]),
     "bbkio_table_rows": (_i64, [_vp]),
     "bbkio_table_n_chrom": (_i32, [_vp]),
@@ -131,3 +135,38 @@ def unpack_scores(codes, chunks, values_p, values_q, m, p_out=None, q_out=None, 
         _raise(lib, "bbkio_unpack_scores", rc)
     return p, q
 
+
+
+def pack_records_bound(rows):
+    """The most bytes the packed records of `rows` layout rows can take (bbk.h, BbkRecHeader)."""
+    return int(load().bbkio_pack_records_bound(int(rows)))
+
+
+def pack_records(shards, out_ptr, capacity, threads=0):
+    """The packed records of shards [(mid1, mid2, count), ...] (int32 columns, numpy or anything numpy views without a copy)
+    laid out by layout_rows, written to the raw host address out_ptr (capacity bytes).  Returns the bytes written; raises
+    ValueError when they do not fit."""
+    lib = load()
+    cols = [[np.ascontiguousarray(c, dtype=np.int32) for c in sh] for sh in shards]
+    for c in cols:
+        if not (len(c) == 3 and len(c[0]) == len(c[1]) == len(c[2])):
+            raise ValueError("a shard is three int32 columns (mid1, mid2, count) of one length")
+    n = len(cols)
+    ptrs = [(_vp * max(n, 1))(*[c[j].ctypes.data for c in cols]) for j in range(3)]
+    sizes = (_i64 * max(n, 1))(*[len(c[0]) for c in cols])
+    used = ctypes.c_uint64(0)
+    rc = lib.bbkio_pack_records(ptrs[0], ptrs[1], ptrs[2], sizes, n, ctypes.c_void_p(out_ptr), int(capacity), ctypes.byref(used), int(threads))
+    if rc != 0:
+        buf = ctypes.create_string_buffer(512)
+        lib.bbkio_last_error(buf, 512)
+        raise ValueError(buf.value.decode(errors="replace"))
+    return int(used.value)
+
+
+def check_records(buf_ptr, nbytes, rows):
+    """Raise ValueError unless the nbytes at buf_ptr are packed records of `rows` rows that bbk_unpack_records may read."""
+    lib = load()
+    if lib.bbkio_check_records(ctypes.c_void_p(buf_ptr), int(nbytes), int(rows)) != 0:
+        buf = ctypes.create_string_buffer(512)
+        lib.bbkio_last_error(buf, 512)
+        raise ValueError(buf.value.decode(errors="replace"))

@@ -119,6 +119,7 @@ SIGNATURES = {
     "bbk_pack_chunks": (_i64, [_i64]),
     "bbk_pack_code_words": (_i64, [_i64]),
     "bbk_pack_scores": (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "bbk_unpack_records": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp]),
     "bbk_bh_qvalues_listed": (ctypes.c_int, [_vp, _i64, _i64, _vp, _vp, ctypes.POINTER(Candidates), _vp, _vp, _sz, _vp]),
     "bbk_bh_segmented_workspace_bytes": (_sz, [_i64, _i32]),
     "bbk_bh_qvalues_segmented": (ctypes.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, _vp, _sz, _vp]),

@@ -50,8 +50,8 @@ def nvcc_path():
 def build_io(force=False, verbose=False):
     os.makedirs(LIBDIR, exist_ok=True)
     src = os.path.join(CSRC, "io_host.cpp")
-    hdr = os.path.join(os.path.dirname(HERE), "include", "bbk_io.h")
-    if not force and os.path.exists(IO_LIB) and os.path.getmtime(IO_LIB) >= max(os.path.getmtime(src), os.path.getmtime(hdr)):
+    deps = [src] + [os.path.join(os.path.dirname(HERE), "include", h) for h in ("bbk_io.h", "bbk.h")]
+    if not force and os.path.exists(IO_LIB) and os.path.getmtime(IO_LIB) >= max(os.path.getmtime(f) for f in deps):
         return IO_LIB
     cmd = [os.environ.get("CXX", "g++"), "-O3", "-std=c++17", "-fPIC", "-shared", "-o", IO_LIB, src, "-lz", "-lpthread"]
     if verbose:

@@ -11,6 +11,7 @@
 #include <vector>
 #include <zlib.h>
 
+#include "../../include/bbk.h"
 #include "../../include/bbk_io.h"
 
 namespace {
@@ -521,3 +522,223 @@ extern "C" int bbkio_copy_bytes(void* dst, const void* src, size_t n, int32_t th
     return BBKIO_OK;
 }
 
+// ---- bbkio_pack_records / bbkio_check_records: the packed contact records of a pass (format: bbk.h, BbkRecHeader) ------
+namespace {
+
+static_assert(sizeof(BbkRecHeader) == 32, "the record header is 32 bytes");
+static_assert(sizeof(BbkRecChunk) == 64, "a chunk record is 64 bytes");
+constexpr int64_t RC = BBK_REC_CHUNK;
+constexpr int REC_MAX_BITS[3] = {32, 33, 32};
+
+int64_t rec_chunks(int64_t rows) { return rows <= 0 ? 0 : (rows + RC - 1) / RC; }
+uint64_t rec_payload(int64_t n, const uint8_t* bits) {
+    return BBK_REC_COL_BYTES(n, bits[0]) + BBK_REC_COL_BYTES(n, bits[1]) + BBK_REC_COL_BYTES(n, bits[2]);
+}
+
+// exact division and divisibility by a fixed d > 0: d = odd << k, and odd * inv == 1 (mod 2^64)
+struct ExactDiv {
+    uint64_t inv = 1, lim = ~0ull;
+    int k = 0;
+    explicit ExactDiv(uint64_t d) {
+        while (!(d & 1)) { d >>= 1; ++k; }
+        uint64_t x = d;                                     // Newton: 3 -> 6 -> 12 -> 24 -> 48 -> 96 correct bits
+        for (int i = 0; i < 5; ++i) x *= 2 - d * x;
+        inv = x;
+        lim = ~0ull / d;
+    }
+    bool divides(uint64_t x) const { return !(x & ((1ull << k) - 1)) && (x >> k) * inv <= lim; }
+    uint64_t div(uint64_t x) const { return (x >> k) * inv; }
+};
+
+uint64_t gcd64(uint64_t a, uint64_t b) {
+    while (b) { const uint64_t t = a % b; a = b; b = t; }
+    return a;
+}
+
+struct RecSource {
+    const int32_t* const* mid1;
+    const int32_t* const* mid2;
+    const int32_t* const* count;
+    std::vector<int64_t> starts, sizes;       // the pass layout: shard i at starts[i], a multiple of 4
+    // rows [r0, r1) of the layout into local columns (padding rows are zeros)
+    void load(int64_t r0, int64_t r1, int32_t* m1, int32_t* m2, int32_t* ct) const {
+        const int64_t n = r1 - r0;
+        memset(m1, 0, n * 4); memset(m2, 0, n * 4); memset(ct, 0, n * 4);
+        size_t i = std::upper_bound(starts.begin(), starts.end(), r0) - starts.begin();
+        i = i ? i - 1 : 0;
+        for (; i < starts.size() && starts[i] < r1; ++i) {
+            const int64_t a = std::max(r0, starts[i]), b = std::min(r1, starts[i] + sizes[i]);
+            if (b <= a) continue;
+            const int64_t o = a - starts[i];
+            memcpy(m1 + (a - r0), mid1[i] + o, (b - a) * 4);
+            memcpy(m2 + (a - r0), mid2[i] + o, (b - a) * 4);
+            memcpy(ct + (a - r0), count[i] + o, (b - a) * 4);
+        }
+    }
+};
+
+inline int64_t rec_value(int j, const int32_t* m1, const int32_t* m2, const int32_t* ct, int64_t i) {
+    return j == 0 ? (int64_t)m1[i] : j == 1 ? (int64_t)m2[i] - (int64_t)m1[i] : (int64_t)ct[i];
+}
+
+// phase 1: base, step, bits of the chunk's three columns
+void rec_stats(const int32_t* m1, const int32_t* m2, const int32_t* ct, int64_t n, BbkRecChunk& C) {
+    for (int j = 0; j < 3; ++j) {
+        const int64_t v0 = rec_value(j, m1, m2, ct, 0);
+        int64_t mn = v0, mx = v0;
+        uint64_t g = 0;                                  // gcd of |v - v0| over the chunk = gcd of v - min
+        ExactDiv dv(1);
+        for (int64_t i = 0; i < n; ++i) {
+            const int64_t v = rec_value(j, m1, m2, ct, i);
+            mn = std::min(mn, v); mx = std::max(mx, v);
+            const uint64_t d = v >= v0 ? (uint64_t)(v - v0) : (uint64_t)(v0 - v);
+            if (g == 1 || d == 0) continue;
+            if (g == 0 || !dv.divides(d)) { g = gcd64(g, d); dv = ExactDiv(g); }
+        }
+        const uint64_t step = g ? g : 1, span = dv.div((uint64_t)(mx - mn));
+        C.base[j] = mn;
+        C.step[j] = step;
+        C.bits[j] = (uint8_t)(span ? 64 - __builtin_clzll(span) : 0);
+    }
+}
+
+// phase 2: u = (v - base) / step, bits[j] bits each, into the column blocks from `dst`
+void rec_encode(const int32_t* m1, const int32_t* m2, const int32_t* ct, int64_t n, const BbkRecChunk& C, uint8_t* dst) {
+    for (int j = 0; j < 3; ++j) {
+        const int b = C.bits[j];
+        const uint64_t bytes = BBK_REC_COL_BYTES(n, b);
+        uint64_t* w = reinterpret_cast<uint64_t*>(dst);
+        memset(dst, 0, bytes);
+        dst += bytes;
+        if (!b) continue;
+        const ExactDiv dv(C.step[j]);
+        const int64_t base = C.base[j];
+        uint64_t acc = 0;
+        int fill = 0;
+        size_t k = 0;
+        for (int64_t i = 0; i < n; ++i) {
+            const uint64_t u = dv.div((uint64_t)(rec_value(j, m1, m2, ct, i) - base));
+            acc |= u << fill;
+            fill += b;
+            if (fill >= 64) {
+                w[k++] = acc;
+                fill -= 64;
+                acc = fill ? u >> (b - fill) : 0;
+            }
+        }
+        if (fill) w[k] = acc;
+    }
+}
+
+template <class F>
+void rec_parallel(int64_t n_chunks, int threads, F&& f) {
+    int nt = threads > 0 ? threads : (int)std::thread::hardware_concurrency();
+    if (nt < 1) nt = 1;
+    if ((int64_t)nt > n_chunks) nt = (int)std::max<int64_t>(1, n_chunks);
+    auto work = [&](int t) {
+        std::vector<int32_t> buf(3 * RC);
+        const int64_t lo = n_chunks * t / nt, hi = n_chunks * (t + 1) / nt;
+        for (int64_t c = lo; c < hi; ++c) f(c, buf.data(), buf.data() + RC, buf.data() + 2 * RC);
+    };
+    std::vector<std::thread> pool;
+    for (int t = 1; t < nt; ++t) pool.emplace_back(work, t);
+    work(0);
+    for (auto& th : pool) th.join();
+}
+
+}  // namespace
+
+extern "C" uint64_t bbkio_pack_records_bound(int64_t rows) {
+    const int64_t nc = rec_chunks(rows);
+    uint64_t total = sizeof(BbkRecHeader) + (uint64_t)nc * sizeof(BbkRecChunk);
+    if (nc) {
+        const uint8_t worst[3] = {32, 33, 32};
+        total += (uint64_t)(nc - 1) * rec_payload(RC, worst) + rec_payload(rows - (nc - 1) * RC, worst);
+    }
+    return total;
+}
+
+extern "C" int bbkio_pack_records(const int32_t* const* mid1, const int32_t* const* mid2, const int32_t* const* count,
+                                  const int64_t* sizes, int32_t n_shards, void* out, uint64_t capacity, uint64_t* bytes,
+                                  int32_t threads) {
+    if (n_shards < 0 || (n_shards > 0 && (!sizes || !mid1 || !mid2 || !count)) || !out || !bytes) {
+        set_error("bbkio_pack_records: bad arguments");
+        return BBKIO_E_INVALID;
+    }
+    RecSource S{mid1, mid2, count, {}, {}};
+    int64_t rows = 0;
+    for (int i = 0; i < n_shards; ++i) {
+        if (sizes[i] < 0 || (sizes[i] > 0 && (!mid1[i] || !mid2[i] || !count[i]))) {
+            set_error("bbkio_pack_records: shard %d: negative size or null column", i);
+            return BBKIO_E_INVALID;
+        }
+        S.starts.push_back(rows);
+        S.sizes.push_back(sizes[i]);
+        rows += (sizes[i] + 3) & ~(int64_t)3;
+    }
+    const int64_t nc = rec_chunks(rows);
+    const uint64_t head = sizeof(BbkRecHeader) + (uint64_t)nc * sizeof(BbkRecChunk);
+    if (capacity < head) { set_error("bbkio_pack_records: capacity %llu below the %llu bytes of the tables", (unsigned long long)capacity, (unsigned long long)head); return BBKIO_E_INVALID; }
+    BbkRecChunk* table = reinterpret_cast<BbkRecChunk*>(static_cast<uint8_t*>(out) + sizeof(BbkRecHeader));
+    // phase 1: every chunk's frame of reference (all cores)
+    rec_parallel(nc, threads, [&](int64_t c, int32_t* m1, int32_t* m2, int32_t* ct) {
+        const int64_t r0 = c * RC, r1 = std::min(rows, r0 + RC);
+        S.load(r0, r1, m1, m2, ct);
+        BbkRecChunk C;
+        memset(&C, 0, sizeof(C));
+        rec_stats(m1, m2, ct, r1 - r0, C);
+        table[c] = C;
+    });
+    // offsets in chunk order: the bytes do not depend on the thread count
+    uint64_t at = head;
+    for (int64_t c = 0; c < nc; ++c) {
+        table[c].offset = at;
+        at += rec_payload(std::min(RC, rows - c * RC), table[c].bits);
+    }
+    *bytes = at;
+    if (at > capacity) {
+        set_error("bbkio_pack_records: %llu bytes needed, capacity %llu", (unsigned long long)at, (unsigned long long)capacity);
+        return BBKIO_E_INVALID;
+    }
+    // phase 2: the bits (all cores)
+    rec_parallel(nc, threads, [&](int64_t c, int32_t* m1, int32_t* m2, int32_t* ct) {
+        const int64_t r0 = c * RC, r1 = std::min(rows, r0 + RC);
+        S.load(r0, r1, m1, m2, ct);
+        rec_encode(m1, m2, ct, r1 - r0, table[c], static_cast<uint8_t*>(out) + table[c].offset);
+    });
+    BbkRecHeader H;
+    memset(&H, 0, sizeof(H));
+    H.magic = BBK_REC_MAGIC;
+    H.version = BBK_REC_VERSION;
+    H.rows = rows;
+    H.bytes = at;
+    memcpy(out, &H, sizeof(H));
+    return BBKIO_OK;
+}
+
+extern "C" int bbkio_check_records(const void* buf, uint64_t bytes, int64_t rows) {
+    if (!buf || rows < 0) { set_error("bbkio_check_records: bad arguments"); return BBKIO_E_INVALID; }
+    if (bytes < sizeof(BbkRecHeader)) { set_error("bbkio_check_records: %llu bytes, shorter than the header", (unsigned long long)bytes); return BBKIO_E_INVALID; }
+    BbkRecHeader H;
+    memcpy(&H, buf, sizeof(H));
+    if (H.magic != BBK_REC_MAGIC || H.version != BBK_REC_VERSION) { set_error("bbkio_check_records: not a packed record buffer (magic / version)"); return BBKIO_E_INVALID; }
+    if (H.rows != rows) { set_error("bbkio_check_records: %lld rows, expected %lld", (long long)H.rows, (long long)rows); return BBKIO_E_INVALID; }
+    if (H.bytes > bytes) { set_error("bbkio_check_records: the buffer says %llu bytes, only %llu given", (unsigned long long)H.bytes, (unsigned long long)bytes); return BBKIO_E_INVALID; }
+    const int64_t nc = rec_chunks(rows);
+    if ((uint64_t)nc > H.bytes / sizeof(BbkRecChunk)) { set_error("bbkio_check_records: the chunk table runs past the end"); return BBKIO_E_INVALID; }
+    const uint64_t head = sizeof(BbkRecHeader) + (uint64_t)nc * sizeof(BbkRecChunk);
+    if (head > H.bytes) { set_error("bbkio_check_records: the chunk table runs past the end"); return BBKIO_E_INVALID; }
+    const uint8_t* p = static_cast<const uint8_t*>(buf) + sizeof(BbkRecHeader);
+    uint64_t end = head;
+    for (int64_t c = 0; c < nc; ++c) {
+        BbkRecChunk C;
+        memcpy(&C, p + c * sizeof(BbkRecChunk), sizeof(C));
+        for (int j = 0; j < 3; ++j)
+            if (C.bits[j] > REC_MAX_BITS[j]) { set_error("bbkio_check_records: chunk %lld column %d: %d bits", (long long)c, j, (int)C.bits[j]); return BBKIO_E_INVALID; }
+        if (C.offset < end || (C.offset & 15)) { set_error("bbkio_check_records: chunk %lld: offset out of order or misaligned", (long long)c); return BBKIO_E_INVALID; }
+        const uint64_t need = rec_payload(std::min(RC, rows - c * RC), C.bits);
+        if (C.offset > H.bytes || need > H.bytes - C.offset) { set_error("bbkio_check_records: chunk %lld: payload past the end", (long long)c); return BBKIO_E_INVALID; }
+        end = C.offset + need;
+    }
+    return BBKIO_OK;
+}

@@ -125,3 +125,83 @@ extern "C" int bbk_pack_scores(const double* d_p, const double* d_q, int64_t m, 
     BBK_CHECK_LAUNCH("pack_scores_kernel");
     return BBK_OK;
 }
+
+// ---- bbk_unpack_records: packed contact records (bbk.h, BbkRecHeader) back into the int32 columns of a pass ------------
+// One CTA per chunk (grid-stride).  Thread t decodes the 4-row groups t, t + 256, ... of its chunk, so every 128-bit store of a
+// warp covers 512 contiguous bytes.  Row i of a column of b bits is bits [i b, i b + b) of its words: one 64-bit funnel shift
+// over the word holding bit i b and the next one, which is read only when the value reaches into it (it then lies inside the
+// column's block, so a buffer bbkio_check_records accepted is never read past its payload).
+namespace {
+
+constexpr int RU_THREADS = 256;
+static_assert(BBK_REC_CHUNK == RU_THREADS * 16, "a thread decodes 16 rows of a chunk");
+
+__device__ __forceinline__ long long rec_get(const unsigned long long* __restrict__ w, int b, long long base, unsigned long long step,
+                                             int i) {
+    if (b == 0) return base;                             // an empty block: nothing to read
+    const unsigned long long bit = (unsigned long long)i * (unsigned)b;
+    const unsigned off = (unsigned)(bit & 63u);
+    const unsigned long long* p = w + (bit >> 6);
+    const unsigned long long lo = __ldg(p), hi = off + (unsigned)b > 64u ? __ldg(p + 1) : 0ull;
+    const unsigned long long u = ((lo >> off) | ((hi << 1) << (63u - off))) & ((1ull << b) - 1ull);
+    return base + (long long)(step * u);
+}
+
+__global__ void __launch_bounds__(RU_THREADS) unpack_records_kernel(const unsigned char* __restrict__ buf, long long rows,
+                                                                    int* __restrict__ mid1, int* __restrict__ mid2,
+                                                                    int* __restrict__ count) {
+    const long long n_chunks = (rows + BBK_REC_CHUNK - 1) / BBK_REC_CHUNK;
+    const BbkRecChunk* table = reinterpret_cast<const BbkRecChunk*>(buf + sizeof(BbkRecHeader));
+    for (long long ch = blockIdx.x; ch < n_chunks; ch += gridDim.x) {
+        const BbkRecChunk C = table[ch];
+        const long long r0 = ch * BBK_REC_CHUNK;
+        const int n = (int)min((long long)BBK_REC_CHUNK, rows - r0);
+        const unsigned long long* w0 = reinterpret_cast<const unsigned long long*>(buf + C.offset);
+        const unsigned long long* w1 = w0 + BBK_REC_COL_BYTES(n, C.bits[0]) / 8;
+        const unsigned long long* w2 = w1 + BBK_REC_COL_BYTES(n, C.bits[1]) / 8;
+        const int b0 = C.bits[0], b1 = C.bits[1], b2 = C.bits[2];
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+            const int i0 = (g * RU_THREADS + (int)threadIdx.x) * 4;
+            if (i0 >= n) break;
+            int m1[4], m2[4], ct[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int i = min(i0 + k, n - 1);              // rows past the end are decoded again, never stored
+                const long long a = rec_get(w0, b0, C.base[0], C.step[0], i);
+                m1[k] = (int)a;
+                m2[k] = (int)(a + rec_get(w1, b1, C.base[1], C.step[1], i));
+                ct[k] = (int)rec_get(w2, b2, C.base[2], C.step[2], i);
+            }
+            const long long r = r0 + i0;
+            if (i0 + 4 <= n) {
+                *reinterpret_cast<int4*>(mid1 + r) = make_int4(m1[0], m1[1], m1[2], m1[3]);
+                *reinterpret_cast<int4*>(mid2 + r) = make_int4(m2[0], m2[1], m2[2], m2[3]);
+                *reinterpret_cast<int4*>(count + r) = make_int4(ct[0], ct[1], ct[2], ct[3]);
+            } else {
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if (i0 + k < n) { mid1[r + k] = m1[k]; mid2[r + k] = m2[k]; count[r + k] = ct[k]; }
+            }
+        }
+    }
+}
+
+}  // namespace
+
+extern "C" int bbk_unpack_records(const void* d_buf, int64_t bytes, int64_t rows, int32_t* d_mid1, int32_t* d_mid2, int32_t* d_count,
+                                  void* stream) {
+    BBK_REQUIRE(rows >= 0 && bytes >= (int64_t)sizeof(BbkRecHeader), "bbk_unpack_records: negative rows or a buffer shorter than its header");
+    if (rows == 0) return BBK_OK;
+    BBK_REQUIRE(d_buf && d_mid1 && d_mid2 && d_count, "bbk_unpack_records: null pointer");
+    BBK_REQUIRE((((uintptr_t)d_buf | (uintptr_t)d_mid1 | (uintptr_t)d_mid2 | (uintptr_t)d_count) & 15) == 0,
+                "bbk_unpack_records: buffer and columns must be 16-byte aligned");
+    const long long n_chunks = (rows + BBK_REC_CHUNK - 1) / BBK_REC_CHUNK;
+    BBK_REQUIRE((uint64_t)bytes >= sizeof(BbkRecHeader) + (uint64_t)n_chunks * sizeof(BbkRecChunk), "bbk_unpack_records: buffer shorter than its chunk table");
+    long long grid = (long long)bbk_num_sms() * 8;
+    if (n_chunks < grid) grid = n_chunks;
+    unpack_records_kernel<<<(unsigned)grid, RU_THREADS, 0, (cudaStream_t)stream>>>(static_cast<const unsigned char*>(d_buf), rows, d_mid1,
+                                                                                     d_mid2, d_count);
+    BBK_CHECK_LAUNCH("unpack_records_kernel");
+    return BBK_OK;
+}

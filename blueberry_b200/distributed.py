@@ -19,7 +19,7 @@ import ctypes
 import numpy as np
 import torch
 
-from . import _lib
+from . import _io, _lib
 from .engine import PassEngine, Shard
 
 
@@ -676,13 +676,16 @@ class HostStream(object):
     class _Slot(object):
         pass
 
-    def __init__(self, genome_pass, sizes, chroms, slots=2, packed=False, cap_p=None, cap_q=None):
+    def __init__(self, genome_pass, sizes, chroms, slots=2, packed=False, cap_p=None, cap_q=None, cap_in=None):
         """genome_pass: a GenomePass or a ChromosomePass.  sizes / chroms: records and chromosome of every shard; the slots hold
         layout_rows(sizes) rows.  packed: results cross the host link as two bits per row + the values that are not 1.0 / NaN
         (bbk_pack_scores); submit_packed() returns a PackedScores whose dense() rebuilds the float64 columns bit for bit, over
         the slot's rows (the padding rows between shards hold NaN; shard i is rows starts[i] .. starts[i] + sizes[i]).
         cap_p / cap_q: rows the packed value lists can hold (default rows / 2 and rows / 16; a pass that needs more comes back
-        dense)."""
+        dense).
+        cap_in: bytes of the one device buffer that packed records (PackedRecords) cross into, shared by all slots; default
+        bbkio_pack_records_bound of the slots' rows, the most any pass can need.  It is allocated by the first submission of
+        packed records."""
         self.gp = genome_pass
         self.sizes, self.chroms = [int(x) for x in sizes], [int(x) for x in chroms]
         self.starts, rows = layout_rows(self.sizes)
@@ -713,33 +716,55 @@ class HostStream(object):
         self.s_run.wait_stream(torch.cuda.current_stream(dev))
         self.submitted = 0
         self._pending = None
+        self.cap_in = int(cap_in) if cap_in is not None else _io.pack_records_bound(layout_rows(self.sizes)[1])
+        self.d_in = None
 
     def _shards(self, s, starts, sizes):
         return [Shard(s.mid1[a:a + n], s.mid2[a:a + n], s.count[a:a + n], chrom=c) for a, n, c in zip(starts, sizes, self.chroms)]
 
     def _run(self, h_mid1, h_mid2, h_count, h_out, n_tests, sizes, q_values, pack=False):
-        """What submit() and submit_packed() share: check the host columns, copy the records into the next slot (stream in)
-        and run the pass there (stream run), packing p / q after it when `pack`.  Returns (slot, rows the pass covers)."""
+        """What submit() and submit_packed() share: check the host columns (or the packed records in h_mid1), copy the records
+        into the next slot (stream in; packed records are decoded there into the slot's columns) and run the pass there
+        (stream run), packing p / q after it when `pack`.  Returns (slot, rows the pass covers)."""
         s = self.slots[self.submitted % len(self.slots)]
         sizes = self.sizes if sizes is None else [int(x) for x in sizes]
         starts, rows = layout_rows(sizes)
         if len(sizes) != len(self.chroms) or rows > self.rows:
             raise ValueError("sizes must give one shard per chromosome of the stream and fit its %d rows" % self.rows)
         n = starts[-1] + sizes[-1] if sizes else 0
-        for t in (h_mid1, h_mid2, h_count) + h_out:
+        rec = h_mid1 if isinstance(h_mid1, PackedRecords) else None
+        if rec is not None:
+            if h_mid2 is not None or h_count is not None:
+                raise ValueError("pass either packed records or the three host columns")
+            if rec.rows != rows or rec.sizes != sizes:
+                raise ValueError("the packed records have layout %s (%d rows); this pass has %s (%d rows)" % (rec.sizes, rec.rows, sizes, rows))
+            if rec.nbytes > self.cap_in:
+                raise ValueError("the packed records take %d bytes; the stream's inbound buffer holds %d (cap_in)" % (rec.nbytes, self.cap_in))
+            rec.check()
+        cols = (h_mid1, h_mid2, h_count) if rec is None else ()
+        for t in cols + h_out:
             if t is not None and (not t.is_pinned() or t.numel() < n):
                 raise ValueError("host columns must be pinned and hold at least %d rows" % n)
         if q_values and s.q is None:
             raise ValueError("the stream's pass was made with q_values=False")
         self.gp.check_sizes(sizes)
         shards = s.shards if sizes is self.sizes else self._shards(s, starts, sizes)
+        if rec is not None and self.d_in is None:
+            with torch.cuda.stream(self.s_in):
+                self.d_in = torch.empty(max(self.cap_in, 16), dtype=torch.uint8, device=s.mid1.device)
         self.submitted += 1
         s.index = self.submitted - 1
         self.s_in.wait_event(s.run_done)        # the pass that last read this slot's records has finished
         with torch.cuda.stream(self.s_in):
-            s.mid1[:n].copy_(h_mid1[:n], non_blocking=True)
-            s.mid2[:n].copy_(h_mid2[:n], non_blocking=True)
-            s.count[:n].copy_(h_count[:n], non_blocking=True)
+            if rec is None:
+                s.mid1[:n].copy_(h_mid1[:n], non_blocking=True)
+                s.mid2[:n].copy_(h_mid2[:n], non_blocking=True)
+                s.count[:n].copy_(h_count[:n], non_blocking=True)
+            else:
+                # one inbound buffer: the next pass' copy queues behind this decode on the same stream
+                self.d_in[:rec.nbytes].copy_(rec.buf[:rec.nbytes], non_blocking=True)
+                _decode_records(self.d_in, rec.nbytes, rec.rows, s.mid1, s.mid2, s.count, self.s_in)
+                self.gp.launches += 1
             s.in_ready.record()
         # the previous packed pass' value lists: their sizes are on the host by now (or soon); their copies overlap these inbound ones
         self._finalize_pending()
@@ -763,12 +788,18 @@ class HostStream(object):
             s.run_done.record()
         return s, n
 
-    def submit(self, h_mid1, h_mid2, h_count, h_p, h_q=None, n_tests=-1, sizes=None):
+    def submit(self, h_mid1, h_mid2=None, h_count=None, h_p=None, h_q=None, n_tests=-1, sizes=None):
         """Enqueue one pass over the host table; returns the event that fires when p (and q) are on the host.
         sizes: this pass' shard sizes, one per chromosome of the stream (default: the sizes it was made with); their
         layout_rows total must fit the slots.  The host columns hold at least the rows the pass covers (up to the end of its
         last shard), and exactly those rows come back.  Without h_q the pass skips the q-value step; at N > 1 that step is
-        collective, so every rank must pass or omit h_q alike."""
+        collective, so every rank must pass or omit h_q alike.
+        h_mid1 may instead be a PackedRecords of exactly this pass' sizes (h_mid2 / h_count omitted): submit(rec, h_p=..,
+        h_q=..).  It is validated on the host, crosses the link as it is and is decoded into the slot on the device; a layout
+        that differs from the pass', more bytes than cap_in, or a buffer that fails validation raise ValueError before
+        anything is copied.  Like h_p, the PackedRecords may be refilled once the returned event has fired."""
+        if h_p is None:
+            raise ValueError("submit needs h_p")
         s, n = self._run(h_mid1, h_mid2, h_count, (h_p, h_q), n_tests, sizes, h_q is not None)
         self.s_out.wait_event(s.run_done)
         with torch.cuda.stream(self.s_out):
@@ -780,10 +811,14 @@ class HostStream(object):
         return s.out_done
 
     # ------------------------------------------------------------------ packed results
-    def submit_packed(self, h_mid1, h_mid2, h_count, out, n_tests=-1):
+    def submit_packed(self, h_mid1, h_mid2=None, h_count=None, out=None, n_tests=-1):
         """Like submit(), but p / q come back packed into `out` (a PackedScores made by packed_buffers()).  The sizes of the two
         value lists are only known once the pass has run, so their copies are issued lazily: by the NEXT submission (after
-        it has put its own inbound copies on the wire) or by drain().  Returns `out`; out.done fires when it is complete."""
+        it has put its own inbound copies on the wire) or by drain().  Returns `out`; out.done fires when it is complete.
+        h_mid1 may be a PackedRecords of the stream's sizes, as in submit(): submit_packed(rec, out=out); it may be refilled
+        once out.done has fired."""
+        if out is None:
+            raise ValueError("submit_packed needs out (packed_buffers())")
         if not self.packed:
             raise ValueError("this stream was not created with packed=True")
         s, _ = self._run(h_mid1, h_mid2, h_count, (), n_tests, None, self.gp.q_values, pack=True)
@@ -900,3 +935,52 @@ class PackedScores(object):
         return _io.unpack_scores(self.codes.numpy(), self.chunks.numpy(), self.vals_p.numpy(),
                                  self.vals_q.numpy() if self.vals_q is not None else None, self.rows, p_out, q_out, threads,
                                  want_q=self.want_q)
+
+
+def _decode_records(d_buf, nbytes, rows, mid1, mid2, count, stream):
+    """bbk_unpack_records on `stream`: packed records already on the device (validated on the host by the caller, as
+    bbkio_check_records) into the first `rows` rows of three int32 columns."""
+    _lib.check(_lib.load().bbk_unpack_records(_lib.ptr(d_buf), int(nbytes), int(rows), _lib.ptr(mid1), _lib.ptr(mid2), _lib.ptr(count),
+                                              _lib.stream_ptr(stream)), "bbk_unpack_records")
+
+
+class PackedRecords(object):
+    """The contact records of one pass packed for the host link (include/bbk.h, BbkRecHeader: a frame-of-reference code per
+    4096 rows, ~3 B/row on Hi-C records against 12 B/row of int32 columns) in a pinned uint8 buffer.  rows / sizes: the pass
+    layout (layout_rows(sizes)); nbytes: bytes of buf in use.  Made and refilled by pack_records()."""
+
+    def __init__(self, capacity):
+        self.buf = torch.empty(max(int(capacity), 32), dtype=torch.uint8).pin_memory()
+        self.rows, self.sizes, self.nbytes = 0, [], 0
+
+    def check(self):
+        """Raise ValueError unless buf holds valid packed records of `rows` rows (bbkio_check_records)."""
+        _io.check_records(self.buf.data_ptr(), self.nbytes, self.rows)
+
+    def to_device(self, device=None):
+        """Validate on the host, copy once and decode on the device (current stream; asynchronous): returns (mid1, mid2, count),
+        int32 tensors of `rows` rows in the pass layout (padding rows between shards are 0).  buf may be refilled once the
+        current stream has passed this call."""
+        self.check()
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        with torch.cuda.device(dev):
+            d_buf = torch.empty(max(self.nbytes, 16), dtype=torch.uint8, device=dev)
+            d_buf[:self.nbytes].copy_(self.buf[:self.nbytes], non_blocking=True)
+            cols = [torch.empty(max(self.rows, 4), dtype=torch.int32, device=dev) for _ in range(3)]
+            _decode_records(d_buf, self.nbytes, self.rows, cols[0], cols[1], cols[2], torch.cuda.current_stream(dev))
+        return tuple(c[:self.rows] for c in cols)
+
+
+def pack_records(shards, out=None, threads=0):
+    """Pack the records of one pass for the host link: shards = [(mid1, mid2, count), ...], int32 host columns (numpy arrays or
+    CPU tensors, any memory) laid out as layout_rows gives, without assembling padded columns first.  All host cores
+    (threads <= 0), two phases over 4096-row chunks; the bytes do not depend on the thread count.  out: a PackedRecords to
+    refill (ValueError when its buffer is too small), or None for a new one sized for the worst case.  Returns it."""
+    sizes = [len(sh[0]) for sh in shards]
+    rows = layout_rows(sizes)[1]
+    if out is None:
+        out = PackedRecords(_io.pack_records_bound(rows))
+    out.rows, out.sizes, out.nbytes = 0, [], 0
+    nbytes = _io.pack_records(shards, out.buf.data_ptr(), out.buf.numel(), threads)
+    out.rows, out.sizes, out.nbytes = rows, sizes, nbytes
+    return out

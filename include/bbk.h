@@ -300,6 +300,46 @@ int bbk_pack_scores(const double* d_p, const double* d_q, int64_t m, uint32_t* d
                     BbkPackState* d_state, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Packed contact records                                 the input side of the host link
+ *
+ * The int32 record columns (mid1, mid2, count) of a pass cost 12 B/row to move in, but carry far fewer bits: mid1 is nearly
+ * constant over a block of rows, mid2 - mid1 is a multiple of the resolution, counts are small.  The packed form is a
+ * frame-of-reference code per BBK_REC_CHUNK rows of the pass layout (layout_rows: shard i at starts[i], the padding rows
+ * between shards encoded as zeros).  Buffer:
+ *     BbkRecHeader | BbkRecChunk[ceil(rows / BBK_REC_CHUNK)] | chunk payloads
+ * Chunk c holds rows [c * BBK_REC_CHUNK, min(rows, (c + 1) * BBK_REC_CHUNK)).  Its three columns j are
+ *     j = 0: mid1    j = 1: e = mid2 - mid1 (in 64 bits)    j = 2: count
+ * each stored as v = base[j] + step[j] * u, base = the chunk minimum, step = gcd(v - base) (1 when all values are equal),
+ * u in bits[j] bits (0..32; 0..33 for e), packed little-endian into 64-bit words: row i of the chunk is bits
+ * [i * bits, (i + 1) * bits) of the column's words.  Column j's block is BBK_REC_COL_BYTES(n, bits[j]) bytes (a multiple of
+ * 16); the three blocks follow each other from `offset` (bytes from the buffer start, a multiple of 16).  Chunks are laid
+ * out in order.  Lossless for every int32 input; the bytes depend on the records only (bbkio_pack_records in bbk_io.h
+ * writes them on the host, bbkio_check_records validates them).
+ * bbk_unpack_records decodes rows [0, rows) into three int32 device columns (16-byte aligned).  It trusts its buffer: the
+ * caller passes only buffers that bbkio_check_records accepted for the same `rows` and `bytes`.
+ * ------------------------------------------------------------------------------------------- */
+#define BBK_REC_MAGIC 0x31434552u       /* "REC1" */
+#define BBK_REC_VERSION 1
+#define BBK_REC_CHUNK 4096
+#define BBK_REC_COL_BYTES(n, bits) ((((uint64_t)(n) * (uint64_t)(bits) + 127u) / 128u) * 16u)
+typedef struct BbkRecHeader {
+    uint32_t magic;          /* BBK_REC_MAGIC */
+    uint32_t version;        /* BBK_REC_VERSION */
+    int64_t rows;            /* rows of the pass layout */
+    uint64_t bytes;          /* bytes of the whole buffer */
+    uint64_t reserved;
+} BbkRecHeader;
+typedef struct BbkRecChunk {
+    int64_t base[3];
+    uint64_t step[3];
+    uint64_t offset;         /* first byte of column 0's block */
+    uint8_t bits[3];
+    uint8_t reserved[5];
+} BbkRecChunk;
+int bbk_unpack_records(const void* d_buf, int64_t bytes, int64_t rows, int32_t* d_mid1, int32_t* d_mid2, int32_t* d_count,
+                       void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K5  Benjamini-Hochberg q-values as the reference computes them: a FORWARD running max of
  *     min(p * N / rank, 1)   (fithic.py:466-487, blueberry.pyx:40-75) - not the textbook reverse
  *     cumulative minimum.  q comes back in input order; NaN p (dropped rows) -> NaN q, not ranked.

@@ -62,6 +62,20 @@ int bbkio_unpack_scores_keep(const uint32_t* codes, const void* chunks, const do
 /* a large host copy by `threads` cores (<= 0: all): numpy columns into pinned staging memory and back */
 int bbkio_copy_bytes(void* dst, const void* src, size_t n, int32_t threads);
 
+/* The packed contact records of a pass (format: bbk.h, BbkRecHeader), written from the shards' own int32 columns (any host
+ * memory) straight into the pass layout: shard i of sizes[i] rows starts at row starts[i] of layout_rows(sizes) (every start
+ * a multiple of 4), the padding rows between shards are zeros.  Two phases over the chunks by all cores (frames of
+ * reference, then bits); the bytes do not depend on `threads` (<= 0: all online cores).  *bytes receives the size; a
+ * capacity below it fails the call (BBKIO_E_INVALID, *bytes still set).  bbkio_pack_records_bound(rows) is the largest
+ * size `rows` layout rows can take. */
+uint64_t bbkio_pack_records_bound(int64_t rows);
+int bbkio_pack_records(const int32_t* const* mid1, const int32_t* const* mid2, const int32_t* const* count, const int64_t* sizes,
+                       int32_t n_shards, void* out, uint64_t capacity, uint64_t* bytes, int32_t threads);
+/* BBKIO_OK when buf[0 .. bytes) is a packed record buffer of `rows` rows that bbk_unpack_records may read: header, chunk
+ * offsets in bounds, aligned and increasing, bits within their limits, every payload ending within the buffer.
+ * BBKIO_E_INVALID otherwise (bbkio_last_error says why). */
+int bbkio_check_records(const void* buf, uint64_t bytes, int64_t rows);
+
 /* "{}".format(float64) into buf (at least 32 bytes); returns the length.  Exposed for the parity tests. */
 int bbkio_format_double(double x, char* buf);
 
