@@ -671,12 +671,17 @@ class HostStream(object):
     float64 columns over the same rows.  Nothing here synchronises the host: call drain() (or wait on the event submit() returns) before reading.
 
     With a ChromosomePass every shard is one chromosome (chroms = its ids, in its order; sizes at most those it was built
-    with), each gets its own fit and q-values, and fit_of(k) returns one FitResult per chromosome."""
+    with), each gets its own fit and q-values, and fit_of(k) returns one FitResult per chromosome.
+
+    With refit=True (a GenomePass on one GPU) every submission is the two-pass workload of BASELINE config 4, as
+    fit_transform_arrays(refit=True) runs it: pass 1 without q-values into the slot's p_first, then the refit pass that leaves
+    the rows with p_first <= 1 / possibleIntraInRangeCount out of the statistics and scores every row again, both on the run
+    stream with no host synchronisation in between.  fit_of(k, first=True) is pass 1's fit."""
 
     class _Slot(object):
         pass
 
-    def __init__(self, genome_pass, sizes, chroms, slots=2, packed=False, cap_p=None, cap_q=None, cap_in=None):
+    def __init__(self, genome_pass, sizes, chroms, slots=2, packed=False, cap_p=None, cap_q=None, cap_in=None, refit=False):
         """genome_pass: a GenomePass or a ChromosomePass.  sizes / chroms: records and chromosome of every shard; the slots hold
         layout_rows(sizes) rows.  packed: results cross the host link as two bits per row + the values that are not 1.0 / NaN
         (bbk_pack_scores); submit_packed() returns a PackedScores whose dense() rebuilds the float64 columns bit for bit, over
@@ -685,7 +690,22 @@ class HostStream(object):
         dense).
         cap_in: bytes of the one device buffer that packed records (PackedRecords) cross into, shared by all slots; default
         bbkio_pack_records_bound of the slots' rows, the most any pass can need.  It is allocated by the first submission of
-        packed records."""
+        packed records.
+        refit: run every submission as two passes (class docstring).  The outlier threshold depends on the fragments alone, so
+        it is computed here, once, as fit_transform_arrays(refit=True) computes it; possibleIntraInRangeCount <= 0 raises
+        ZeroDivisionError.  A ChromosomePass, or a GenomePass across ranks, raises NotImplementedError."""
+        self.refit = bool(refit)
+        if self.refit:
+            if not isinstance(genome_pass, GenomePass):
+                raise NotImplementedError("refit=True streams a GenomePass; per_chromosome=True does not take refit=True")
+            if genome_pass.world > 1:
+                raise NotImplementedError("refit=True runs on one GPU")
+            from .fithic import _in_range_possible
+            eng = genome_pass.eng
+            in_rng = _in_range_possible(eng.possible.cpu().numpy(), eng.R, eng.min_dist, eng.max_dist)
+            if in_rng <= 0:
+                raise ZeroDivisionError("float division by zero (possibleIntraInRangeCount == 0)")
+            self.p_outlier = 1.0 / in_rng
         self.gp = genome_pass
         self.sizes, self.chroms = [int(x) for x in sizes], [int(x) for x in chroms]
         self.starts, rows = layout_rows(self.sizes)
@@ -703,6 +723,10 @@ class HostStream(object):
             s.in_ready, s.run_done, s.out_done, s.counts_ready = (torch.cuda.Event() for _ in range(4))
             s.fit = torch.zeros(nf, dtype=torch.uint8, device=dev)
             s.h_fit = torch.zeros(nf, dtype=torch.uint8).pin_memory()
+            if self.refit:
+                s.p_first = torch.full((self.rows,), float("nan"), dtype=torch.float64, device=dev)
+                s.fit_first = torch.zeros(nf, dtype=torch.uint8, device=dev)
+                s.h_fit_first = torch.zeros(nf, dtype=torch.uint8).pin_memory()
             if self.packed:
                 s.pack = DevicePack(self.rows, dev, genome_pass.q_values, cap_p, cap_q)
                 s.h_pack_state = torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8).pin_memory()
@@ -722,10 +746,26 @@ class HostStream(object):
     def _shards(self, s, starts, sizes):
         return [Shard(s.mid1[a:a + n], s.mid2[a:a + n], s.count[a:a + n], chrom=c) for a, n, c in zip(starts, sizes, self.chroms)]
 
-    def _run(self, h_mid1, h_mid2, h_count, h_out, n_tests, sizes, q_values, pack=False):
+    def _smoothing(self, smoothing):
+        """smoothing= of a submission, checked: (s_first, s_second) with refit, else one s (None: the kernel's own)."""
+        if isinstance(self.gp, ChromosomePass):
+            if smoothing is not None:
+                raise ValueError("a ChromosomePass stream takes chromosome i's s from pass.smoothing[i], not smoothing=")
+            return None
+        if not self.refit:
+            return None if smoothing is None else float(smoothing)
+        if smoothing is None:
+            return None, None
+        if isinstance(smoothing, (str, bytes)) or np.ndim(smoothing) != 1 or len(smoothing) != 2:
+            raise ValueError("a refit stream takes smoothing=(s_first, s_second), each None or a float")
+        return tuple(None if v is None else float(v) for v in smoothing)
+
+    def _run(self, h_mid1, h_mid2, h_count, h_out, n_tests, sizes, q_values, pack=False, smoothing=None):
         """What submit() and submit_packed() share: check the host columns (or the packed records in h_mid1), copy the records
         into the next slot (stream in; packed records are decoded there into the slot's columns) and run the pass there
-        (stream run), packing p / q after it when `pack`.  Returns (slot, rows the pass covers)."""
+        (stream run; with refit, pass 1 into the slot's p_first, its fit copied aside, then the refit pass), packing p / q
+        after it when `pack`.  Returns (slot, rows the pass covers)."""
+        smoothing = self._smoothing(smoothing)
         s = self.slots[self.submitted % len(self.slots)]
         sizes = self.sizes if sizes is None else [int(x) for x in sizes]
         starts, rows = layout_rows(sizes)
@@ -772,10 +812,24 @@ class HostStream(object):
         self.s_run.wait_event(s.out_done)       # this slot's previous p / q have left the device
         gp = self.gp
         with torch.cuda.stream(self.s_run):
-            keep_q, gp.q_values = gp.q_values, q_values
+            keep_q = gp.q_values
             try:
-                gp.attach(shards, s.p, s.q)
-                gp.enqueue(n_tests)
+                if self.refit:
+                    # one pass object for both passes: they share its deferred list, which has a place for every slot row
+                    gp.q_values = False
+                    gp.attach(shards, s.p_first, None)
+                    gp.enqueue(-1, smoothing=smoothing[0])
+                    s.fit_first.copy_(gp.eng.fit_result, non_blocking=True)
+                    gp.q_values = q_values
+                    gp.attach(shards, s.p, s.q)
+                    gp.enqueue(n_tests, smoothing=smoothing[1], exclude=(s.p_first, self.p_outlier))
+                else:
+                    gp.q_values = q_values
+                    gp.attach(shards, s.p, s.q)
+                    if isinstance(gp, ChromosomePass):
+                        gp.enqueue(n_tests)
+                    else:
+                        gp.enqueue(n_tests, smoothing=smoothing)
             finally:
                 gp.q_values = keep_q
             o = 0
@@ -788,7 +842,7 @@ class HostStream(object):
             s.run_done.record()
         return s, n
 
-    def submit(self, h_mid1, h_mid2=None, h_count=None, h_p=None, h_q=None, n_tests=-1, sizes=None):
+    def submit(self, h_mid1, h_mid2=None, h_count=None, h_p=None, h_q=None, n_tests=-1, sizes=None, h_p_first=None, smoothing=None):
         """Enqueue one pass over the host table; returns the event that fires when p (and q) are on the host.
         sizes: this pass' shard sizes, one per chromosome of the stream (default: the sizes it was made with); their
         layout_rows total must fit the slots.  The host columns hold at least the rows the pass covers (up to the end of its
@@ -797,38 +851,54 @@ class HostStream(object):
         h_mid1 may instead be a PackedRecords of exactly this pass' sizes (h_mid2 / h_count omitted): submit(rec, h_p=..,
         h_q=..).  It is validated on the host, crosses the link as it is and is decoded into the slot on the device; a layout
         that differs from the pass', more bytes than cap_in, or a buffer that fails validation raise ValueError before
-        anything is copied.  Like h_p, the PackedRecords may be refilled once the returned event has fired."""
+        anything is copied.  Like h_p, the PackedRecords may be refilled once the returned event has fired.
+        smoothing: the s a GenomePass stream's fit takes (None: the kernel's min(y) * min(y)); a pass whose fit_of(k) gives
+        PassEngine.reference_smoothing(fit) != None is submitted again with that value to equal GenomePass.run.  With refit,
+        a pair (s_first, s_second) for the two passes, each None or a float: settle s_first by fit_of(k, first=True), then
+        s_second by fit_of(k), as fit_transform_arrays(refit=True) does.  A ChromosomePass stream takes pass.smoothing[i]
+        instead, and smoothing= raises ValueError there.
+        h_p_first (refit only): an optional pinned float64 column that receives pass 1's p over the same rows as h_p."""
         if h_p is None:
             raise ValueError("submit needs h_p")
-        s, n = self._run(h_mid1, h_mid2, h_count, (h_p, h_q), n_tests, sizes, h_q is not None)
+        if h_p_first is not None and not self.refit:
+            raise ValueError("h_p_first needs a stream made with refit=True")
+        s, n = self._run(h_mid1, h_mid2, h_count, (h_p, h_q, h_p_first), n_tests, sizes, h_q is not None, smoothing=smoothing)
         self.s_out.wait_event(s.run_done)
         with torch.cuda.stream(self.s_out):
             h_p[:n].copy_(s.p[:n], non_blocking=True)
             if h_q is not None:
                 h_q[:n].copy_(s.q[:n], non_blocking=True)
-            s.h_fit.copy_(s.fit, non_blocking=True)
+            if h_p_first is not None:
+                h_p_first[:n].copy_(s.p_first[:n], non_blocking=True)
+            self._fits_out(s)
             s.out_done.record()
         return s.out_done
 
+    def _fits_out(self, s):
+        s.h_fit.copy_(s.fit, non_blocking=True)
+        if self.refit:
+            s.h_fit_first.copy_(s.fit_first, non_blocking=True)
+
     # ------------------------------------------------------------------ packed results
-    def submit_packed(self, h_mid1, h_mid2=None, h_count=None, out=None, n_tests=-1):
+    def submit_packed(self, h_mid1, h_mid2=None, h_count=None, out=None, n_tests=-1, smoothing=None):
         """Like submit(), but p / q come back packed into `out` (a PackedScores made by packed_buffers()).  The sizes of the two
         value lists are only known once the pass has run, so their copies are issued lazily: by the NEXT submission (after
         it has put its own inbound copies on the wire) or by drain().  Returns `out`; out.done fires when it is complete.
         h_mid1 may be a PackedRecords of the stream's sizes, as in submit(): submit_packed(rec, out=out); it may be refilled
-        once out.done has fired."""
+        once out.done has fired.  smoothing: as in submit().  With refit, `out` holds the refit pass' p / q; pass 1's p does
+        not come back (its fit does: fit_of(k, first=True))."""
         if out is None:
             raise ValueError("submit_packed needs out (packed_buffers())")
         if not self.packed:
             raise ValueError("this stream was not created with packed=True")
-        s, _ = self._run(h_mid1, h_mid2, h_count, (), n_tests, None, self.gp.q_values, pack=True)
+        s, _ = self._run(h_mid1, h_mid2, h_count, (), n_tests, None, self.gp.q_values, pack=True, smoothing=smoothing)
         self.s_out.wait_event(s.run_done)
         with torch.cuda.stream(self.s_out):
             s.h_pack_state.copy_(s.pack.state, non_blocking=True)
             s.counts_ready.record()
             out.codes.copy_(s.pack.codes, non_blocking=True)
             out.chunks.copy_(s.pack.chunks, non_blocking=True)
-            s.h_fit.copy_(s.fit, non_blocking=True)
+            self._fits_out(s)
         out.rows, out.want_q = self.rows, s.q is not None
         out.done = None
         self._pending = (s, out)
@@ -862,16 +932,25 @@ class HostStream(object):
         pk = self.slots[0].pack
         return PackedScores(self.rows, pk.codes.numel(), pk.chunks.numel() // 24, pk.cap_p, pk.cap_q)
 
-    def fit_of(self, index):
+    def fit_of(self, index, first=False):
         """Fit result of submission `index` once its outputs are on the host (raises the reference's exception for a failed
-        fit); PassEngine.reference_smoothing(result) tells whether that pass must be repeated with the reference's own s.
+        fit); PassEngine.reference_smoothing(result) tells whether that pass must be repeated with the reference's own s
+        (submit(..., smoothing=...)).
         With a ChromosomePass: one FitResult per chromosome, in its order; a failed fit raises for the lowest failing id,
         naming it, and a chromosome is repeated with its own s by setting pass.smoothing[i] and submitting again.
+        With refit: the refit pass' fit, after raising pass 1's exception if pass 1 failed (what fit_transform_arrays(refit=True)
+        raises first); first=True: pass 1's fit.
         Only the last `slots` submissions are held."""
+        if first and not self.refit:
+            raise ValueError("first=True needs a stream made with refit=True")
         s = self.slots[int(index) % len(self.slots)]
         if s.index != int(index):
             raise KeyError("submission %d is no longer (or not yet) held by the stream" % int(index))
         s.out_done.synchronize()
+        if self.refit:
+            fit1 = self.gp.decode_fits(s.h_fit_first.numpy().tobytes())
+            if first:
+                return fit1
         return self.gp.decode_fits(s.h_fit.numpy().tobytes())
 
     def drain(self):

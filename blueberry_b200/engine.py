@@ -228,7 +228,8 @@ class PassEngine(object):
             req = _lib.FitResult()
             req.status = _lib.FIT_S_GIVEN
             req.smoothing = float(smoothing)
-            self.fit_result.copy_(torch.frombuffer(bytearray(bytes(req)), dtype=torch.uint8))
+            # non_blocking: a pageable source is staged at once, and the stream (HostStream's run stream) is not synchronised
+            self.fit_result.copy_(torch.frombuffer(bytearray(bytes(req)), dtype=torch.uint8), non_blocking=True)
         _lib.check(self.lib.bbk_fit(_lib.ptr(self.possible), _lib.ptr(self.obs_sum), self.nkeys, _lib.ptr(self.totals),
                                     self.n_bins, self.R, self.min_dist, self.max_dist, self.max_bins,
                                     _lib.ptr(self.fit_result), _lib.ptr(self.x), _lib.ptr(self.y), _lib.ptr(self.bin_of_key),
