@@ -127,6 +127,7 @@ SIGNATURES = {
     "bbk_bh_gathered_workspace_bytes": (_sz, [_i32, _i64]),
     "bbk_bh_pack_count": (ctypes.c_int, [_vp, _vp, _vp]),
     "bbk_bh_rank_gathered_padded": (ctypes.c_int, [_vp, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "bbk_bh_rank_gathered_all": (ctypes.c_int, [_vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "bbk_synth_contacts_range": (ctypes.c_int, [_i64, _i64, _i64, _f64, _f64, ctypes.c_uint64, _vp, _i64, _i64, _vp, _vp, _vp, _vp]),
     "bbk_synth_n_pairs": (_i64, [_i64, _i64]),
     "bbk_synth_contacts": (ctypes.c_int, [_i64, _i64, _i64, _f64, _f64, ctypes.c_uint64, _vp, _vp, _vp, _vp, _vp]),

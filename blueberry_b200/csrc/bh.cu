@@ -1274,15 +1274,18 @@ __global__ void gathered_prepare_kernel(const unsigned long long* recv, int worl
     st->use_list = 0;
 }
 
+// the rank kernel writes q[idx]: idx = the compacted position (padded = 0), or the key's place in the gathered blocks, r * cap + i
 __global__ void __launch_bounds__(BH_THREADS) gathered_compact_kernel(const unsigned long long* recv, int world, long long cap,
-                                                                      const unsigned long long* offsets, unsigned long long* keys, unsigned* idx) {
+                                                                      const unsigned long long* offsets, unsigned long long* keys, unsigned* idx,
+                                                                      int padded) {
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (int r = 0; r < world; ++r) {
         const unsigned long long off = offsets[r], n = offsets[r + 1] - off;
         const unsigned long long* src = recv + (size_t)r * (size_t)(cap + 1) + 1;
+        const unsigned long long dst0 = padded ? (unsigned long long)r * (unsigned long long)cap : off;
         for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)n; i += stride) {
             keys[off + i] = src[i];
-            idx[off + i] = (unsigned)(off + i);
+            idx[off + i] = (unsigned)(dst0 + i);
         }
     }
 }
@@ -1311,13 +1314,18 @@ extern "C" int bbk_bh_pack_count(const uint64_t* d_state, uint64_t* d_send, void
     return BBK_OK;
 }
 
-extern "C" int bbk_bh_rank_gathered_padded(const uint64_t* d_recv, int32_t world, int64_t cap, int32_t rank, const uint64_t* d_state,
-                                           const uint32_t* d_idx_local, double* d_q_dst, double* d_q_ones, int32_t* d_overflow,
-                                           void* d_workspace, size_t workspace_bytes, void* stream) {
-    BBK_REQUIRE(world > 0 && rank >= 0 && rank < world && cap >= 0, "bbk_bh_rank_gathered_padded: bad world / rank / capacity");
-    BBK_REQUIRE((long long)world * cap < (1ll << 32), "bbk_bh_rank_gathered_padded: world * cap must be below 2^32");
-    BBK_REQUIRE(d_recv && d_state && d_q_ones && d_overflow && d_workspace, "bbk_bh_rank_gathered_padded: null pointer");
-    BBK_REQUIRE(((uintptr_t)d_workspace & 255) == 0, "bbk_bh_rank_gathered_padded: workspace must be 256-byte aligned");
+// what both gathered entries share: prepare, compact, rank (q of gathered key k lands in q_all[idx of k]), export q_ones.
+// rank < 0 (bbk_bh_rank_gathered_all): q_all is the caller's world * cap array in the padded order; otherwise it is the
+// workspace array in compacted order and this rank's slice is scattered to its rows.
+static int rank_gathered(const char* name, const uint64_t* d_recv, int32_t world, int64_t cap, int32_t rank, const uint64_t* d_state,
+                         const uint32_t* d_idx_local, double* d_q_dst, double* d_q_ones, int32_t* d_overflow, void* d_workspace,
+                         size_t workspace_bytes, void* stream) {
+    const char* bad = !(world > 0 && rank < world && cap >= 0) ? "bad world / rank / capacity"
+                    : !((long long)world * cap < (1ll << 32)) ? "world * cap must be below 2^32"
+                    : !(d_recv && d_state && d_q_ones && d_overflow && d_workspace) ? "null pointer"
+                    : !(rank >= 0 || cap == 0 || d_q_dst) ? "null q array"
+                    : ((uintptr_t)d_workspace & 255) ? "workspace must be 256-byte aligned" : nullptr;
+    if (bad) { bbk_set_error("invalid argument: %s: %s", name, bad); return BBK_E_INVALID; }
     const long long n_max = (long long)world * cap;
     const int G = sort_blocks();
     BhLayout L;
@@ -1326,27 +1334,43 @@ extern "C" int bbk_bh_rank_gathered_padded(const uint64_t* d_recv, int32_t world
     used += align256(sizeof(double) * (size_t)(n_max + 1));
     unsigned long long* offsets = (unsigned long long*)((char*)d_workspace + used);
     used += align256(8 * (size_t)(world + 1));
-    if (workspace_bytes < used) { bbk_set_error("bbk_bh_rank_gathered_padded: workspace too small (%zu < %zu bytes)", workspace_bytes, used); return BBK_E_WORKSPACE; }
+    if (workspace_bytes < used) { bbk_set_error("%s: workspace too small (%zu < %zu bytes)", name, workspace_bytes, used); return BBK_E_WORKSPACE; }
+    if (rank < 0) q_all = d_q_dst;
     cudaStream_t st = (cudaStream_t)stream;
     gathered_prepare_kernel<<<1, 32, 0, st>>>((const unsigned long long*)d_recv, world, cap, (const unsigned long long*)d_state, L.st, offsets, d_overflow);
     BBK_CHECK_LAUNCH("gathered_prepare_kernel");
     if (n_max > 0) {
         long long want = (cap + BH_THREADS - 1) / BH_THREADS;
         int grid = (int)(want < (long long)bbk_num_sms() * 4 ? (want > 0 ? want : 1) : (long long)bbk_num_sms() * 4);
-        gathered_compact_kernel<<<grid, BH_THREADS, 0, st>>>((const unsigned long long*)d_recv, world, cap, offsets, L.keys[0], L.idx[0]);
+        gathered_compact_kernel<<<grid, BH_THREADS, 0, st>>>((const unsigned long long*)d_recv, world, cap, offsets, L.keys[0], L.idx[0],
+                                                             rank < 0 ? 1 : 0);
         BBK_CHECK_LAUNCH("gathered_compact_kernel");
     }
     int rc = launch_rank(L, q_all, nullptr, st);
     if (rc != BBK_OK) return rc;
     export_ones_kernel<<<1, 1, 0, st>>>(L.st, d_q_ones);
     BBK_CHECK_LAUNCH("export_ones_kernel");
-    if (cap > 0 && d_idx_local && d_q_dst) {
+    if (rank >= 0 && cap > 0 && d_idx_local && d_q_dst) {
         long long want = (cap + BH_THREADS - 1) / BH_THREADS;
         int grid = (int)(want < (long long)bbk_num_sms() * 4 ? want : (long long)bbk_num_sms() * 4);
         scatter_slice_kernel<<<grid, BH_THREADS, 0, st>>>(q_all, offsets, rank, d_idx_local, d_q_dst);
         BBK_CHECK_LAUNCH("scatter_slice_kernel");
     }
     return BBK_OK;
+}
+
+extern "C" int bbk_bh_rank_gathered_padded(const uint64_t* d_recv, int32_t world, int64_t cap, int32_t rank, const uint64_t* d_state,
+                                           const uint32_t* d_idx_local, double* d_q_dst, double* d_q_ones, int32_t* d_overflow,
+                                           void* d_workspace, size_t workspace_bytes, void* stream) {
+    BBK_REQUIRE(rank >= 0, "bbk_bh_rank_gathered_padded: bad world / rank / capacity");
+    return rank_gathered("bbk_bh_rank_gathered_padded", d_recv, world, cap, rank, d_state, d_idx_local, d_q_dst, d_q_ones, d_overflow,
+                         d_workspace, workspace_bytes, stream);
+}
+
+extern "C" int bbk_bh_rank_gathered_all(const uint64_t* d_recv, int32_t world, int64_t cap, const uint64_t* d_state, double* d_q_all,
+                                        double* d_q_ones, int32_t* d_overflow, void* d_workspace, size_t workspace_bytes, void* stream) {
+    return rank_gathered("bbk_bh_rank_gathered_all", d_recv, world, cap, -1, d_state, nullptr, d_q_all, d_q_ones, d_overflow,
+                         d_workspace, workspace_bytes, stream);
 }
 
 extern "C" int bbk_bh_fix_ones_dev(const double* d_p, int64_t m, const double* d_q_ones, double* d_q, void* stream) {

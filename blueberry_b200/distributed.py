@@ -1063,3 +1063,522 @@ def pack_records(shards, out=None, threads=0):
     nbytes = _io.pack_records(shards, out.buf.data_ptr(), out.buf.numel(), threads)
     out.rows, out.sizes, out.nbytes = rows, sizes, nbytes
     return out
+
+
+# ---------------------------------------------------------------------------------------------------------------------------
+# One genome-wide pass larger than the device: row blocks streamed from host memory
+# ---------------------------------------------------------------------------------------------------------------------------
+BLOCK_ALIGN = _lib.PACK_CHUNK       # every piece starts on a packed-results chunk: its rows unpack straight into the shard's output
+_SMALL_P_KEY = int(np.array([0.03125]).view(np.uint64)[0]) | (1 << 63)      # bbk_key_of(BBK_SMALL_P)
+
+
+def plan_blocks(sizes, block_rows, align=BLOCK_ALIGN):
+    """Cut shards of these sizes, laid end to end, into row blocks of at most `block_rows` rows.  A block is a list of
+    pieces (shard, first row of the shard, rows, device row); every piece starts on a multiple of `align` in the block's
+    device buffers (so of 4, as in layout_rows), the rows between pieces are padding, and a block's device rows
+    (block_device_rows) are at most block_rows rounded up to `align`.  A shard is cut wherever a block fills up (records
+    are independent).  Empty shards get no piece.  Returns the list of blocks."""
+    block_rows, align = int(block_rows), int(align)
+    if align <= 0 or align & 3:
+        raise ValueError("align must be a positive multiple of 4")
+    if block_rows < 1 or (block_rows + align - 1) // align * align >= (1 << 32):
+        raise ValueError("block_rows must be positive and, rounded up to %d, below 2^32; got %d" % (align, block_rows))
+    blocks, cur, used = [], [], 0
+    for s, n in enumerate(sizes):
+        n = int(n)
+        if n < 0:
+            raise ValueError("shard %d has a negative size" % s)
+        first = 0
+        while first < n:
+            take = min(n - first, block_rows - used)
+            cur.append((s, first, take, used))
+            used = (used + take + align - 1) // align * align
+            first += take
+            if used >= block_rows:
+                blocks.append(cur)
+                cur, used = [], 0
+    if cur:
+        blocks.append(cur)
+    return blocks
+
+
+def block_device_rows(block, align=BLOCK_ALIGN):
+    """Device rows of one block of plan_blocks: its last piece's end, rounded up to `align`."""
+    _, _, n, off = block[-1]
+    return (off + n + align - 1) // align * align
+
+
+def resident_pass_bytes(rows, q_values=True):
+    """Device bytes of a resident genome-wide pass over `rows` layout rows (GenomePass, streaming K4): 12 B of records, 8 B of
+    p (and 8 B of q), the deferred list (rows / 4 x 16 B) and the candidate list (rows / 16 x 12 B), plus the q-value
+    workspace of one GPU (bbk_bh_workspace_bytes: 24 B a row)."""
+    rows = int(rows)
+    per = 12 + 8 + 16 / 4 + 12 / 16 + ((8 + 24) if q_values else 0)
+    return int(rows * per)
+
+
+def needs_blocked_pass(rows, free_bytes, q_values=True, margin=1 << 30):
+    """Whether a genome-wide pass over `rows` layout rows cannot run resident on one GPU with `free_bytes` of free device
+    memory (torch.cuda.mem_get_info): 2^32 rows or more, or more bytes than are free after a margin."""
+    return int(rows) >= (1 << 32) or resident_pass_bytes(rows, q_values) + int(margin) > int(free_bytes)
+
+
+def _host_f64(a, n, what):
+    """A float64 host output column of exactly n rows as a numpy view (numpy array or CPU tensor)."""
+    if isinstance(a, torch.Tensor):
+        if a.is_cuda or a.dtype != torch.float64 or not a.is_contiguous():
+            raise ValueError("%s: contiguous float64 host columns (numpy or CPU tensors)" % what)
+        a = a.numpy()
+    if not isinstance(a, np.ndarray) or a.dtype != np.float64 or a.ndim != 1 or not a.flags.c_contiguous or not a.flags.writeable:
+        raise ValueError("%s: contiguous, writable float64 host columns" % what)
+    if a.shape[0] != n:
+        raise ValueError("%s: the column has %d rows, its shard %d" % (what, a.shape[0], n))
+    return a
+
+
+def _host_rows(a, what):
+    """Rows of a host record column (numpy array of integers or a CPU tensor)."""
+    if isinstance(a, torch.Tensor):
+        if a.is_cuda:
+            raise ValueError("%s: host columns (numpy or CPU tensors), not device tensors" % what)
+        return int(a.shape[0]) if a.dim() == 1 else -1
+    a = np.asarray(a)
+    if a.ndim != 1 or a.dtype.kind not in "iu":
+        raise ValueError("%s: one-dimensional integer columns" % what)
+    return int(a.shape[0])
+
+
+class BlockedPass(object):
+    """One genome-wide Fit-Hi-C pass on one GPU over records held in host memory, in row blocks, so that a pass larger than
+    the device (BASELINE config 5: 6.03e9 records, past 2^32 rows and ~197 GB resident) runs, with the same bits as
+    GenomePass(engine, group=False).run over the same shards held resident.
+
+        sweep 1: K1 per piece, block after block, into one table  ->  fit, settled with ONE synchronisation (more bins, the
+        reference's own s, a failed fit raising before any p exists)  ->  sweep 2: per block guard, streaming K4, patch pass,
+        results packed and unpacked into the caller's columns by all host cores  ->  q-values: every block's candidates
+        selected against the genome-wide histogram, as ranks would be, ranked together ONCE (bbk_bh_rank_gathered_all) and
+        scattered on the host  [-> a third sweep over p from the host when the candidate lists do not cover every candidate]
+
+    Blocks whose records fit `resident_bytes` stay on the device between the sweeps; the others are sent again.  The inbound
+    copy of block k + 1 overlaps the kernels of block k, which overlap the outbound copy of block k - 1.
+    engine: a PassEngine over the whole genome (set_fragments / set_bias as for GenomePass), with the streaming K4's
+    conditions (GenomePass.listed): 0 <= min_dist <= max_dist, max_dist + resolution < 2^31, resolution >= 2, no bias table
+    of step 1.  Otherwise ValueError."""
+
+    def __init__(self, engine, q_values=True, block_rows=1 << 27, resident_bytes=None, cand_capacity=None):
+        e = engine
+        if not (0 <= e.min_dist <= e.max_dist and e.max_dist + e.R < (1 << 31) and e.R >= 2) or \
+                (e.bias is not None and e.bias.step == 1):
+            raise ValueError("BlockedPass runs the streaming K4 only (the conditions of GenomePass.listed)")
+        plan_blocks([], block_rows)                       # checks block_rows
+        self.eng, self.lib, self.device = e, e.lib, e.device
+        self.q_values = bool(q_values)
+        self.block_rows = int(block_rows)
+        self.resident_bytes = None if resident_bytes is None else int(resident_bytes)
+        self.cand_capacity = None if cand_capacity is None else max(int(cand_capacity), 1)
+        self.force_exact = False        # tests: raise BbkScoreState.exact whatever the guard says
+        self.blocks, self.resident = [], []
+        self.bytes_in = self.bytes_out = 0
+        self.host_unpack_s = 0.0
+
+    @property
+    def launches(self):
+        """Kernel launches counted so far (the engine's counter)."""
+        return self.eng.launches
+
+    @launches.setter
+    def launches(self, n):
+        self.eng.launches = n
+
+    # ------------------------------------------------------------------ checks
+    def check(self, shards, p_out, q_out=None):
+        """Raise ValueError unless the arguments of run() are complete; returns (sizes, p columns, q columns)."""
+        shards = list(shards)
+        sizes, ps, qs = [], [], []
+        if p_out is None or len(p_out) != len(shards):
+            raise ValueError("p_out: one column per shard")
+        if self.q_values and (q_out is None or len(q_out) != len(shards)):
+            raise ValueError("q_out: one column per shard (the pass was made with q_values=True)")
+        if not self.q_values and q_out is not None:
+            raise ValueError("q_out given, but the pass was made with q_values=False")
+        for i, sh in enumerate(shards):
+            if len(sh) != 4:
+                raise ValueError("shard %d: (chrom, mid1, mid2, count); BlockedPass takes one-chromosome shards" % i)
+            n = _host_rows(sh[1], "shard %d" % i)
+            if n < 0 or _host_rows(sh[2], "shard %d" % i) != n or _host_rows(sh[3], "shard %d" % i) != n:
+                raise ValueError("shard %d: the columns differ in length" % i)
+            sizes.append(n)
+            ps.append(_host_f64(p_out[i], n, "p_out[%d]" % i))
+            qs.append(_host_f64(q_out[i], n, "q_out[%d]" % i) if self.q_values else None)
+        blocks = plan_blocks(sizes, self.block_rows)
+        cc = self._cand_cap(blocks)
+        if len(blocks) * cc >= (1 << 32):
+            raise ValueError("%d blocks of %d candidate places reach 2^32: use larger blocks" % (len(blocks), cc))
+        return sizes, ps, qs
+
+    def _cand_cap(self, blocks):
+        if self.cand_capacity:
+            return self.cand_capacity
+        most = max([block_device_rows(b) for b in blocks] + [4])
+        return min(most, max(1 << 20, self.block_rows // 16))
+
+    # ------------------------------------------------------------------ helpers
+    def _copy_piece(self, dst, col, lo, n):
+        """Rows [lo, lo + n) of a host column into the device view dst (current stream)."""
+        if isinstance(col, torch.Tensor) and col.dtype == torch.int32 and col.is_pinned():
+            dst.copy_(col[lo:lo + n], non_blocking=True)
+        else:
+            from .fithic import _to_device_i32
+            dst.copy_(_to_device_i32(col, self.device, lo, lo + n), non_blocking=True)
+        self.bytes_in += 4 * n
+
+    def _records_in(self, k, cols, stream, ready):
+        """The pieces of block k into its record columns, on `stream`; `ready` fires when they are there."""
+        with torch.cuda.stream(stream):
+            for (s, lo, n, off) in self.blocks[k]:
+                for dst, j in zip(cols, (1, 2, 3)):
+                    self._copy_piece(dst[off:off + n], self._shards[s][j], lo, n)
+            ready.record(stream)
+
+    def _pieces(self, k, cols):
+        return [(self._shards[s][0], Shard(cols[0][off:off + n], cols[1][off:off + n], cols[2][off:off + n], chrom=self._shards[s][0]), off)
+                for (s, lo, n, off) in self.blocks[k]]
+
+    def _nan_padding(self, k, p, q):
+        """Padding rows of block k (between its pieces and up to its device rows) = NaN in p / q (the pack sees them as empty)."""
+        blk = self.blocks[k]
+        ends = [off + n for (_, _, n, off) in blk]
+        starts = [off for (_, _, _, off) in blk[1:]] + [block_device_rows(blk)]
+        for a, b in zip(ends, starts):
+            if b > a:
+                p[a:b] = float("nan")
+                if q is not None:
+                    q[a:b] = float("nan")
+                self.eng.launches += 1 if q is None else 2
+
+    # ------------------------------------------------------------------ the pass
+    def run(self, shards, p_out, q_out=None, n_tests=-1, marks=None):
+        """Run the pass.  shards: [(chrom, mid1, mid2, count)], host columns (numpy integer arrays, or CPU tensors; pinned int32
+        tensors go by one asynchronous copy each).  p_out / q_out: one float64 host column per shard, exactly as long as it
+        (numpy arrays or CPU tensors); q_out only with q_values.  n_tests: N of the q-values (-1: the number of non-NaN p).
+        marks (optional dict): CUDA events recorded after each stage.  Returns the FitResult; a failed fit raises what
+        GenomePass.run raises, before any p is computed and with p_out / q_out untouched."""
+        sizes, ps, qs = self.check(shards, p_out, q_out)
+        eng, lib, dev = self.eng, self.lib, self.device
+        self._shards = [tuple(sh) for sh in shards]
+        self.blocks = plan_blocks(sizes, self.block_rows)
+        self.bytes_in = self.bytes_out = 0
+        self.host_unpack_s = 0.0
+        nb = len(self.blocks)
+        dev_rows = [block_device_rows(b) for b in self.blocks]
+        main = torch.cuda.current_stream(dev)
+        st = _lib.stream_ptr(main)
+
+        def mark(name):
+            if marks is not None:
+                ev = torch.cuda.Event(enable_timing=True)
+                ev.record(main)
+                marks[name] = ev
+
+        mark("start")
+        # the working set (sized by block_rows), then the records of as many blocks as the budget holds, in order
+        br = self.block_rows
+        ns = ctypes.sizeof(_lib.ScoreState)
+        self.score_state = torch.zeros(max(nb, 1) * ns, dtype=torch.uint8, device=dev)
+        self._h_state = torch.zeros(max(nb, 1) * ns, dtype=torch.uint8).pin_memory()
+        slot_rows = max(dev_rows + [4])
+        pq = [(torch.empty(slot_rows, dtype=torch.float64, device=dev),
+               torch.empty(slot_rows, dtype=torch.float64, device=dev) if self.q_values else None) for _ in range(min(nb, 2))]
+        packs = [DevicePack(slot_rows, dev, self.q_values) for _ in range(len(pq))]
+        h_packs = [PackedScores(slot_rows, pk.codes.numel(), pk.chunks.numel() // 24, pk.cap_p, pk.cap_q) for pk in packs]
+        h_pack_state = [torch.zeros(ctypes.sizeof(_lib.PackState), dtype=torch.uint8).pin_memory() for _ in packs]
+        l_cap = slot_rows                                  # the deferred list has a place for every row of a block: no overflow
+        l_row = torch.empty(l_cap, dtype=torch.int32, device=dev)
+        l_cnt = torch.empty(l_cap, dtype=torch.int32, device=dev)
+        l_prior = torch.empty(l_cap, dtype=torch.float64, device=dev)
+        deferred = _lib.DeferredList(l_row.data_ptr(), l_cnt.data_ptr(), l_prior.data_ptr(), l_cap)
+        ccap = self._cand_cap(self.blocks)
+        cands = []
+        if self.q_values:
+            for _ in range(nb):
+                keys = torch.empty(ccap, dtype=torch.int64, device=dev)
+                rows = torch.empty(ccap, dtype=torch.int32, device=dev)
+                cands.append((keys, rows, _lib.Candidates(keys.data_ptr(), rows.data_ptr(), ccap)))
+        slot_bytes = 12 * slot_rows
+        budget = self.resident_bytes
+        if budget is None:
+            free, total = torch.cuda.mem_get_info(dev)
+            budget = free - max(1 << 30, total // 50) - 2 * slot_bytes
+        self.resident, used = [], 0
+        for r in dev_rows:
+            keep = used + 12 * r <= budget
+            self.resident.append(keep)
+            used += 12 * r if keep else 0
+        # resident blocks get their own columns; the others share two slots
+        cols = [tuple(torch.empty(r, dtype=torch.int32, device=dev) for _ in range(3)) if keep else None
+                for r, keep in zip(dev_rows, self.resident)]
+        slots = [tuple(torch.empty(slot_rows, dtype=torch.int32, device=dev) for _ in range(3)) for _ in range(2)] \
+            if not all(self.resident) else []
+        far = [k for k in range(nb) if not self.resident[k]]         # blocks sent again in sweep 2, in turn through the two slots
+        slot_of = {k: i & 1 for i, k in enumerate(far)}
+        s_in, s_out = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
+        s_in.wait_stream(main)
+        s_out.wait_stream(main)
+        in_ready = [torch.cuda.Event() for _ in range(nb)]
+        slot_free = [torch.cuda.Event() for _ in range(2)]
+
+        def block_cols(k):
+            return cols[k] if self.resident[k] else slots[slot_of[k]]
+
+        def send(k):
+            if not self.resident[k]:
+                s_in.wait_event(slot_free[slot_of[k]])        # the kernels that last read this slot have finished
+            self._records_in(k, block_cols(k), s_in, in_ready[k])
+
+        # ---- sweep 1: K1 into one table
+        _lib.check(lib.bbk_hist_init(_lib.ptr(eng.obs_sum), eng.nkeys, _lib.ptr(eng.totals), st), "bbk_hist_init")
+        eng.launches += 1
+        if nb:
+            send(0)
+        for k in range(nb):
+            if k + 1 < nb:
+                send(k + 1)
+            main.wait_event(in_ready[k])
+            for _, sh, _ in self._pieces(k, block_cols(k)):
+                _lib.check(lib.bbk_hist_pairs(None, None, _lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, eng.R, eng.min_dist,
+                                              eng.max_dist, eng.nkeys, _lib.ptr(eng.obs_sum), _lib.ptr(eng.totals), st), "bbk_hist_pairs")
+                eng.launches += 1
+            if not self.resident[k]:
+                slot_free[slot_of[k]].record(main)
+        mark("hist")
+
+        # ---- the fit, settled on the host once
+        fit = self._settle_fit()
+        mark("fit")
+
+        # ---- sweep 2: scores, block after block; results packed, unpacked into the caller's columns by the host
+        want_q = self.q_values
+        hist = _lib.ptr(eng.p_hist) if want_q else None
+        bias = ctypes.byref(eng.bias.struct) if eng.bias is not None else None
+        flags = _lib.ptr(eng.bias.flags) if eng.bias is not None else None
+        run_done = [torch.cuda.Event() for _ in range(2)]
+        counts_ready = [torch.cuda.Event() for _ in range(2)]
+        out_free = [torch.cuda.Event() for _ in range(2)]
+        if nb == 0 and want_q:
+            eng.p_hist.zero_()
+            eng.launches += 1
+        pending = None
+        if far:
+            send(far[0])
+        for k in range(nb):
+            if not self.resident[k]:
+                i = far.index(k)
+                if i + 1 < len(far):
+                    send(far[i + 1])                      # into the other slot, while block k is scored
+                main.wait_event(in_ready[k])
+            j = k & 1
+            p, q = pq[j]
+            main.wait_event(out_free[j])                  # this slot's previous results have left the device
+            self._nan_padding(k, p, q)
+            state = ctypes.c_void_p(self.score_state.data_ptr() + k * ns)
+            _lib.check(lib.bbk_score_begin(state, hist if k == 0 else None, st), "bbk_score_begin")
+            _lib.check(lib.bbk_score_guard(_lib.ptr(eng.fit_result), _lib.ptr(eng.spline_y), state, st), "bbk_score_guard")
+            eng.launches += 2
+            if self.force_exact:
+                self.score_state[k * ns + 24:k * ns + 28] = torch.tensor([1, 0, 0, 0], dtype=torch.uint8, device=dev)
+            cand = ctypes.byref(cands[k][2]) if want_q else None
+            pieces = self._pieces(k, block_cols(k))
+            for (_, sh, off), st_i in zip(pieces, eng.fan_out(len(pieces))):
+                _lib.check(lib.bbk_score_pairs(_lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, sh.chrom, eng.R, eng.min_dist,
+                                               eng.max_dist, _lib.ptr(eng.fit_result), _lib.ptr(eng.spline_y), bias, flags, off,
+                                               _lib.ptr(p), _lib.ptr(q) if want_q else None, hist, cand, ctypes.byref(deferred), state,
+                                               st_i), "bbk_score_pairs")
+                eng.launches += 1
+            eng.fan_in()
+            _lib.check(lib.bbk_score_deferred(ctypes.byref(deferred), _lib.ptr(eng.fit_result), _lib.ptr(p), _lib.ptr(q) if want_q else None,
+                                              hist, cand, state, st), "bbk_score_deferred")
+            eng.launches += 1
+            if not self.resident[k]:
+                slot_free[slot_of[k]].record(main)
+            pk = packs[j]
+            pk.rows = dev_rows[k]
+            pk.pack(p, q, main)
+            eng.launches += 2
+            run_done[j].record(main)
+            s_out.wait_event(run_done[j])
+            hp = h_packs[j]
+            with torch.cuda.stream(s_out):
+                h_pack_state[j].copy_(pk.state, non_blocking=True)
+                self._h_state[k * ns:(k + 1) * ns].copy_(self.score_state[k * ns:(k + 1) * ns], non_blocking=True)
+                nw, nc = int(lib.bbk_pack_code_words(dev_rows[k])), int(lib.bbk_pack_chunks(dev_rows[k])) * 24
+                hp.codes[:nw].copy_(pk.codes[:nw], non_blocking=True)
+                hp.chunks[:nc].copy_(pk.chunks[:nc], non_blocking=True)
+                self.bytes_out += 4 * nw + nc
+                counts_ready[j].record(s_out)
+            if pending is not None:
+                self._unpack(*pending)
+            pending = (k, j, p, q, pk, hp, h_pack_state[j], counts_ready[j], out_free[j], s_out, ps, qs)
+        if pending is not None:
+            self._unpack(*pending)
+        s_out.synchronize()
+        mark("pvalues")
+        states = [_lib.ScoreState.from_buffer_copy(self._h_state.numpy().tobytes()[k * ns:(k + 1) * ns]) for k in range(nb)]
+        if any(s.overflow for s in states):
+            raise _lib.BbkError("a block's deferred list overflowed")     # it has a place for every row: cannot happen
+        self.last_states = states
+        # the records are not needed any more: the q-value step gets their memory
+        cols = slots = packs = pq = pending = None
+        if want_q and nb:
+            self._qvalues(int(n_tests), states, cands, ps, qs, dev_rows)
+        mark("bh")
+        return fit
+
+    def _settle_fit(self, smoothing=None):
+        eng = self.eng
+        host = torch.zeros(eng.fit_result.numel(), dtype=torch.uint8).pin_memory()
+        for _ in range(6):
+            eng.fit(smoothing)
+            host.copy_(eng.fit_result, non_blocking=True)
+            torch.cuda.current_stream(self.device).synchronize()
+            raw = host.numpy().tobytes()
+            if _lib.FitResult.from_buffer_copy(raw).status == _lib.FIT_TOO_MANY_BINS and eng.grow_bins():
+                continue                                          # more bins than the default buffers hold: one per key
+            fit = PassEngine.decode_fit(raw)                      # raises what the reference would raise
+            s_ref = PassEngine.reference_smoothing(fit)
+            if s_ref is None:
+                return fit
+            smoothing = s_ref
+        raise _lib.BbkError("the fit did not settle after 6 attempts")
+
+    def _unpack(self, k, j, p, q, pk, hp, h_state, counts_ready, out_free, s_out, ps, qs):
+        """Block k's packed results (slot j) into the caller's columns: the value lists follow once their sizes are known, then
+        every piece is unpacked by all host cores straight into its shard's rows."""
+        import time
+        counts_ready.synchronize()
+        pst = _lib.PackState.from_buffer_copy(h_state.numpy().tobytes())
+        blk = self.blocks[k]
+        with torch.cuda.stream(s_out):
+            if pst.overflow:                      # more values than the lists hold: the columns come back dense, piece by piece
+                for (s, lo, n, off) in blk:
+                    torch.from_numpy(ps[s][lo:lo + n]).copy_(p[off:off + n])
+                    if q is not None:
+                        torch.from_numpy(qs[s][lo:lo + n]).copy_(q[off:off + n])
+                    self.bytes_out += 8 * n * (2 if q is not None else 1)
+                out_free.record(s_out)
+                return
+            n_p, n_q = int(pst.n_p), int(pst.n_q)
+            if n_p:
+                hp.vals_p[:n_p].copy_(pk.vals_p[:n_p], non_blocking=True)
+            if n_q and pk.vals_q is not None:
+                hp.vals_q[:n_q].copy_(pk.vals_q[:n_q], non_blocking=True)
+            self.bytes_out += 8 * (n_p + n_q)
+            out_free.record(s_out)
+        out_free.synchronize()
+        t0 = time.perf_counter()
+        codes, chunks = hp.codes.numpy(), hp.chunks.numpy()
+        vp, vq = hp.vals_p.numpy(), (hp.vals_q.numpy() if hp.vals_q is not None else None)
+        for (s, lo, n, off) in blk:
+            _io.unpack_scores(codes[off // 16:], chunks[off // _lib.PACK_CHUNK * 24:], vp, vq, n, ps[s][lo:lo + n],
+                              qs[s][lo:lo + n] if q is not None else None, want_q=q is not None)
+        self.host_unpack_s += time.perf_counter() - t0
+
+    # ------------------------------------------------------------------ q-values across blocks
+    def _qvalues(self, n_tests, states, cands, ps, qs, dev_rows):
+        """The genome-wide q-value step with the blocks as ranks: candidates selected per block against the global histogram,
+        ranked together once, scattered into q_out through the piece map; the p == 1.0 group fixed on the host when its q is
+        below 1.  The candidate lists cover every candidate unless the saturation bucket is at or above 2^-5 or a list
+        overflowed: then a third sweep selects from p itself, uploaded from p_out."""
+        eng, lib, dev = self.eng, self.lib, self.device
+        nb = len(self.blocks)
+        ns = ctypes.sizeof(_lib.ScoreState)
+        st = _lib.stream_ptr()
+        self.sel_ws = torch.empty(int(lib.bbk_bh_workspace_bytes(0)), dtype=torch.uint8, device=dev)
+        listed = not any(s.cand_overflow for s in states)
+        cap = max([int(s.n_cand) for s in states] + [1])
+        scratch = None
+        for _ in range(4):
+            if nb * cap >= (1 << 32):
+                raise _lib.BbkError("%d blocks of %d q-value candidates reach 2^32: use larger blocks" % (nb, cap))
+            recv = torch.zeros(nb * (cap + 1), dtype=torch.int64, device=dev)
+            idx = torch.empty(nb * cap, dtype=torch.int32, device=dev)
+            bh_state = torch.zeros(4 * nb, dtype=torch.int64, device=dev)
+            q_all = torch.empty(nb * cap, dtype=torch.float64, device=dev)
+            q_ones = torch.zeros(2, dtype=torch.float64, device=dev)
+            overflow = torch.zeros(1, dtype=torch.int32, device=dev)
+            ws = torch.empty(int(lib.bbk_bh_gathered_workspace_bytes(nb, cap)), dtype=torch.uint8, device=dev)
+            if scratch is None:
+                rows = max(dev_rows)
+                scratch = (torch.empty(rows, dtype=torch.float64, device=dev), torch.empty(rows, dtype=torch.float64, device=dev))
+            sp, sq = scratch
+            for k in range(nb):
+                keys = ctypes.c_void_p(recv.data_ptr() + 8 * (k * (cap + 1) + 1))
+                kidx = ctypes.c_void_p(idx.data_ptr() + 4 * k * cap)
+                kst = ctypes.c_void_p(bh_state.data_ptr() + 32 * k)
+                m = dev_rows[k]
+                if listed:
+                    # p / q are read only when the list does not cover every candidate: that result is discarded below
+                    _lib.check(lib.bbk_bh_select_listed(_lib.ptr(sp), m, n_tests, _lib.ptr(eng.p_hist), _lib.ptr(sq), ctypes.byref(cands[k][2]),
+                                                        ctypes.c_void_p(self.score_state.data_ptr() + k * ns), keys, kidx, cap, kst,
+                                                        _lib.ptr(self.sel_ws), self.sel_ws.numel(), st), "bbk_bh_select_listed")
+                    eng.launches += 5           # init, threshold, candidate filter, compact (returns at once), export
+                else:
+                    self._p_in(k, sp, ps)
+                    _lib.check(lib.bbk_bh_select(_lib.ptr(sp), m, n_tests, _lib.ptr(eng.p_hist), _lib.ptr(sq), keys, kidx, cap, kst,
+                                                 _lib.ptr(self.sel_ws), self.sel_ws.numel(), st), "bbk_bh_select")
+                    eng.launches += 4           # init, threshold, compact, export
+                _lib.check(lib.bbk_bh_pack_count(kst, ctypes.c_void_p(recv.data_ptr() + 8 * k * (cap + 1)), st), "bbk_bh_pack_count")
+                eng.launches += 1
+            _lib.check(lib.bbk_bh_rank_gathered_all(_lib.ptr(recv), nb, cap, _lib.ptr(bh_state), _lib.ptr(q_all), _lib.ptr(q_ones),
+                                                    _lib.ptr(overflow), _lib.ptr(ws), ws.numel(), st), "bbk_bh_rank_gathered_all")
+            eng.launches += 4                   # prepare, compact, rank, export
+            h_state = bh_state.cpu().numpy().view(np.uint64).reshape(nb, 4)
+            ov = int(overflow.item())
+            if listed and int(h_state[0, 1]) > _SMALL_P_KEY:
+                listed = False                  # saturation at or above 2^-5: the lists miss candidates
+                continue
+            if ov:
+                cap = ov                        # the largest block count: every block fits now
+                continue
+            break
+        else:
+            raise _lib.BbkError("the q-value step did not settle")
+        counts = h_state[:, 0].astype(np.int64)
+        self.tau_key, self.n_candidates = int(h_state[0, 1]), int(counts.sum())       # for a caller's checks
+        h_q, h_idx = q_all.cpu().numpy(), idx.cpu().numpy().view(np.uint32)
+        h_ones = q_ones.cpu().numpy()
+        for k, blk in enumerate(self.blocks):
+            n = int(counts[k])
+            if not n:
+                continue
+            rows = h_idx[k * cap:k * cap + n].astype(np.int64)
+            vals = h_q[k * cap:k * cap + n]
+            offs = np.array([off for (_, _, _, off) in blk], dtype=np.int64)
+            which = np.searchsorted(offs, rows, side="right") - 1
+            for i, (s, lo, pn, off) in enumerate(blk):
+                sel = which == i
+                if sel.any():
+                    qs[s][lo + rows[sel] - off] = vals[sel]
+        if h_ones[1] != 0.0:                    # q of the p == 1.0 group is below 1 (N below the number of emitted rows)
+            self._fix_ones(ps, qs, float(h_ones[0]))
+
+    def _p_in(self, k, sp, ps):
+        """Block k's p from the caller's columns into the device column sp (padding rows NaN), for the pass over p."""
+        blk = self.blocks[k]
+        self._nan_padding(k, sp, None)
+        for (s, lo, n, off) in blk:
+            sp[off:off + n].copy_(torch.from_numpy(ps[s][lo:lo + n]), non_blocking=True)
+            self.bytes_in += 8 * n
+
+    @staticmethod
+    def _fix_ones(ps, qs, q_ones, chunk=1 << 24):
+        """q = q_ones wherever p == 1.0, by all host cores (numpy releases the GIL in both calls)."""
+        import os
+        from concurrent.futures import ThreadPoolExecutor
+        jobs = [(p, q, a) for p, q in zip(ps, qs) for a in range(0, len(p), chunk)]
+
+        def one(job):
+            p, q, a = job
+            np.copyto(q[a:a + chunk], q_ones, where=p[a:a + chunk] == 1.0)
+
+        with ThreadPoolExecutor(max_workers=os.cpu_count() or 1) as ex:
+            list(ex.map(one, jobs))

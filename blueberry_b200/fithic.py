@@ -356,7 +356,7 @@ def _in_range_possible(possible, resolution, min_dist, max_dist):
 
 def _run_pass(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1, mid1, chr2, mid2, count,
               bias_dic=None, want_q=False, n_tests=None, keep_device=False, refit=False, group=None):
-    from .distributed import GenomePass, _world, shard_rows
+    from .distributed import BlockedPass, GenomePass, _world, shard_rows
     dev = _device()
     info = _frag_info(frag_chrom, frag_mid, resolution)
     eng = PassEngine(resolution, n_bins, min_dist, max_dist, info.nkeys, dev)
@@ -392,6 +392,18 @@ def _run_pass(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1
         fit = gp2.run(n_tests=nt, exclude=(gp1.p, 1.0 / in_rng))      # raises what the reference would raise
         first = gp1.shard_p(0)
         p_rows, q_rows = gp2.shard_p(0), (gp2.shard_q(0) if want_q else None)
+    elif world == 1 and group is False and _blocked_ok(eng) and use_blocked_pass(n_rows + 3 * 64, want_q, dev) and \
+            (runs := compact_runs(chr1, chr2, n_rows)) is not None:
+        # (n_rows + 3 * 64: at least the layout rows of the runs, at most 64 of them)
+        # larger than the device (or than 2^32 rows): the same pass in row blocks from host memory
+        p = np.empty(n_rows, dtype=np.float64)
+        q = np.empty(n_rows, dtype=np.float64) if want_q else None
+        bp = BlockedPass(eng, q_values=want_q)
+        fit = bp.run([(c, mid1[a:b], mid2[a:b], count[a:b]) for c, a, b in runs], [p[a:b] for _, a, b in runs],
+                     [q[a:b] for _, a, b in runs] if want_q else None, n_tests=nt)
+        out = _pass_output(eng, fit, info, resolution, min_dist, max_dist, None, None, None, dev, scores=(p, q))
+        out.rows = (lo, hi)
+        return out
     else:
         gp = GenomePass(eng, group=group, q_values=want_q)
         shards = _rows_to_shards(chr1, mid1, chr2, mid2, count, lo, hi, dev)
@@ -408,8 +420,41 @@ def _run_pass(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1
     return out
 
 
-def _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows, first, dev):
-    """PassOutput of one finished pass: the engine's tables and fit, p / q / keep of the given rows."""
+def compact_runs(chr1, chr2, n_rows, max_runs=64):
+    """The compact shards _rows_to_shards forms, found on the host: [(chrom, first row, end row)] of the runs of
+    intra-chromosomal rows (one run of chromosome 0 without chromosome columns), or None when the records do not fall into
+    fewer than max_runs such runs (inter-chromosomal rows, interleaved chromosomes)."""
+    if chr1 is None:
+        return [(0, 0, int(n_rows))]
+    c1, c2 = np.asarray(chr1), np.asarray(chr2)
+    if int(n_rows) == 0 or not np.array_equal(c1, c2):
+        return None
+    cuts = np.flatnonzero(c1[1:] != c1[:-1]) + 1
+    if len(cuts) >= max_runs:
+        return None
+    bounds = [0] + cuts.tolist() + [int(n_rows)]
+    return [(int(c1[a]), a, b) for a, b in zip(bounds[:-1], bounds[1:])]
+
+
+def _blocked_ok(eng):
+    """The streaming K4 applies to this engine (GenomePass.listed without chromosome columns)."""
+    return 0 <= eng.min_dist <= eng.max_dist and eng.max_dist + eng.R < (1 << 31) and eng.R >= 2 and \
+        not (eng.bias is not None and eng.bias.step == 1)
+
+
+def use_blocked_pass(rows, want_q, dev):
+    """Whether a single-GPU genome-wide pass over `rows` layout rows goes through distributed.BlockedPass: when the resident
+    pass cannot run (2^32 rows or more, or more device memory than is free: distributed.needs_blocked_pass)."""
+    from .distributed import needs_blocked_pass
+    if int(rows) >= (1 << 32):
+        return True
+    free, _ = torch.cuda.mem_get_info(dev)
+    return needs_blocked_pass(rows, free, want_q)
+
+
+def _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows, first, dev, scores=None):
+    """PassOutput of one finished pass: the engine's tables and fit, p / q / keep of the given rows (or of the host columns
+    scores = (p, q) a BlockedPass has filled)."""
     out = PassOutput()
     out.fit = fit
     out.frag = info
@@ -417,7 +462,11 @@ def _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows,
             "spline_y": _to_host(eng.spline_y[:fit.L]), "spline_raw": _to_host(eng.spline_raw[:fit.L]),
             "possible": _to_host(eng.possible), "observed": _to_host(eng.obs_sum), "bin_of_key": _to_host(eng.bin_of_key),
             "totals": _to_host(eng.totals), "first": _to_host(first) if first is not None else None}
-    out.p, out.q, out.keep = _scores_to_host(p_rows, q_rows, dev)    # keep: fithic.py:434 (NaN = not scored or dropped)
+    if scores is None:
+        out.p, out.q, out.keep = _scores_to_host(p_rows, q_rows, dev)    # keep: fithic.py:434 (NaN = not scored or dropped)
+    else:
+        out.p, out.q = scores
+        out.keep = out.p <= 1.0
     torch.cuda.current_stream(dev).synchronize()
     out.x = host["x"].numpy()
     out.y = host["y"].numpy()

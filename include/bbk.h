@@ -418,6 +418,12 @@ int bbk_bh_pack_count(const uint64_t* d_state, uint64_t* d_send, void* stream);
 int bbk_bh_rank_gathered_padded(const uint64_t* d_recv, int32_t world, int64_t cap, int32_t rank, const uint64_t* d_state,
                                 const uint32_t* d_idx_local, double* d_q_dst, double* d_q_ones, int32_t* d_overflow,
                                 void* d_workspace, size_t workspace_bytes, void* stream);
+/* The same ranking without the per-rank scatter, for one GPU that plays every rank itself (row blocks of a pass larger than
+ * the device, distributed.BlockedPass): all gathered keys are sorted once and d_q_all[r * cap + i] receives the q of block
+ * r's candidate i, for i below that block's count (the other places are left as they are).  d_q_all: world * cap doubles;
+ * d_q_ones and d_overflow as above; world * cap < 2^32.  Workspace: bbk_bh_gathered_workspace_bytes(world, cap). */
+int bbk_bh_rank_gathered_all(const uint64_t* d_recv, int32_t world, int64_t cap, const uint64_t* d_state, double* d_q_all,
+                             double* d_q_ones, int32_t* d_overflow, void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K6  count_band_regions                               replaces blueberry.pyx:77-91
