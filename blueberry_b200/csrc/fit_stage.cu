@@ -293,9 +293,11 @@ __device__ __forceinline__ void fit_body(const FitParams& P) {
             }
             __syncthreads();
             const int n = sh.st.n;
+            // the search solves for n - 4 coefficients and never writes c[n-4 .. n): that is stale pool or workspace memory,
+            // where scipy's array (ius._data[9]) holds zeros
             for (int i = tid; i < m + 4; i += FIT_THREADS) {
                 P.knots[i] = i < n ? cw.w.t[i] : 0.0;
-                P.coefs[i] = i < n ? cw.w.c[i] : 0.0;
+                P.coefs[i] = i < n - 4 ? cw.w.c[i] : 0.0;
             }
             __syncthreads();
         }
