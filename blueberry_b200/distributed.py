@@ -1108,19 +1108,21 @@ def block_device_rows(block, align=BLOCK_ALIGN):
     return (off + n + align - 1) // align * align
 
 
-def resident_pass_bytes(rows, q_values=True):
+def resident_pass_bytes(rows, q_values=True, refit=False):
     """Device bytes of a resident genome-wide pass over `rows` layout rows (GenomePass, streaming K4): 12 B of records, 8 B of
     p (and 8 B of q), the deferred list (rows / 4 x 16 B) and the candidate list (rows / 16 x 12 B), plus the q-value
-    workspace of one GPU (bbk_bh_workspace_bytes: 24 B a row)."""
+    workspace of one GPU (bbk_bh_workspace_bytes: 24 B a row).  refit: the two-pass workload of fit_transform_arrays(refit=True),
+    whose pass 1 holds its own p, deferred list and candidate list while the refit pass runs."""
     rows = int(rows)
-    per = 12 + 8 + 16 / 4 + 12 / 16 + ((8 + 24) if q_values else 0)
+    per = 12 + 8 + 16 / 4 + 12 / 16 + ((8 + 24) if q_values else 0) + ((8 + 16 / 4 + 12 / 16) if refit else 0)
     return int(rows * per)
 
 
-def needs_blocked_pass(rows, free_bytes, q_values=True, margin=1 << 30):
+def needs_blocked_pass(rows, free_bytes, q_values=True, margin=1 << 30, refit=False):
     """Whether a genome-wide pass over `rows` layout rows cannot run resident on one GPU with `free_bytes` of free device
-    memory (torch.cuda.mem_get_info): 2^32 rows or more, or more bytes than are free after a margin."""
-    return int(rows) >= (1 << 32) or resident_pass_bytes(rows, q_values) + int(margin) > int(free_bytes)
+    memory (torch.cuda.mem_get_info): 2^32 rows or more, or more bytes than are free after a margin.  refit: the two-pass
+    workload (resident_pass_bytes)."""
+    return int(rows) >= (1 << 32) or resident_pass_bytes(rows, q_values, refit) + int(margin) > int(free_bytes)
 
 
 def _host_f64(a, n, what):
@@ -1163,9 +1165,22 @@ class BlockedPass(object):
     copy of block k + 1 overlaps the kernels of block k, which overlap the outbound copy of block k - 1.
     engine: a PassEngine over the whole genome (set_fragments / set_bias as for GenomePass), with the streaming K4's
     conditions (GenomePass.listed): 0 <= min_dist <= max_dist, max_dist + resolution < 2^31, resolution >= 2, no bias table
-    of step 1.  Otherwise ValueError."""
+    of step 1.  Otherwise ValueError.
 
-    def __init__(self, engine, q_values=True, block_rows=1 << 27, resident_bytes=None, cand_capacity=None):
+    refit=True runs the two-pass workload of BASELINE config 4 (fit_transform_arrays(refit=True)) with the same bits as the
+    resident two-pass (GenomePass(q_values=False).run, then GenomePass.run(exclude=(p_first, p_outlier)) on the same engine):
+
+        sweep 1: K1 into table 1  ->  fit 1, settled (fit_first)  ->  sweep 2: per block pass 1's scores into the block's p
+        slot, then K1 over the block's rows whose pass-1 p is not <= p_outlier into table 2 (the engine's tables, refilled:
+        pass-1 scoring reads only the fit and the spline)  [-> pass 1's p packed into p_first_out]  ->  fit 2, settled  ->
+        sweep 3 and the q-values as above
+
+    Pass 1's p never crosses the link for the refit itself; the records of the blocks that are not resident cross it once
+    per sweep.  The outlier threshold p_outlier = 1 / possibleIntraInRangeCount depends on the fragments alone and is
+    computed here, as fit_transform_arrays(refit=True) computes it; a count <= 0 raises ZeroDivisionError before any device
+    work."""
+
+    def __init__(self, engine, q_values=True, block_rows=1 << 27, resident_bytes=None, cand_capacity=None, refit=False):
         e = engine
         if not (0 <= e.min_dist <= e.max_dist and e.max_dist + e.R < (1 << 31) and e.R >= 2) or \
                 (e.bias is not None and e.bias.step == 1):
@@ -1176,8 +1191,17 @@ class BlockedPass(object):
         self.block_rows = int(block_rows)
         self.resident_bytes = None if resident_bytes is None else int(resident_bytes)
         self.cand_capacity = None if cand_capacity is None else max(int(cand_capacity), 1)
+        self.refit = bool(refit)
+        self.p_outlier = None
+        if self.refit:
+            from .fithic import _in_range_possible
+            in_rng = _in_range_possible(e.possible.cpu().numpy(), e.R, e.min_dist, e.max_dist)
+            if in_rng <= 0:
+                raise ZeroDivisionError("float division by zero (possibleIntraInRangeCount == 0)")
+            self.p_outlier = 1.0 / in_rng
         self.force_exact = False        # tests: raise BbkScoreState.exact whatever the guard says
         self.blocks, self.resident = [], []
+        self.fit_first = None
         self.bytes_in = self.bytes_out = 0
         self.host_unpack_s = 0.0
 
@@ -1191,16 +1215,25 @@ class BlockedPass(object):
         self.eng.launches = n
 
     # ------------------------------------------------------------------ checks
-    def check(self, shards, p_out, q_out=None):
+    def check(self, shards, p_out, q_out=None, p_first_out=None):
         """Raise ValueError unless the arguments of run() are complete; returns (sizes, p columns, q columns)."""
+        return self._check(shards, p_out, q_out, p_first_out)[:3]
+
+    def _check(self, shards, p_out, q_out, p_first_out):
         shards = list(shards)
-        sizes, ps, qs = [], [], []
+        sizes, ps, qs, p1s = [], [], [], None
         if p_out is None or len(p_out) != len(shards):
             raise ValueError("p_out: one column per shard")
         if self.q_values and (q_out is None or len(q_out) != len(shards)):
             raise ValueError("q_out: one column per shard (the pass was made with q_values=True)")
         if not self.q_values and q_out is not None:
             raise ValueError("q_out given, but the pass was made with q_values=False")
+        if p_first_out is not None:
+            if not self.refit:
+                raise ValueError("p_first_out needs a pass made with refit=True")
+            if len(p_first_out) != len(shards):
+                raise ValueError("p_first_out: one column per shard")
+            p1s = []
         for i, sh in enumerate(shards):
             if len(sh) != 4:
                 raise ValueError("shard %d: (chrom, mid1, mid2, count); BlockedPass takes one-chromosome shards" % i)
@@ -1210,11 +1243,13 @@ class BlockedPass(object):
             sizes.append(n)
             ps.append(_host_f64(p_out[i], n, "p_out[%d]" % i))
             qs.append(_host_f64(q_out[i], n, "q_out[%d]" % i) if self.q_values else None)
+            if p1s is not None:
+                p1s.append(_host_f64(p_first_out[i], n, "p_first_out[%d]" % i))
         blocks = plan_blocks(sizes, self.block_rows)
         cc = self._cand_cap(blocks)
         if len(blocks) * cc >= (1 << 32):
             raise ValueError("%d blocks of %d candidate places reach 2^32: use larger blocks" % (len(blocks), cc))
-        return sizes, ps, qs
+        return sizes, ps, qs, p1s
 
     def _cand_cap(self, blocks):
         if self.cand_capacity:
@@ -1257,18 +1292,23 @@ class BlockedPass(object):
                 self.eng.launches += 1 if q is None else 2
 
     # ------------------------------------------------------------------ the pass
-    def run(self, shards, p_out, q_out=None, n_tests=-1, marks=None):
+    def run(self, shards, p_out, q_out=None, n_tests=-1, marks=None, p_first_out=None):
         """Run the pass.  shards: [(chrom, mid1, mid2, count)], host columns (numpy integer arrays, or CPU tensors; pinned int32
         tensors go by one asynchronous copy each).  p_out / q_out: one float64 host column per shard, exactly as long as it
-        (numpy arrays or CPU tensors); q_out only with q_values.  n_tests: N of the q-values (-1: the number of non-NaN p).
-        marks (optional dict): CUDA events recorded after each stage.  Returns the FitResult; a failed fit raises what
-        GenomePass.run raises, before any p is computed and with p_out / q_out untouched."""
-        sizes, ps, qs = self.check(shards, p_out, q_out)
+        (numpy arrays or CPU tensors); q_out only with q_values.  n_tests: N of the q-values (-1: the number of non-NaN p); with
+        refit, of the refit pass.  marks (optional dict): CUDA events recorded after each stage ("start", "hist", "fit",
+        "pvalues", "bh"; with refit also "hist_first" and "fit_first" after sweep 1 and fit 1, and "hist" after sweep 2).
+        Returns the FitResult (with refit: the refit pass', pass 1's is fit_first); a failed fit raises what GenomePass.run
+        raises, before any p of its pass is computed and with p_out / q_out untouched.
+        p_first_out (refit only): one float64 host column per shard, like p_out, that receives pass 1's p.  It is written
+        during sweep 2, so it already holds pass 1's p when the refit pass' fit fails."""
+        sizes, ps, qs, p1s = self._check(shards, p_out, q_out, p_first_out)
         eng, lib, dev = self.eng, self.lib, self.device
         self._shards = [tuple(sh) for sh in shards]
         self.blocks = plan_blocks(sizes, self.block_rows)
         self.bytes_in = self.bytes_out = 0
         self.host_unpack_s = 0.0
+        self.fit_first = None
         nb = len(self.blocks)
         dev_rows = [block_device_rows(b) for b in self.blocks]
         main = torch.cuda.current_stream(dev)
@@ -1319,7 +1359,7 @@ class BlockedPass(object):
                 for r, keep in zip(dev_rows, self.resident)]
         slots = [tuple(torch.empty(slot_rows, dtype=torch.int32, device=dev) for _ in range(3)) for _ in range(2)] \
             if not all(self.resident) else []
-        far = [k for k in range(nb) if not self.resident[k]]         # blocks sent again in sweep 2, in turn through the two slots
+        far = [k for k in range(nb) if not self.resident[k]]         # blocks sent again in each later sweep, in turn through the two slots
         slot_of = {k: i & 1 for i, k in enumerate(far)}
         s_in, s_out = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
         s_in.wait_stream(main)
@@ -1335,6 +1375,82 @@ class BlockedPass(object):
                 s_in.wait_event(slot_free[slot_of[k]])        # the kernels that last read this slot have finished
             self._records_in(k, block_cols(k), s_in, in_ready[k])
 
+        def sweep():
+            """The blocks in order, each once its records are on the device: the resident ones are, the others are sent again
+            through the two slots, the next one while this one's kernels run."""
+            if far:
+                send(far[0])
+            for k in range(nb):
+                if not self.resident[k]:
+                    i = far.index(k)
+                    if i + 1 < len(far):
+                        send(far[i + 1])                      # into the other slot, while block k is scored
+                    main.wait_event(in_ready[k])
+                yield k
+
+        def records_done(k):
+            if not self.resident[k]:
+                slot_free[slot_of[k]].record(main)
+
+        bias = ctypes.byref(eng.bias.struct) if eng.bias is not None else None
+        flags = _lib.ptr(eng.bias.flags) if eng.bias is not None else None
+
+        def score(k, p, q, hist, cand):
+            """K4 of block k into the device columns p / q: score state k, the guard, the streaming pass per piece, the patch
+            pass.  Returns the pieces."""
+            state = ctypes.c_void_p(self.score_state.data_ptr() + k * ns)
+            _lib.check(lib.bbk_score_begin(state, hist if k == 0 else None, st), "bbk_score_begin")
+            _lib.check(lib.bbk_score_guard(_lib.ptr(eng.fit_result), _lib.ptr(eng.spline_y), state, st), "bbk_score_guard")
+            eng.launches += 2
+            if self.force_exact:
+                self.score_state[k * ns + 24:k * ns + 28] = torch.tensor([1, 0, 0, 0], dtype=torch.uint8, device=dev)
+            c = ctypes.byref(cand) if cand is not None else None
+            pieces = self._pieces(k, block_cols(k))
+            for (_, sh, off), st_i in zip(pieces, eng.fan_out(len(pieces))):
+                _lib.check(lib.bbk_score_pairs(_lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, sh.chrom, eng.R, eng.min_dist,
+                                               eng.max_dist, _lib.ptr(eng.fit_result), _lib.ptr(eng.spline_y), bias, flags, off,
+                                               _lib.ptr(p), _lib.ptr(q), hist, c, ctypes.byref(deferred), state,
+                                               st_i), "bbk_score_pairs")
+                eng.launches += 1
+            eng.fan_in()
+            _lib.check(lib.bbk_score_deferred(ctypes.byref(deferred), _lib.ptr(eng.fit_result), _lib.ptr(p), _lib.ptr(q),
+                                              hist, c, state, st), "bbk_score_deferred")
+            eng.launches += 1
+            return pieces
+
+        run_done = [torch.cuda.Event() for _ in range(2)]
+        counts_ready = [torch.cuda.Event() for _ in range(2)]
+        out_free = [torch.cuda.Event() for _ in range(2)]
+        pending = []
+
+        def send_back(k, j, p, q, p_cols, q_cols, with_state):
+            """Block k's results in slot j packed on the device and sent to the host; the previous block's are unpacked into
+            p_cols / q_cols meanwhile.  with_state: block k's score state comes back too."""
+            pk = packs[j]
+            pk.rows = dev_rows[k]
+            pk.pack(p, q, main)
+            eng.launches += 2
+            run_done[j].record(main)
+            s_out.wait_event(run_done[j])
+            hp = h_packs[j]
+            with torch.cuda.stream(s_out):
+                h_pack_state[j].copy_(pk.state, non_blocking=True)
+                if with_state:
+                    self._h_state[k * ns:(k + 1) * ns].copy_(self.score_state[k * ns:(k + 1) * ns], non_blocking=True)
+                nw, nc = int(lib.bbk_pack_code_words(dev_rows[k])), int(lib.bbk_pack_chunks(dev_rows[k])) * 24
+                hp.codes[:nw].copy_(pk.codes[:nw], non_blocking=True)
+                hp.chunks[:nc].copy_(pk.chunks[:nc], non_blocking=True)
+                self.bytes_out += 4 * nw + nc
+                counts_ready[j].record(s_out)
+            if pending:
+                self._unpack(*pending.pop())
+            pending.append((k, j, p, q, pk, hp, h_pack_state[j], counts_ready[j], out_free[j], s_out, p_cols, q_cols))
+
+        def drain():
+            if pending:
+                self._unpack(*pending.pop())
+            s_out.synchronize()
+
         # ---- sweep 1: K1 into one table
         _lib.check(lib.bbk_hist_init(_lib.ptr(eng.obs_sum), eng.nkeys, _lib.ptr(eng.totals), st), "bbk_hist_init")
         eng.launches += 1
@@ -1348,86 +1464,60 @@ class BlockedPass(object):
                 _lib.check(lib.bbk_hist_pairs(None, None, _lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, eng.R, eng.min_dist,
                                               eng.max_dist, eng.nkeys, _lib.ptr(eng.obs_sum), _lib.ptr(eng.totals), st), "bbk_hist_pairs")
                 eng.launches += 1
-            if not self.resident[k]:
-                slot_free[slot_of[k]].record(main)
+            records_done(k)
+
+        if self.refit:
+            mark("hist_first")
+            self.fit_first = self._settle_fit()                  # pass 1's fit: raises before any p exists
+            mark("fit_first")
+            # ---- sweep 2: pass 1's p per block into its p slot, then K1 into table 2 over the rows that are not outliers
+            _lib.check(lib.bbk_hist_init(_lib.ptr(eng.obs_sum), eng.nkeys, _lib.ptr(eng.totals), st), "bbk_hist_init")
+            eng.launches += 1
+            for k in sweep():
+                j = k & 1
+                p = pq[j][0]
+                main.wait_event(out_free[j])              # this slot's previous pass-1 p has left the device
+                if p1s is not None:
+                    self._nan_padding(k, p, None)
+                pieces = score(k, p, None, None, None)
+                for _, sh, off in pieces:
+                    _lib.check(lib.bbk_hist_pairs_excluding(None, None, _lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count),
+                                                             _lib.ptr(p[off:off + sh.n]), self.p_outlier, sh.n, eng.R, eng.min_dist,
+                                                             eng.max_dist, eng.nkeys, _lib.ptr(eng.obs_sum), _lib.ptr(eng.totals), st),
+                               "bbk_hist_pairs_excluding")
+                    eng.launches += 1
+                records_done(k)
+                if p1s is not None:
+                    send_back(k, j, p, None, p1s, None, False)
+            drain()
         mark("hist")
 
         # ---- the fit, settled on the host once
         fit = self._settle_fit()
         mark("fit")
 
-        # ---- sweep 2: scores, block after block; results packed, unpacked into the caller's columns by the host
+        # ---- the scoring sweep: block after block; results packed, unpacked into the caller's columns by the host
         want_q = self.q_values
         hist = _lib.ptr(eng.p_hist) if want_q else None
-        bias = ctypes.byref(eng.bias.struct) if eng.bias is not None else None
-        flags = _lib.ptr(eng.bias.flags) if eng.bias is not None else None
-        run_done = [torch.cuda.Event() for _ in range(2)]
-        counts_ready = [torch.cuda.Event() for _ in range(2)]
-        out_free = [torch.cuda.Event() for _ in range(2)]
         if nb == 0 and want_q:
             eng.p_hist.zero_()
             eng.launches += 1
-        pending = None
-        if far:
-            send(far[0])
-        for k in range(nb):
-            if not self.resident[k]:
-                i = far.index(k)
-                if i + 1 < len(far):
-                    send(far[i + 1])                      # into the other slot, while block k is scored
-                main.wait_event(in_ready[k])
+        for k in sweep():
             j = k & 1
             p, q = pq[j]
             main.wait_event(out_free[j])                  # this slot's previous results have left the device
             self._nan_padding(k, p, q)
-            state = ctypes.c_void_p(self.score_state.data_ptr() + k * ns)
-            _lib.check(lib.bbk_score_begin(state, hist if k == 0 else None, st), "bbk_score_begin")
-            _lib.check(lib.bbk_score_guard(_lib.ptr(eng.fit_result), _lib.ptr(eng.spline_y), state, st), "bbk_score_guard")
-            eng.launches += 2
-            if self.force_exact:
-                self.score_state[k * ns + 24:k * ns + 28] = torch.tensor([1, 0, 0, 0], dtype=torch.uint8, device=dev)
-            cand = ctypes.byref(cands[k][2]) if want_q else None
-            pieces = self._pieces(k, block_cols(k))
-            for (_, sh, off), st_i in zip(pieces, eng.fan_out(len(pieces))):
-                _lib.check(lib.bbk_score_pairs(_lib.ptr(sh.mid1), _lib.ptr(sh.mid2), _lib.ptr(sh.count), sh.n, sh.chrom, eng.R, eng.min_dist,
-                                               eng.max_dist, _lib.ptr(eng.fit_result), _lib.ptr(eng.spline_y), bias, flags, off,
-                                               _lib.ptr(p), _lib.ptr(q) if want_q else None, hist, cand, ctypes.byref(deferred), state,
-                                               st_i), "bbk_score_pairs")
-                eng.launches += 1
-            eng.fan_in()
-            _lib.check(lib.bbk_score_deferred(ctypes.byref(deferred), _lib.ptr(eng.fit_result), _lib.ptr(p), _lib.ptr(q) if want_q else None,
-                                              hist, cand, state, st), "bbk_score_deferred")
-            eng.launches += 1
-            if not self.resident[k]:
-                slot_free[slot_of[k]].record(main)
-            pk = packs[j]
-            pk.rows = dev_rows[k]
-            pk.pack(p, q, main)
-            eng.launches += 2
-            run_done[j].record(main)
-            s_out.wait_event(run_done[j])
-            hp = h_packs[j]
-            with torch.cuda.stream(s_out):
-                h_pack_state[j].copy_(pk.state, non_blocking=True)
-                self._h_state[k * ns:(k + 1) * ns].copy_(self.score_state[k * ns:(k + 1) * ns], non_blocking=True)
-                nw, nc = int(lib.bbk_pack_code_words(dev_rows[k])), int(lib.bbk_pack_chunks(dev_rows[k])) * 24
-                hp.codes[:nw].copy_(pk.codes[:nw], non_blocking=True)
-                hp.chunks[:nc].copy_(pk.chunks[:nc], non_blocking=True)
-                self.bytes_out += 4 * nw + nc
-                counts_ready[j].record(s_out)
-            if pending is not None:
-                self._unpack(*pending)
-            pending = (k, j, p, q, pk, hp, h_pack_state[j], counts_ready[j], out_free[j], s_out, ps, qs)
-        if pending is not None:
-            self._unpack(*pending)
-        s_out.synchronize()
+            score(k, p, q, hist, cands[k][2] if want_q else None)
+            records_done(k)
+            send_back(k, j, p, q, ps, qs, True)
+        drain()
         mark("pvalues")
         states = [_lib.ScoreState.from_buffer_copy(self._h_state.numpy().tobytes()[k * ns:(k + 1) * ns]) for k in range(nb)]
         if any(s.overflow for s in states):
             raise _lib.BbkError("a block's deferred list overflowed")     # it has a place for every row: cannot happen
         self.last_states = states
         # the records are not needed any more: the q-value step gets their memory
-        cols = slots = packs = pq = pending = None
+        cols = slots = packs = pq = None
         if want_q and nb:
             self._qvalues(int(n_tests), states, cands, ps, qs, dev_rows)
         mark("bh")

@@ -372,6 +372,18 @@ def _run_pass(resolution, n_bins, min_dist, max_dist, frag_chrom, frag_mid, chr1
     if refit:
         if world > 1:
             raise NotImplementedError("refit=True runs on one GPU")
+        if group is False and _blocked_ok(eng) and use_blocked_pass(n_rows + 3 * 64, want_q, dev, refit=True) and \
+                (runs := compact_runs(chr1, chr2, n_rows)) is not None:
+            # both passes larger than the device (or than 2^32 rows): the two-pass workload in row blocks from host memory
+            p = np.empty(n_rows, dtype=np.float64)
+            q = np.empty(n_rows, dtype=np.float64) if want_q else None
+            p1 = np.empty(n_rows, dtype=np.float64)
+            bp = BlockedPass(eng, q_values=want_q, refit=True)
+            fit = bp.run([(c, mid1[a:b], mid2[a:b], count[a:b]) for c, a, b in runs], [p[a:b] for _, a, b in runs],
+                         [q[a:b] for _, a, b in runs] if want_q else None, n_tests=nt, p_first_out=[p1[a:b] for _, a, b in runs])
+            out = _pass_output(eng, fit, info, resolution, min_dist, max_dist, None, None, p1, dev, scores=(p, q))
+            out.rows = (lo, hi)
+            return out
         same = chr1 is None or (np.asarray(chr1) == np.asarray(chr2)).all() and np.unique(np.asarray(chr1)).size <= 1
         if same:
             chrom = int(np.asarray(chr1).flat[0]) if chr1 is not None and len(chr1) else 0
@@ -442,26 +454,28 @@ def _blocked_ok(eng):
         not (eng.bias is not None and eng.bias.step == 1)
 
 
-def use_blocked_pass(rows, want_q, dev):
+def use_blocked_pass(rows, want_q, dev, refit=False):
     """Whether a single-GPU genome-wide pass over `rows` layout rows goes through distributed.BlockedPass: when the resident
-    pass cannot run (2^32 rows or more, or more device memory than is free: distributed.needs_blocked_pass)."""
+    pass cannot run (2^32 rows or more, or more device memory than is free: distributed.needs_blocked_pass).  refit: the
+    resident two-pass workload."""
     from .distributed import needs_blocked_pass
     if int(rows) >= (1 << 32):
         return True
     free, _ = torch.cuda.mem_get_info(dev)
-    return needs_blocked_pass(rows, free, want_q)
+    return needs_blocked_pass(rows, free, want_q, refit=refit)
 
 
 def _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows, first, dev, scores=None):
     """PassOutput of one finished pass: the engine's tables and fit, p / q / keep of the given rows (or of the host columns
-    scores = (p, q) a BlockedPass has filled)."""
+    scores = (p, q) a BlockedPass has filled).  first: pass 1's p of a refit, a device tensor or the host column a
+    BlockedPass has filled (or None)."""
     out = PassOutput()
     out.fit = fit
     out.frag = info
     host = {"x": _to_host(eng.x[:fit.n_out]), "y": _to_host(eng.y[:fit.n_out]),
             "spline_y": _to_host(eng.spline_y[:fit.L]), "spline_raw": _to_host(eng.spline_raw[:fit.L]),
             "possible": _to_host(eng.possible), "observed": _to_host(eng.obs_sum), "bin_of_key": _to_host(eng.bin_of_key),
-            "totals": _to_host(eng.totals), "first": _to_host(first) if first is not None else None}
+            "totals": _to_host(eng.totals), "first": _to_host(first) if isinstance(first, torch.Tensor) else None}
     if scores is None:
         out.p, out.q, out.keep = _scores_to_host(p_rows, q_rows, dev)    # keep: fithic.py:434 (NaN = not scored or dropped)
     else:
@@ -488,7 +502,7 @@ def _pass_output(eng, fit, info, resolution, min_dist, max_dist, p_rows, q_rows,
         "possibleIntraInRangeCount": _in_range_possible(out.possible, resolution, min_dist, max_dist),
     }
     out.gpu_launches = eng.launches
-    out.p_first = host["first"].numpy() if first is not None else None
+    out.p_first = host["first"].numpy() if host["first"] is not None else first
     return out
 
 
